@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Headline benchmark: dense SDF grid_eval throughput (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid 1024]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid 1024] [--dump-outputs DIR]
 
 One *step* = one pass of the grid_eval kernel (float4 gradient+distance output, the
 reference's INDEX3 layout) over the whole 1024^3 grid of the planetary-gearbox scene
@@ -21,6 +21,8 @@ Our arm prints ONE JSON line with
             bounded sample of the same grid, all host threads.
 `--impl reference` times the reference-side CPU implementation alone: oracle/_ref (the
 reference's own .cl sources compiled for the host) when it was built, else the oracle port.
+`--dump-outputs DIR` writes a fixed sample of the grid the last timed step computed to DIR
+(dump_grid_sample), so that two builds run with the same arguments can be compared point for point.
 """
 import argparse
 import ctypes
@@ -583,6 +585,47 @@ def d2h_probe(L, _lib, device_ptr, host_array, nbytes, torch, dist):
     return nbytes / dt / 1e9, nbytes / max_over_ranks(torch, dist, dt) / 1e9
 
 
+DUMP_POINTS = 1 << 20   # 16 MB of float4 values + 24 MB of their grid indices
+
+
+class _CudaArray:
+    """A device allocation of the library seen through the CUDA array interface: torch.as_tensor() wraps it without a
+    copy (the library allocates with the runtime API, in the primary context torch uses too)."""
+
+    def __init__(self, ptr, shape):
+        self.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": "<f4", "data": (int(ptr), False),
+                                         "strides": None, "version": 2}
+
+
+def dump_grid_sample(out_dir, L, _lib, out_buffer, x0, x1, n, rank, torch, dist):
+    """--dump-outputs: the float4 values (gradient x, y, z, distance) the last step left in the output grid, at a
+    fixed sample of its points: all of them when the n^3 grid has at most DUMP_POINTS, else DUMP_POINTS flat indices
+    drawn with seed 0 (sorted, duplicates dropped).  Writes grid_eval.npy, float32 [M][4], and grid_eval_index.npy,
+    float64 [M][3], the x, y, z grid indices of those points.  Each rank gathers on its GPU the sample points of its
+    slab [x0, x1) (out_buffer holds plane x0 first); rank 0 writes the files."""
+    total = n ** 3
+    if total <= DUMP_POINTS:
+        flat = np.arange(total, dtype=np.int64)
+    else:
+        flat = np.unique(np.random.default_rng(0).integers(0, total, DUMP_POINTS, dtype=np.int64))
+    lo, hi = x0 * n * n, x1 * n * n
+    mine = (flat >= lo) & (flat < hi)
+    _lib.check(L.cc_synchronize())
+    slab = torch.as_tensor(_CudaArray(out_buffer.device_ptr.value, ((x1 - x0) * n * n, 4)), device="cuda")
+    values = torch.zeros((len(flat), 4), dtype=torch.float32, device="cuda")
+    values[torch.from_numpy(mine).cuda()] = slab[torch.from_numpy(flat[mine] - lo).cuda()]
+    if dist is not None:
+        # each point was filled by the one rank whose slab holds it and is zero elsewhere: an integer sum of the bits
+        # over the ranks is that rank's value
+        dist.all_reduce(values.view(torch.int32))
+    values = values.cpu().numpy()
+    if rank == 0:
+        xs, yz = np.divmod(flat, n * n)
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, "grid_eval.npy"), values)
+        np.save(os.path.join(out_dir, "grid_eval_index.npy"), np.stack([xs, yz // n, yz % n], axis=1).astype(np.float64))
+
+
 def single_process_leg(n_devices):
     """One process, n GPUs (cc_init_devices): the unmodified module calls — the reference's user is a
     single Python script — fan out inside the library.  Prints one JSON object."""
@@ -785,6 +828,10 @@ def run_ours(args):
             t_load = time.time()
         clk = clocks.stop((t_begin, t_load))
         clk["window_s"] = {"timed_region": t_end - t_begin, "same_steps_continued_untimed": t_load - t_end}
+    if args.dump_outputs:
+        # on rank 0 the buffer was last written by the untimed steps that continued the timed ones for the clock
+        # samples: the same launch on the same inputs, whose result does not depend on how often it ran
+        dump_grid_sample(args.dump_outputs, L, _lib, out, kx0, kx1, n, rank, torch, dist)
     ms_total = max_over_ranks(torch, dist, ms_total)
     ms_step = ms_total / args.steps
     total_points = float(n) ** 3
@@ -1045,8 +1092,12 @@ def main():
     ap.add_argument("--grid", type=int, default=1024)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config dense grids and the single-process leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of the grid the last timed step computed to DIR as .npy files")
     ap.add_argument("--single-process-leg", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU arm's grid; --impl reference has none")
     if args.single_process_leg:
         return single_process_leg(args.single_process_leg)
     if args.impl == "reference":
