@@ -356,9 +356,8 @@ int launch_forest(const cc_program *prog, cc_eval_args &a, uint64_t points)
     // error budget of the primitives' bounds: 2^-16 of the magnitudes that enter their arithmetic
     const double ext[3] = {std::fabs((double)a.step) * (double)(a.nx + a.x_offset), std::fabs((double)a.step) * a.ny,
                            std::fabs((double)a.step) * a.nz};
-    // (launches over blocks: the caller's bound on every block's coordinates)
-    const double pmax = a.blocks ? (double)a.coord_max + std::max(ext[0], std::max(ext[1], ext[2]))
-                                 : std::max(std::fabs((double)a.cx) + ext[0], std::max(std::fabs((double)a.cy) + ext[1], std::fabs((double)a.cz) + ext[2]));
+    // (forest_applies admits no launch over blocks: the grid's own corner bounds the coordinates)
+    const double pmax = std::max(std::fabs((double)a.cx) + ext[0], std::max(std::fabs((double)a.cy) + ext[1], std::fabs((double)a.cz) + ext[2]));
     f.slack = (float)(((double)prog->dec.forest.err_a + (double)prog->dec.forest.err_b * pmax) / 65536.0);
     if (!std::isfinite(f.slack)) return fail(CC_ERR_INVALID_ARGUMENT, "grid coordinates out of range");
     const size_t ow = cc_forest_overflow_words(a);
@@ -412,7 +411,10 @@ int prepare_part_masks(const cc_program *prog, cc_eval_args &a, uint64_t nb)
     // most a few hundred fp32 operations deep: ~1e-5 relative; this allows 1.2e-4)
     const double ext[3] = {std::fabs((double)a.step) * (double)(a.nx + a.x_offset), std::fabs((double)a.step) * a.ny,
                            std::fabs((double)a.step) * a.nz};
-    const double pmax = std::max(std::fabs((double)a.cx) + ext[0], std::max(std::fabs((double)a.cy) + ext[1], std::fabs((double)a.cz) + ext[2]));
+    // (launches over blocks: a.cx/cy/cz are zero and the corners are in the block descriptors; the caller's
+    // bound on every block's coordinates stands in for them)
+    const double pmax = a.blocks ? (double)a.coord_max + std::max(ext[0], std::max(ext[1], ext[2]))
+                                 : std::max(std::fabs((double)a.cx) + ext[0], std::max(std::fabs((double)a.cy) + ext[1], std::fabs((double)a.cz) + ext[2]));
     a.part_slack = (float)(((double)prog->dec.parts.magnitude_a + (double)prog->dec.parts.magnitude_b * pmax) / 8192.0);
     if (!std::isfinite(a.part_slack)) return fail(CC_ERR_INVALID_ARGUMENT, "grid coordinates out of range");
     a.part_masks = g.d_part_masks;

@@ -668,18 +668,32 @@ void analyse_parts(const std::vector<uint32_t> &code, cc_parts *out)
         case MOP_LOAD: r = ls; coords_of[(size_t)v] = o.in_s >= 0 ? coords_of[(size_t)o.in_s] : -1; break;
         case MOP_NOP: r = li; coords_of[(size_t)v] = o.in_l >= 0 ? coords_of[(size_t)o.in_l] : -1; break;
         case MOP_MIRROR: case MOP_SYM_TO: case MOP_REV_TO: r = li; break;
-        case MOP_CIRCLE: case MOP_RECTANGLE: case MOP_POLYGON:
+        case MOP_CIRCLE: case MOP_RECTANGLE:  // r (and a zero word) / half width, half height
             r = li;
             coords_of[(size_t)v] = o.in_l;
             mag_a = std::max(mag_a, (double)std::fabs(fl(o.pc, 0)) + std::fabs(fl(o.pc, 1)));
             break;
+        case MOP_POLYGON: {
+            // the words are the vertex count and the edge table's offset: the magnitudes are the vertices'
+            // (every vertex is the start point of one edge)
+            const uint32_t nv = (uint32_t)fl(o.pc, 0), off = code[o.pc + 2];
+            for (uint32_t k = 0; k < nv; ++k) {
+                float px, py;
+                std::memcpy(&px, &code[off + CC_POLY_EDGE_WORDS * k], 4);
+                std::memcpy(&py, &code[off + CC_POLY_EDGE_WORDS * k + 1], 4);
+                mag_a = std::max(mag_a, (double)std::fabs(px) + std::fabs(py));
+            }
+            r = li;
+            coords_of[(size_t)v] = o.in_l;
+            break;
+        }
         case MOP_SPHERE: case MOP_HALF_SPACE: r = li; mag_a = std::max(mag_a, (double)std::fabs(fl(o.pc, 0))); break;
         case MOP_GEAR: {
             const double tooth = fl(o.pc, 1), half = fl(o.pc, 2);
             const double gmax = std::max(std::fabs(half), std::fabs(tooth - half));
             r = li * std::sqrt(1 + gmax * gmax) * (1 + 1e-5);
             coords_of[(size_t)v] = o.in_l;
-            mag_a = std::max(mag_a, 8.0);  // angles up to 4 pi enter the arithmetic
+            mag_a = std::max(mag_a, 4.0 * M_PI);  // angles up to 4 pi enter the arithmetic
             break;
         }
         case MOP_OFFSET: case MOP_SHELL:
