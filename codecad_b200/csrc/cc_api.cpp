@@ -49,7 +49,7 @@ struct Context {
     bool mesh_tables = false;       // marching-cubes tables uploaded to this device
     // look-back scratch
     uint32_t *d_forest_scratch = nullptr;  // deferred super-tiles of the union-forest kernel
-    size_t forest_scratch_words = 0;
+    size_t forest_scratch_cap = 0;
     uint32_t *d_ticket = nullptr;
     unsigned long long *d_status = nullptr;
     size_t status_cap = 0;
@@ -116,15 +116,16 @@ int make_event(cc_event **ev, cudaStream_t st)
     return CC_OK;
 }
 
-int ensure_status(size_t tiles)
+// grows a scratch buffer of the context to at least `bytes` (cap: its size); what it held is not kept
+template <class T>
+int grow(T *&ptr, size_t &cap, size_t bytes)
 {
-    if (!g.d_ticket) CU(cudaMalloc(&g.d_ticket, 4));
-    if (tiles > g.status_cap) {
-        if (g.d_status) CU(cudaFree(g.d_status));
-        size_t cap = std::max<size_t>(tiles, 1 << 16);
-        CU(cudaMalloc(&g.d_status, cap * sizeof(unsigned long long)));
-        g.status_cap = cap;
-    }
+    if (bytes <= cap) return CC_OK;
+    if (ptr) CU(cudaFree(ptr));
+    ptr = nullptr;
+    cap = 0;
+    CU(cudaMalloc(&ptr, bytes));
+    cap = bytes;
     return CC_OK;
 }
 
@@ -251,24 +252,30 @@ struct PinnedPool {
 };
 PinnedPool g_pinned;
 
-// the program's microcode on the current device (replicated on first use)
+// `d`: a program's table on the current device, copied there on first use (`n0` bytes from `h0`, then `n1` from `h1`)
+template <class T>
+int replicate(T *&d, const void *h0, size_t n0, const void *h1, size_t n1, const char *what)
+{
+    if (d) return CC_OK;
+    cudaError_t e = cudaMalloc(&d, n0 + n1);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d, h0, n0, cudaMemcpyHostToDevice, g.compute);
+    if (e == cudaSuccess && n1) e = cudaMemcpyAsync((char *)d + n0, h1, n1, cudaMemcpyHostToDevice, g.compute);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(g.compute);
+    if (e != cudaSuccess) {
+        if (d) cudaFree(d);
+        d = nullptr;
+        return cuda_fail(e, what);
+    }
+    return CC_OK;
+}
+
+// the program's microcode on the current device
 int program_on_device(const cc_program *prog, const uint32_t **out)
 {
-    cc_program *p = const_cast<cc_program *>(prog);
-    uint32_t *&d = p->d_code[g.index];
-    if (!d) {
-        const size_t bytes = p->dec.microcode.size() * 4;
-        cudaError_t e = cudaMalloc(&d, bytes);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d, p->dec.microcode.data(), bytes, cudaMemcpyHostToDevice, g.compute);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(g.compute);
-        if (e != cudaSuccess) {
-            if (d) cudaFree(d);
-            d = nullptr;
-            return cuda_fail(e, "program upload");
-        }
-    }
+    uint32_t *&d = const_cast<cc_program *>(prog)->d_code[g.index];
+    int rc = replicate(d, prog->dec.microcode.data(), prog->dec.microcode.size() * 4, nullptr, 0, "program upload");
     *out = d;
-    return CC_OK;
+    return rc;
 }
 
 int fill_common(cc_eval_args *a, const cc_program *prog)
@@ -313,24 +320,13 @@ bool jit_ready(cc_program *p, int sink)
     return r == 1;
 }
 
-// tables of a union-forest program on the current device (replicated on first use)
+// tables of a union-forest program on the current device
 int forest_on_device(const cc_program *prog, cc_forest_launch *out)
 {
-    cc_program *p = const_cast<cc_program *>(prog);
-    const cc_forest &f = p->dec.forest;
-    void *&d = p->d_forest[g.index];
+    const cc_forest &f = prog->dec.forest;
+    void *&d = const_cast<cc_program *>(prog)->d_forest[g.index];
     const size_t nb = f.bounds.size() * 4, ne = f.events.size() * 4;
-    if (!d) {
-        cudaError_t e = cudaMalloc(&d, nb + ne);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d, f.bounds.data(), nb, cudaMemcpyHostToDevice, g.compute);
-        if (e == cudaSuccess) e = cudaMemcpyAsync((char *)d + nb, f.events.data(), ne, cudaMemcpyHostToDevice, g.compute);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(g.compute);
-        if (e != cudaSuccess) {
-            if (d) cudaFree(d);
-            d = nullptr;
-            return cuda_fail(e, "forest table upload");
-        }
-    }
+    if (int rc = replicate(d, f.bounds.data(), nb, f.events.data(), ne, "forest table upload")) return rc;
     out->bounds = (const float *)d;
     out->events = (const uint32_t *)((char *)d + nb);
     out->n_leaves = f.n_leaves;
@@ -340,12 +336,40 @@ int forest_on_device(const cc_program *prog, cc_forest_launch *out)
     return CC_OK;
 }
 
-bool forest_applies(int sink_kind, const cc_program *prog, const cc_eval_args &a)
+// cc_parts::table on the current device
+int parts_on_device(const cc_program *prog, const uint32_t **out)
 {
-    if (!g.forest_mode || sink_kind != CC_SINK_FLOAT4 || a.points || a.blocks) return false;
-    const cc_forest &f = prog->dec.forest;
-    return f.enabled && cc_forest_smem_bytes(f) <= (size_t)g.prop.sharedMemPerBlockOptin && f.n_events <= 8192 &&
-           f.n_leaves <= 8192;
+    uint32_t *&d = const_cast<cc_program *>(prog)->d_parts[g.index];
+    int rc = replicate(d, prog->dec.parts.table.data(), prog->dec.parts.table.size() * 4, nullptr, 0, "part table upload");
+    *out = d;
+    return rc;
+}
+
+// What a program can use under the current modes.  The specialised part, column and tile kernels exist for programs that
+// are not cut into segments (cc_jit_is_segmented); the interpreter's part culling serves segmented ones too.
+struct Structures {
+    bool forest;        // union forest within the culling kernel's limits, forest mode on
+    bool parts;         // an assembly, parts mode on
+    bool parts_jit;     // ... through the specialised part kernels
+    bool parts_interp;  // ... through the interpreter's segment table (microcode in shared memory, two CTAs per SM)
+    bool columns;       // the column split, columns mode on (specialised kernels only)
+    bool tiles;         // tile units of the hierarchy sinks: part masks and / or the column split
+};
+
+Structures structures_of(const cc_program *prog)
+{
+    const cc_decoded &d = prog->dec;
+    const bool whole = !cc_jit_is_segmented(d);
+    Structures s;
+    s.forest = g.forest_mode && d.forest.enabled && cc_forest_smem_bytes(d.forest) <= (size_t)g.prop.sharedMemPerBlockOptin &&
+               d.forest.n_events <= 8192 && d.forest.n_leaves <= 8192;
+    s.parts = g.parts_mode && d.parts.enabled;
+    s.parts_jit = s.parts && whole;
+    s.parts_interp = s.parts && !d.parts.table.empty() && d.parts.n_parts <= 32 &&
+                     cc_parts_smem_bytes(d.info.n_slots, d.info.n_micro_words, 2) * 2 <= (size_t)g.prop.sharedMemPerMultiprocessor;
+    s.columns = g.columns_mode && d.columns.enabled && whole;
+    s.tiles = s.parts_jit || s.columns;
+    return s;
 }
 
 int launch_forest(const cc_program *prog, cc_eval_args &a, uint64_t points)
@@ -356,18 +380,11 @@ int launch_forest(const cc_program *prog, cc_eval_args &a, uint64_t points)
     // error budget of the primitives' bounds: 2^-16 of the magnitudes that enter their arithmetic
     const double ext[3] = {std::fabs((double)a.step) * (double)(a.nx + a.x_offset), std::fabs((double)a.step) * a.ny,
                            std::fabs((double)a.step) * a.nz};
-    // (forest_applies admits no launch over blocks: the grid's own corner bounds the coordinates)
+    // (the forest serves no launch over blocks: the grid's own corner bounds the coordinates)
     const double pmax = std::max(std::fabs((double)a.cx) + ext[0], std::max(std::fabs((double)a.cy) + ext[1], std::fabs((double)a.cz) + ext[2]));
     f.slack = (float)(((double)prog->dec.forest.err_a + (double)prog->dec.forest.err_b * pmax) / 65536.0);
     if (!std::isfinite(f.slack)) return fail(CC_ERR_INVALID_ARGUMENT, "grid coordinates out of range");
-    const size_t ow = cc_forest_overflow_words(a);
-    if (ow > g.forest_scratch_words) {
-        if (g.d_forest_scratch) CU(cudaFree(g.d_forest_scratch));
-        g.d_forest_scratch = nullptr;
-        g.forest_scratch_words = 0;
-        CU(cudaMalloc(&g.d_forest_scratch, ow * 4));
-        g.forest_scratch_words = ow;
-    }
+    if ((rc = grow(g.d_forest_scratch, g.forest_scratch_cap, (size_t)cc_forest_overflow_words(a) * 4))) return rc;
     int e = cc_launch_forest(a, f, g.d_forest_scratch, g.prop.multiProcessorCount, g.compute);
     if (e) return cuda_fail((cudaError_t)e, "cc_forest_kernel launch");
     g.launches += 1;
@@ -375,38 +392,16 @@ int launch_forest(const cc_program *prog, cc_eval_args &a, uint64_t points)
     return CC_OK;
 }
 
-// Dense float4 grid of an assembly through the part-culling kernels (DESIGN.md 4.9); the caller checked
-// that the specialised kernels of CC_SINK_PARTS are loaded.
-// cc_parts::table on the current device (replicated on first use)
-int parts_on_device(const cc_program *prog, const uint32_t **out)
+// 8 x 8 x 16 bricks covering an nx x ny x nz grid
+uint64_t brick_count(uint32_t nx, uint32_t ny, uint32_t nz)
 {
-    cc_program *p = const_cast<cc_program *>(prog);
-    uint32_t *&d = p->d_parts[g.index];
-    if (!d) {
-        const size_t bytes = p->dec.parts.table.size() * 4;
-        cudaError_t e = cudaMalloc(&d, bytes);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d, p->dec.parts.table.data(), bytes, cudaMemcpyHostToDevice, g.compute);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(g.compute);
-        if (e != cudaSuccess) {
-            if (d) cudaFree(d);
-            d = nullptr;
-            return cuda_fail(e, "part table upload");
-        }
-    }
-    *out = d;
-    return CC_OK;
+    return (uint64_t)((nx + CC_BRICK_X - 1) / CC_BRICK_X) * ((ny + CC_BRICK_Y - 1) / CC_BRICK_Y) * ((nz + CC_BRICK_Z - 1) / CC_BRICK_Z);
 }
 
-// the brick masks' buffer and the rounding budget of the parts' values
+// the masks' buffer (one per brick or tile) and the rounding budget of the parts' values
 int prepare_part_masks(const cc_program *prog, cc_eval_args &a, uint64_t nb)
 {
-    if (nb > g.part_masks_cap) {
-        if (g.d_part_masks) CU(cudaFree(g.d_part_masks));
-        g.d_part_masks = nullptr;
-        g.part_masks_cap = 0;
-        CU(cudaMalloc(&g.d_part_masks, (size_t)nb * 4));
-        g.part_masks_cap = (size_t)nb;
-    }
+    if (int rc = grow(g.d_part_masks, g.part_masks_cap, (size_t)nb * 4)) return rc;
     // rounding budget of a part's value: 2^-13 of the magnitudes that enter its arithmetic (a part is at
     // most a few hundred fp32 operations deep: ~1e-5 relative; this allows 1.2e-4)
     const double ext[3] = {std::fabs((double)a.step) * (double)(a.nx + a.x_offset), std::fabs((double)a.step) * a.ny,
@@ -421,229 +416,157 @@ int prepare_part_masks(const cc_program *prog, cc_eval_args &a, uint64_t nb)
     return CC_OK;
 }
 
-// `specialised`: the NVRTC pair is loaded; otherwise the interpreter-tier pair of cc_parts.cu
-int launch_parts(const cc_program *prog, cc_eval_args &a, uint64_t points, bool specialised)
+// bytes of the column buffer's values: 4 floats per carried value (at least one) and column
+uint64_t column_values_bytes(uint64_t n_columns, const cc_columns_meta &meta)
 {
-    const uint64_t nb = (uint64_t)((a.nx + CC_BRICK_X - 1) / CC_BRICK_X) * ((a.ny + CC_BRICK_Y - 1) / CC_BRICK_Y) *
-                        ((a.nz + CC_BRICK_Z - 1) / CC_BRICK_Z);
-    if (nb >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many bricks in one launch");
-    int prc = prepare_part_masks(prog, a, nb);
-    if (prc) return prc;
-    int e;
-    if (specialised) {
-        e = cc_jit_launch_parts(prog, a, (uint32_t)nb, g.compute, g.index);
-    } else {
-        const uint32_t *table = nullptr;
-        int rc = parts_on_device(prog, &table);
-        if (rc) return rc;
-        e = cc_launch_parts_interp(a, table, (uint32_t)nb, g.compute);
-    }
-    if (e) return cuda_fail((cudaError_t)e, "part-culling kernel launch");
-    g.launches += 2;
-    g.points += points;
-    return CC_OK;
+    return n_columns * 16 * std::max(1u, meta.n_values);
 }
 
-// Dense float4 grid through the column kernel (DESIGN.md 4.10): one warp per 8 x 8 x 16 brick, what does not
-// depend on z evaluated once per column; with the parts' masks when the scene is an assembly.
-int launch_columns(const cc_program *prog, cc_eval_args &a, uint64_t points, bool with_parts)
+// The column buffer of every block's columns: the values; when some transform row is checked per column, a flag per
+// column behind them and, for a launch over `n_bricks` bricks (0: over tiles), the count and list of the bricks whose full
+// walk the check asks for.
+int prepare_columns(const cc_columns_meta &meta, cc_eval_args &a, uint64_t n_bricks)
 {
-    const uint64_t nb = (uint64_t)((a.nx + CC_BRICK_X - 1) / CC_BRICK_X) * ((a.ny + CC_BRICK_Y - 1) / CC_BRICK_Y) *
-                        ((a.nz + CC_BRICK_Z - 1) / CC_BRICK_Z);
-    if (nb >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many bricks in one launch");
-    const cc_columns_meta &meta = prog->jit_columns;
-    const int axis = meta.axis;
-    const uint64_t ncol = axis == 2 ? (uint64_t)a.nx * a.ny : axis == 1 ? (uint64_t)a.nx * a.nz : (uint64_t)a.ny * a.nz;
-    // column buffer (+ flags, brick list, counter behind it when some transform row is checked per column)
-    const size_t values = (size_t)ncol * 4 * std::max(1u, meta.n_values) * sizeof(float);
+    const uint64_t ncol = std::max(1u, a.n_blocks) * columns_along(meta.axis, a.nx, a.ny, a.nz);
+    const size_t values = column_values_bytes(ncol, meta);
     const size_t flags_at = (values + 255) & ~(size_t)255, list_at = (flags_at + ncol + 255) & ~(size_t)255;
-    const size_t bytes = meta.checks ? list_at + ((size_t)nb + 1) * 4 : values;
-    if (bytes > g.columns_cap) {
-        if (g.d_columns) CU(cudaFree(g.d_columns));
-        g.d_columns = nullptr;
-        g.columns_cap = 0;
-        CU(cudaMalloc(&g.d_columns, bytes));
-        g.columns_cap = bytes;
-    }
-    a.columns = reinterpret_cast<float *>(g.d_columns);
-    a.column_flags = nullptr;
-    a.brick_list = a.brick_count = nullptr;
-    if (meta.checks) {
-        a.column_flags = reinterpret_cast<unsigned char *>(g.d_columns) + flags_at;
-        a.brick_count = reinterpret_cast<uint32_t *>(reinterpret_cast<char *>(g.d_columns) + list_at);
-        a.brick_list = a.brick_count + 1;
-        CU(cudaMemsetAsync(a.brick_count, 0, 4, g.compute));
-    }
-    a.part_masks = nullptr;
-    if (with_parts) {
-        int rc = prepare_part_masks(prog, a, nb);
-        if (rc) return rc;
-    }
-    int n_launches = 0;
-    int e = cc_jit_launch_columns(prog, a, (uint32_t)nb, g.prop.multiProcessorCount, g.compute, g.index, &n_launches);
-    if (e) return cuda_fail((cudaError_t)e, "column kernel launch");
-    g.launches += (uint64_t)n_launches;
-    g.points += points;
+    const size_t bytes = !meta.checks ? values : n_bricks ? list_at + ((size_t)n_bricks + 1) * 4 : flags_at + ncol;
+    if (int rc = grow(g.d_columns, g.columns_cap, bytes)) return rc;
+    char *base = static_cast<char *>(g.d_columns);
+    a.columns = reinterpret_cast<float *>(base);
+    a.column_flags = meta.checks ? reinterpret_cast<unsigned char *>(base + flags_at) : nullptr;
+    a.brick_count = meta.checks && n_bricks ? reinterpret_cast<uint32_t *>(base + list_at) : nullptr;
+    a.brick_list = a.brick_count ? a.brick_count + 1 : nullptr;
+    if (a.brick_count) CU(cudaMemsetAsync(a.brick_count, 0, 4, g.compute));
     return CC_OK;
 }
 
-// The hierarchy sinks (ordered hit lists, mass sums, PyMCubes fields of blocks) through the brick units' tile
-// kernels: with `columns` the column pass covers the columns of every block of the launch and the tile kernel
-// runs the per-cell body; with `masks` a tile-centre pass writes a part mask per tile first.
+// tiles_per_block for tiles of `tile` cells; the sinks that compact their output (CLASSIFY, MASS) also get a zeroed
+// ticket and look-back status per tile
+int prepare_tiles(int sink_kind, uint32_t tile, cc_eval_args &a)
+{
+    a.tiles_per_block = (uint32_t)(((uint64_t)a.nx * a.ny * a.nz + tile - 1) / tile);
+    const uint64_t tiles = (uint64_t)a.tiles_per_block * a.n_blocks;
+    if (tiles >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many tiles in one launch");
+    if (sink_kind != CC_SINK_CLASSIFY && sink_kind != CC_SINK_MASS) return CC_OK;
+    if (!g.d_ticket) CU(cudaMalloc(&g.d_ticket, 4));
+    if (int rc = grow(g.d_status, g.status_cap, std::max<size_t>(tiles, 1 << 16) * sizeof(unsigned long long))) return rc;
+    CU(cudaMemsetAsync(g.d_ticket, 0, 4, g.compute));
+    CU(cudaMemsetAsync(g.d_status, 0, (size_t)tiles * sizeof(unsigned long long), g.compute));
+    a.ticket = g.d_ticket;
+    a.tile_status = g.d_status;
+    return CC_OK;
+}
+
 int tile_sink_of(int sink_kind)
 {
     return sink_kind == CC_SINK_PYMCUBES ? CC_SINK_TILES_PYMCUBES : sink_kind == CC_SINK_CLASSIFY ? CC_SINK_TILES_CLASSIFY : CC_SINK_TILES_MASS;
 }
 
-int launch_tiles(int sink_kind, const cc_program *prog, cc_eval_args &a, uint64_t points, bool columns, bool masks)
+// The kernels that serve a launch.
+enum class Path {
+    forest,        // dense float4 grid of a union forest: the culling kernel (cc_forest.cu)
+    columns,       // dense float4 grid: column pass + brick kernel (DESIGN.md 4.10), with the part masks of an assembly
+    tiles,         // hierarchy sinks: a tile unit's per-cell body of the column split and / or a part mask per tile
+    parts_jit,     // dense float4 grid of an assembly: brick centres + culled brick kernel (DESIGN.md 4.9), specialised
+    parts_interp,  // ... the same culling on the interpreter tier (cc_parts.cu)
+    specialised,   // blocks x linear tiles: the scene-specialised kernel of the sink
+    interpreter,   // blocks x linear tiles: the interpreter (cc_kernels.cu)
+};
+struct Route {
+    Path path;
+    int sink;              // the specialised unit
+    bool masks, columns;   // the unit's part masks / column buffer are needed
+};
+
+// The tests run in order of preference.  The order of the jit_ready calls belongs to it: on a program's first
+// launches they start the background compiles of the units asked for.
+Route route(int sink_kind, const cc_program *prog, const cc_eval_args &a)
 {
-    const int sink = tile_sink_of(sink_kind);
-    const cc_columns_meta &meta = prog->jit_tiles[sink - CC_SINK_TILES_PYMCUBES];
-    const uint32_t tile = (uint32_t)(prog->jit_cfg[sink].threads * prog->jit_cfg[sink].pts);
+    cc_program *p = const_cast<cc_program *>(prog);
+    const Structures can = structures_of(prog);
     const uint64_t cells = (uint64_t)a.nx * a.ny * a.nz;
-    a.tiles_per_block = (uint32_t)((cells + tile - 1) / tile);
-    const uint64_t tiles = (uint64_t)a.tiles_per_block * a.n_blocks;
-    if (tiles >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many tiles in one launch");
-    if (sink_kind == CC_SINK_CLASSIFY || sink_kind == CC_SINK_MASS) {
-        int rc = ensure_status((size_t)tiles);
-        if (rc) return rc;
-        CU(cudaMemsetAsync(g.d_ticket, 0, 4, g.compute));
-        CU(cudaMemsetAsync(g.d_status, 0, (size_t)tiles * sizeof(unsigned long long), g.compute));
-        a.ticket = g.d_ticket;
-        a.tile_status = g.d_status;
-    }
-    a.columns = nullptr;
-    a.column_flags = nullptr;
-    if (columns) {
-        const int axis = meta.axis;
-        const uint64_t ncol = (uint64_t)a.n_blocks * (axis == 2 ? (uint64_t)a.nx * a.ny : axis == 1 ? (uint64_t)a.nx * a.nz : (uint64_t)a.ny * a.nz);
-        const size_t values = (size_t)ncol * 4 * std::max(1u, meta.n_values) * sizeof(float);
-        const size_t flags_at = (values + 255) & ~(size_t)255;
-        const size_t bytes = meta.checks ? flags_at + ncol : values;
-        if (bytes > g.columns_cap) {
-            if (g.d_columns) CU(cudaFree(g.d_columns));
-            g.d_columns = nullptr;
-            g.columns_cap = 0;
-            CU(cudaMalloc(&g.d_columns, bytes));
-            g.columns_cap = bytes;
+    const int axis = prog->dec.columns.axis;
+    const uint32_t along = axis == 0 ? a.nx : axis == 1 ? a.ny : a.nz;  // cells per column
+    const uint64_t n_columns = std::max(1u, a.n_blocks) * columns_along(axis, a.nx, a.ny, a.nz);
+    const bool dense = sink_kind == CC_SINK_FLOAT4 && !a.points && !a.blocks;
+    if (dense && can.forest) return {Path::forest, -1, false, false};
+    const bool dense_parts = dense && can.parts && cells >= 4096;
+    // (the specialised column kernels or nothing: until they are loaded the other paths serve the launch)
+    if (dense && can.columns && along >= 8 && cells >= 4096 && jit_ready(p, CC_SINK_COLUMNS) &&
+        column_values_bytes(n_columns, p->jit_meta[CC_SINK_COLUMNS]) <= (8ull << 30))
+        return {Path::columns, CC_SINK_COLUMNS, dense_parts, true};
+    if ((sink_kind == CC_SINK_CLASSIFY || sink_kind == CC_SINK_MASS || (sink_kind == CC_SINK_PYMCUBES && a.blocks)) && !a.points &&
+        can.tiles && cells >= 512) {
+        const int sink = tile_sink_of(sink_kind);
+        const bool masks = can.parts && (!a.blocks || a.coord_max > 0.0f);
+        const bool cols = can.columns && along >= 8;
+        if ((masks || cols) && jit_ready(p, sink)) {
+            const cc_columns_meta &meta = p->jit_meta[sink];
+            // (the unit's per-cell body reads the column buffer whenever the program has a split: no columns, no unit)
+            if (!meta.columns || (cols && column_values_bytes(n_columns, meta) <= (8ull << 30)))
+                return {Path::tiles, sink, masks, meta.columns};
         }
-        a.columns = reinterpret_cast<float *>(g.d_columns);
-        a.column_flags = meta.checks ? reinterpret_cast<unsigned char *>(g.d_columns) + flags_at : nullptr;
     }
-    a.part_masks = nullptr;
-    if (masks) {
-        int rc = prepare_part_masks(prog, a, tiles);
-        if (rc) return rc;
+    if (dense_parts) {
+        if (can.parts_jit && jit_ready(p, CC_SINK_PARTS)) return {Path::parts_jit, CC_SINK_PARTS, true, false};
+        if (can.parts_interp) return {Path::parts_interp, -1, true, false};
     }
-    int n_launches = 0;
-    int e = cc_jit_launch_tiles(prog, sink, a, g.compute, g.index, &n_launches);
-    if (e) return cuda_fail((cudaError_t)e, "tile kernel launch");
-    g.launches += (uint64_t)n_launches;
-    g.points += points;
-    return CC_OK;
-}
-
-uint64_t axis_len(const cc_program *prog, const cc_eval_args &a)
-{
-    const int axis = prog->dec.columns.axis;
-    return std::max(1u, axis == 0 ? a.nx : axis == 1 ? a.ny : a.nz);
-}
-
-bool columns_apply(int sink_kind, const cc_program *prog, const cc_eval_args &a)
-{
-    const int axis = prog->dec.columns.axis;
-    return g.columns_mode && sink_kind == CC_SINK_FLOAT4 && !a.points && !a.blocks && prog->dec.columns.enabled && !cc_jit_is_segmented(prog->dec) &&
-           (axis == 0 ? a.nx : axis == 1 ? a.ny : a.nz) >= 8 && (uint64_t)a.nx * a.ny * a.nz >= 4096;
-}
-
-bool parts_apply(int sink_kind, const cc_program *prog, const cc_eval_args &a)
-{
-    return g.parts_mode && sink_kind == CC_SINK_FLOAT4 && !a.points && !a.blocks && prog->dec.parts.enabled &&
-           (uint64_t)a.nx * a.ny * a.nz >= 4096;
+    // point lists have their own specialised kernel (cc_jit_points)
+    const int sink = a.points ? (int)CC_SINK_POINTS : sink_kind;
+    if (jit_ready(p, sink)) return {Path::specialised, sink, false, false};
+    return {Path::interpreter, -1, false, false};
 }
 
 int launch(int sink_kind, const cc_program *prog, cc_eval_args &a, uint64_t points)
 {
-    if (forest_applies(sink_kind, prog, a)) return launch_forest(prog, a, points);
-    if (columns_apply(sink_kind, prog, a)) {
-        cc_program *p = const_cast<cc_program *>(prog);
-        const bool with_parts = parts_apply(sink_kind, prog, a);
-        // (the specialised column kernels or nothing: until they are loaded the other paths serve the launch)
-        if (jit_ready(p, CC_SINK_COLUMNS) && (uint64_t)a.nx * a.ny * a.nz / (axis_len(prog, a)) * 16 * std::max(1u, p->jit_columns.n_values) <= (8ull << 30))
-            return launch_columns(prog, a, points, with_parts);
-    }
-    if ((sink_kind == CC_SINK_CLASSIFY || sink_kind == CC_SINK_MASS || (sink_kind == CC_SINK_PYMCUBES && a.blocks)) && !a.points &&
-        !cc_jit_is_segmented(prog->dec) && (uint64_t)a.nx * a.ny * a.nz >= 512) {
-        // blocks x linear tiles: the per-cell body of the column split and / or a part mask per tile (one unit per sink)
-        cc_program *p = const_cast<cc_program *>(prog);
-        const bool masks = g.parts_mode && prog->dec.parts.enabled && (!a.blocks || a.coord_max > 0.0f);
-        const bool cols = g.columns_mode && prog->dec.columns.enabled && axis_len(prog, a) >= 8;
-        if ((masks || cols) && jit_ready(p, tile_sink_of(sink_kind))) {
-            const cc_columns_meta &meta = p->jit_tiles[tile_sink_of(sink_kind) - CC_SINK_TILES_PYMCUBES];
-            const bool fits = (uint64_t)a.n_blocks * a.nx * a.ny * a.nz / axis_len(prog, a) * 16 * std::max(1u, meta.n_values) <= (8ull << 30);
-            // (the unit's per-cell body reads the column buffer whenever the program has a split: no columns, no unit)
-            if (!meta.columns || (cols && fits)) return launch_tiles(sink_kind, prog, a, points, meta.columns, masks);
+    const Route r = route(sink_kind, prog, a);
+    int rc, e, n_launches = 1;
+    const char *what;
+    if (r.path == Path::forest) return launch_forest(prog, a, points);
+    if (r.path == Path::interpreter) {
+        cc_launch_cfg cfg;
+        if ((rc = choose_cfg(prog, points, &cfg))) return rc;
+        if (a.points) {  // the point-list kernels exist for 1 / 2 points per thread, constant or shared program
+            if (cfg.pts > 2) cfg.pts = 2;
+            if (cfg.prog_space == 3) cfg.prog_space = 1;
         }
-    }
-    if (parts_apply(sink_kind, prog, a)) {
-        if (!cc_jit_is_segmented(prog->dec) && jit_ready(const_cast<cc_program *>(prog), CC_SINK_PARTS)) return launch_parts(prog, a, points, true);
-        // interpreter tier: the same culling by walking the segment table (needs the microcode in shared memory)
-        if (!prog->dec.parts.table.empty() && prog->dec.parts.n_parts <= 32 &&
-            cc_parts_smem_bytes(prog->dec.info.n_slots, prog->dec.info.n_micro_words, 2) * 2 <= (size_t)g.prop.sharedMemPerMultiprocessor)
-            return launch_parts(prog, a, points, false);
-    }
-    // which specialised kernel serves the launch: point lists have their own (cc_jit_points)
-    const int sink = a.points ? (int)CC_SINK_POINTS : sink_kind;
-    if (jit_ready(const_cast<cc_program *>(prog), sink)) {
+        if ((rc = prepare_program(prog, cfg))) return rc;
+        if ((rc = prepare_tiles(sink_kind, cc_tile_points(cfg), a))) return rc;
+        e = cc_launch_eval(sink_kind, cfg, a, g.compute);
+        what = "cc_eval_kernel launch";
+    } else if (r.path == Path::specialised) {
         // scene-specialised kernel: slots are registers, parameters immediates
-        const uint32_t tile = (uint32_t)(prog->jit_cfg[sink].threads * prog->jit_cfg[sink].pts);
-        const uint64_t cells = (uint64_t)a.nx * a.ny * a.nz;
-        a.tiles_per_block = (uint32_t)((cells + tile - 1) / tile);
-        const uint64_t tiles = (uint64_t)a.tiles_per_block * a.n_blocks;
-        if (tiles >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many tiles in one launch");
-        if (sink == CC_SINK_CLASSIFY || sink == CC_SINK_MASS) {
-            int rc = ensure_status((size_t)tiles);
-            if (rc) return rc;
-            CU(cudaMemsetAsync(g.d_ticket, 0, 4, g.compute));
-            CU(cudaMemsetAsync(g.d_status, 0, (size_t)tiles * sizeof(unsigned long long), g.compute));
-            a.ticket = g.d_ticket;
-            a.tile_status = g.d_status;
+        if ((rc = prepare_tiles(sink_kind, (uint32_t)(prog->jit_cfg[r.sink].threads * prog->jit_cfg[r.sink].pts), a))) return rc;
+        e = cc_jit_launch(prog, r.sink, a, g.compute, g.index);
+        what = "specialised kernel launch";
+    } else {
+        // one CTA per 8 x 8 x 16 brick of a dense grid, or per linear tile of the hierarchy sinks' blocks
+        uint64_t units;
+        if (r.path == Path::tiles) {
+            if ((rc = prepare_tiles(sink_kind, (uint32_t)(prog->jit_cfg[r.sink].threads * prog->jit_cfg[r.sink].pts), a))) return rc;
+            units = (uint64_t)a.tiles_per_block * a.n_blocks;
+        } else {
+            units = brick_count(a.nx, a.ny, a.nz);
+            if (units >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many bricks in one launch");
         }
-        int e = cc_jit_launch(prog, sink, a, g.compute, g.index);
-        if (e) return cuda_fail((cudaError_t)e, "specialised kernel launch");
-        g.launches += 1;
-        g.points += points;
-        return CC_OK;
+        if (r.columns && (rc = prepare_columns(prog->jit_meta[r.sink], a, r.path == Path::tiles ? 0 : units))) return rc;
+        if (r.masks && (rc = prepare_part_masks(prog, a, units))) return rc;
+        if (r.path == Path::parts_interp) {
+            const uint32_t *table = nullptr;
+            if ((rc = parts_on_device(prog, &table))) return rc;
+            e = cc_launch_parts_interp(a, table, (uint32_t)units, g.compute);
+            n_launches = 2;
+        } else {
+            e = cc_jit_launch_units(prog, r.sink, a, units, g.prop.multiProcessorCount, g.compute, g.index, &n_launches);
+        }
+        what = r.path == Path::columns ? "column kernel launch" : r.path == Path::tiles ? "tile kernel launch" : "part-culling kernel launch";
     }
-    cc_launch_cfg cfg;
-    int rc = choose_cfg(prog, points, &cfg);
-    if (rc) return rc;
-    if (a.points) {  // the point-list kernels exist for 1 / 2 points per thread, constant or shared program
-        if (cfg.pts > 2) cfg.pts = 2;
-        if (cfg.prog_space == 3) cfg.prog_space = 1;
-    }
-    rc = prepare_program(prog, cfg);
-    if (rc) return rc;
-    const uint32_t tile = cc_tile_points(cfg);
-    const uint64_t cells = (uint64_t)a.nx * a.ny * a.nz;
-    a.tiles_per_block = (uint32_t)((cells + tile - 1) / tile);
-    const uint64_t tiles = (uint64_t)a.tiles_per_block * a.n_blocks;
-    if (tiles >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many tiles in one launch");
-    if (sink == CC_SINK_CLASSIFY || sink == CC_SINK_MASS) {
-        rc = ensure_status((size_t)tiles);
-        if (rc) return rc;
-        CU(cudaMemsetAsync(g.d_ticket, 0, 4, g.compute));
-        CU(cudaMemsetAsync(g.d_status, 0, (size_t)tiles * sizeof(unsigned long long), g.compute));
-        a.ticket = g.d_ticket;
-        a.tile_status = g.d_status;
-    }
-    int e = cc_launch_eval(sink_kind, cfg, a, g.compute);
-    if (e) return cuda_fail((cudaError_t)e, "cc_eval_kernel launch");
-    g.launches += 1;
+    if (e) return cuda_fail((cudaError_t)e, what);
+    g.launches += (uint64_t)n_launches;
     g.points += points;
     return CC_OK;
 }
-
 
 int init_context(Context &c, int device, int index)
 {
@@ -1051,11 +974,12 @@ int cc_grid_eval_cost_profile(const cc_program *prog, const float corner[3], flo
     if (!prog || !corner || !layer_cost) return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
     int rc = check_dims(nx, ny, nz);
     if (rc) return rc;
-    const uint32_t nbx = (nx + CC_BRICK_X - 1) / CC_BRICK_X, nby = (ny + CC_BRICK_Y - 1) / CC_BRICK_Y, nbz = (nz + CC_BRICK_Z - 1) / CC_BRICK_Z;
-    if (n_layers != nbx) return fail(CC_ERR_INVALID_ARGUMENT, "one cost per layer of 8 x-planes: n_layers must be ceil(nx / 8)");
+    if (n_layers != (nx + CC_BRICK_X - 1) / CC_BRICK_X)
+        return fail(CC_ERR_INVALID_ARGUMENT, "one cost per layer of 8 x-planes: n_layers must be ceil(nx / 8)");
     const cc_parts &parts = prog->dec.parts;
-    const uint64_t per_layer = (uint64_t)nby * nbz, nb = per_layer * nbx;
-    if (!g.parts_mode || !parts.enabled || parts.table.empty() || nb >= (1ull << 31)) {
+    const Structures can = structures_of(prog);
+    const uint64_t per_layer = brick_count(CC_BRICK_X, ny, nz), nb = per_layer * n_layers;  // (one layer: 8 x-planes)
+    if (!can.parts || parts.table.empty() || nb >= (1ull << 31)) {
         for (uint32_t i = 0; i < n_layers; ++i) layer_cost[i] = (double)per_layer;  // nothing known: every layer the same
         return CC_OK;
     }
@@ -1064,10 +988,9 @@ int cc_grid_eval_cost_profile(const cc_program *prog, const float corner[3], flo
     a.cx = corner[0]; a.cy = corner[1]; a.cz = corner[2]; a.step = step;
     a.nx = nx; a.ny = ny; a.nz = nz; a.x_offset = x_offset; a.n_blocks = 1;
     if ((rc = prepare_part_masks(prog, a, nb))) return rc;
-    int e;
-    cc_program *p = const_cast<cc_program *>(prog);
-    if (!cc_jit_is_segmented(prog->dec) && jit_ready(p, CC_SINK_PARTS)) {
-        e = cc_jit_launch_parts(prog, a, (uint32_t)nb, g.compute, g.index, true);
+    int e, n_launches;
+    if (can.parts_jit && jit_ready(const_cast<cc_program *>(prog), CC_SINK_PARTS)) {
+        e = cc_jit_launch_units(prog, CC_SINK_PARTS, a, nb, g.prop.multiProcessorCount, g.compute, g.index, &n_launches, true);
     } else {
         const uint32_t *table = nullptr;
         if ((rc = parts_on_device(prog, &table))) return rc;
@@ -1079,11 +1002,10 @@ int cc_grid_eval_cost_profile(const cc_program *prog, const float corner[3], flo
     w.base = 60.0f;
     for (int k = 0; k < 32; ++k) w.part[k] = 0.0f;
     const cc_columns &cols = prog->dec.columns;
-    const bool split = g.columns_mode && cols.enabled && !cc_jit_is_segmented(prog->dec);  // (the dense path then runs the per-cell body only)
     for (size_t v = 0; v < parts.part_of_op.size(); ++v) {
         const int part = parts.part_of_op[v];
         if (part < 0 || part >= 32) continue;
-        if (split && v < cols.phase.size() && !(cols.phase[v] & 2)) continue;
+        if (can.columns && v < cols.phase.size() && !(cols.phase[v] & 2)) continue;  // (the dense path runs the per-cell body only)
         w.part[part] += v < cols.op_cost.size() ? (float)cols.op_cost[v] : 10.0f;
     }
     double *d_cost = nullptr;
@@ -1129,13 +1051,12 @@ int cc_program_specialize_wait(cc_program *prog, unsigned sink_mask, double *com
     NEED_INIT();
     if (!prog) return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
     if ((sink_mask & CC_SINK_MASK_ALL) == 0) sink_mask = 15u;
-    // dense float4 grids of an assembly run on the part-culling kernels: "ready" includes them
-    const bool small = !cc_jit_is_segmented(prog->dec);
-    const bool parts = small && prog->dec.parts.enabled && g.parts_mode, cols = small && prog->dec.columns.enabled && g.columns_mode;
-    if ((sink_mask & (1u << CC_SINK_FLOAT4)) && parts) sink_mask |= 1u << CC_SINK_PARTS;
-    if ((sink_mask & (1u << CC_SINK_FLOAT4)) && cols) sink_mask |= 1u << CC_SINK_COLUMNS;
+    // the units that serve these sinks' launches of this program (route()): "ready" includes them
+    const Structures can = structures_of(prog);
+    if ((sink_mask & (1u << CC_SINK_FLOAT4)) && can.parts_jit) sink_mask |= 1u << CC_SINK_PARTS;
+    if ((sink_mask & (1u << CC_SINK_FLOAT4)) && can.columns) sink_mask |= 1u << CC_SINK_COLUMNS;
     for (int k : {(int)CC_SINK_PYMCUBES, (int)CC_SINK_CLASSIFY, (int)CC_SINK_MASS})
-        if ((sink_mask & (1u << k)) && (parts || cols)) sink_mask |= 1u << tile_sink_of(k);
+        if ((sink_mask & (1u << k)) && can.tiles) sink_mask |= 1u << tile_sink_of(k);
     int ready = 0;
     for (int k = 0; k < CC_N_SINKS; ++k) {
         if (!(sink_mask & (1u << k))) continue;
@@ -1522,6 +1443,19 @@ int check_levels(const cc_level *levels, uint32_t n_levels)
 
 // subdivision() on the current device for share `rank` of `world`: appends the int corners of the
 // share's leaf blocks to *out (host), in the order the levels produce them
+// Every block of every level of a hierarchy lies inside its root block: a bound on the coordinates of all of them, which
+// the tile masks' rounding budget needs.
+float root_coord_bound(const double origin[3], const cc_level *levels, double resolution)
+{
+    float m = 0.0f;
+    for (int i = 0; i < 3; ++i) {
+        const double n0 = i == 0 ? levels[0].nx : i == 1 ? levels[0].ny : levels[0].nz;
+        const double far = origin[i] + (n0 + 1.0) * (double)levels[0].cell_size * resolution;
+        m = std::max(m, (float)std::max(std::fabs(origin[i]), std::fabs(far)));
+    }
+    return m;
+}
+
 int subdivide_share(const cc_program *prog, const double origin[3], double resolution, const cc_level *levels,
                     uint32_t n_levels, int dimension, uint32_t rank, uint32_t world, std::vector<int64_t> *out,
                     uint64_t *dealt_blocks)
@@ -1537,13 +1471,7 @@ int subdivide_share(const cc_program *prog, const double origin[3], double resol
     DevBuf *cur = &corners_a, *nxt = &corners_b;
     const uint32_t deal = deal_level_subdiv(n_levels);
     if (dealt_blocks) *dealt_blocks = 0;
-    // every block of every level lies inside the root block: the bound on coordinates the tile masks' rounding budget needs
-    float coord_max = 0.0f;
-    for (int i = 0; i < 3; ++i) {
-        const double n0 = i == 0 ? levels[0].nx : i == 1 ? levels[0].ny : levels[0].nz;
-        const double far = origin[i] + (n0 + 1.0) * (double)levels[0].cell_size * resolution;
-        coord_max = std::max(coord_max, (float)std::max(std::fabs(origin[i]), std::fabs(far)));
-    }
+    const float coord_max = root_coord_bound(origin, levels, resolution);
 
     for (uint32_t l = 0; l + 1 < n_levels; ++l) {
         const cc_level &L = levels[l];
@@ -1688,12 +1616,7 @@ int mass_share(const cc_program *prog, const double box_a[3], double resolution,
     DevBuf *cur = &corners_a, *nxt = &corners_b;
     uint64_t n_cur = 1, n_launch = 0, n_cells = 0, n_blocks_total = 0, n_dealt = 0;
     const uint32_t deal = deal_level_mass(n_levels);
-    float coord_max = 0.0f;  // (as in subdivide_share)
-    for (int i = 0; i < 3; ++i) {
-        const double n0 = i == 0 ? levels[0].nx : i == 1 ? levels[0].ny : levels[0].nz;
-        const double far = box_a[i] + (n0 + 1.0) * (double)levels[0].cell_size * resolution;
-        coord_max = std::max(coord_max, (float)std::max(std::fabs(box_a[i]), std::fabs(far)));
-    }
+    const float coord_max = root_coord_bound(box_a, levels, resolution);
 
     for (uint32_t l = 0; l < n_levels && n_cur; ++l) {
         const cc_level &L = levels[l];

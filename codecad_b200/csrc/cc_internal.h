@@ -89,14 +89,23 @@ struct cc_jit_cfg {
     int segment_ops = 96;    // programs longer than ~1.5x this are cut into functions of this many micro-ops
 };
 struct cc_jit_job;
-// what the column kernels of a program need from the host (filled by the code generator)
+// what the column kernels of a program need from the host (filled by the code generator; default for a unit without them)
 struct cc_columns_meta {
     uint32_t n_values = 0;  // carried values: the column buffer holds 4 * n_values floats per column
     bool checks = false;    // some transform row is verified per column: flags, brick list and the full-walk kernel exist
-    bool centers = false;   // the program has parts: the library has its own brick-centre kernel
     int axis = 2;           // the grid axis of the columns
     bool columns = false;   // the unit has the column split (a tile unit of a program with parts only has not)
 };
+
+#define CC_AUX_CENTERS 0
+#define CC_AUX_COLUMNS 1
+#define CC_AUX_FULL 2
+
+// columns of an nx x ny x nz grid along `axis`: the cells of the plane across it
+inline uint64_t columns_along(int axis, uint32_t nx, uint32_t ny, uint32_t nz)
+{
+    return axis == 2 ? (uint64_t)nx * ny : axis == 1 ? (uint64_t)nx * nz : (uint64_t)ny * nz;
+}
 
 #define CC_MAX_DEVICES 16  // devices one process can drive (cc_init_devices)
 
@@ -109,11 +118,11 @@ struct cc_program {
     // scene-specialised kernels (cc_jit.cpp), one library per sink; null until compiled
     void *jit_library[CC_N_SINKS] = {};
     void *jit_kernel[CC_N_SINKS] = {};
-    void *jit_kernel_centers = nullptr;  // CC_SINK_PARTS: the brick-centre pass of the same library
-    void *jit_columns_kernels[3] = {};   // CC_SINK_COLUMNS: centres, profiles, full walk (jit_kernel[]: the brick kernel)
-    void *jit_tile_kernels[3][2] = {};   // CC_SINK_TILES_*: tile centres, column pass (jit_kernel[]: the tile kernel); null where not applicable
-    cc_columns_meta jit_tiles[3];        // CC_SINK_TILES_*: column buffer layout of that unit (n_values 0: no column split)
-    cc_columns_meta jit_columns;
+    // companion kernels of the same library (CC_SINK_PARTS, CC_SINK_COLUMNS, CC_SINK_TILES_*), null where a slot does not
+    // apply: [CC_AUX_CENTERS] brick / tile centres (part masks), [CC_AUX_COLUMNS] column pass, [CC_AUX_FULL] full walk of the
+    // flagged bricks
+    void *jit_aux[CC_N_SINKS][3] = {};
+    cc_columns_meta jit_meta[CC_N_SINKS];  // column buffer layout of each unit (columns false: no column split)
     cc_jit_cfg jit_cfg[CC_N_SINKS];
     size_t jit_smem[CC_N_SINKS] = {};  // dynamic shared memory of each specialised kernel
     bool jit_attr_done[CC_N_SINKS][CC_MAX_DEVICES] = {};  // MaxDynamicSharedMemorySize is a per-device attribute
@@ -135,12 +144,11 @@ int cc_jit_poll(cc_program *prog, int sink, bool wait, std::string *err);
 void cc_jit_release(cc_program *prog);
 // dev_index = index of the library context (device) the launch goes to
 int cc_jit_launch(const cc_program *prog, int sink, const cc_eval_args &a, void *stream, int dev_index);
-// part culling: the centre pass over `n_bricks` bricks, then one CTA per brick
-int cc_jit_launch_parts(const cc_program *prog, const cc_eval_args &a, uint32_t n_bricks, void *stream, int dev_index,
-                        bool centers_only = false);
-int cc_jit_launch_columns(const cc_program *prog, const cc_eval_args &a, uint32_t n_bricks, int sm_count, void *stream, int dev_index,
-                          int *n_launches);
-int cc_jit_launch_tiles(const cc_program *prog, int sink, const cc_eval_args &a, void *stream, int dev_index, int *n_launches);
+// the brick and tile units (CC_SINK_PARTS, CC_SINK_COLUMNS, CC_SINK_TILES_*) over `n_units` bricks or tiles, one CTA each:
+// [centres ->] [column pass ->] main kernel [-> full walk of the flagged bricks].  A companion runs where the unit has it and
+// the caller prepared its buffer (a.part_masks, a.columns, a.column_flags); `centers_only` stops after the centres.
+int cc_jit_launch_units(const cc_program *prog, int sink, const cc_eval_args &a, uint64_t n_units, int sm_count, void *stream,
+                        int dev_index, int *n_launches, bool centers_only = false);
 int cc_jit_launch_render(const cc_program *prog, int sink, const cc_render_args &a, void *stream, int dev_index);
 cc_jit_cfg cc_jit_render_cfg(const cc_decoded &dec);
 #define CC_SINK_MASK_ALL ((1u << CC_N_SINKS) - 1u)

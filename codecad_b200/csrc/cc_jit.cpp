@@ -666,7 +666,6 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
         if (columns_meta) {
             columns_meta->n_values = n_carried;
             columns_meta->checks = !chk.str().empty();
-            columns_meta->centers = parts_mode;
             columns_meta->axis = cols.axis;
             columns_meta->columns = true;
         }
@@ -1004,10 +1003,10 @@ void mkdirs(const std::string &d)
 
 // source for ONE sink -> cubin, through the caches.  Host-only work: safe on a background thread.
 static int build_cubin(const cc_decoded &dec, const cc_jit_cfg &cfg, int sink, Cubin *out, size_t *smem_bytes,
-                       bool *cached, std::string *err)
+                       cc_columns_meta *meta, bool *cached, std::string *err)
 {
     std::string src;
-    int rc = generate(dec, cfg, 1u << sink, &src, smem_bytes, err);
+    int rc = generate(dec, cfg, 1u << sink, &src, smem_bytes, err, meta);
     if (rc) return rc;
     const uint64_t key = source_key(src);
     if (cached) *cached = true;
@@ -1093,7 +1092,7 @@ void release_library(cudaLibrary_t lib)
 }  // namespace
 
 static int load_cubin(cc_program *prog, int sink, const Cubin &bin, const cc_jit_cfg &cfg, size_t smem_bytes,
-                      std::string *err)
+                      const cc_columns_meta &meta, std::string *err)
 {
     static const char *names[CC_N_SINKS] = {"cc_jit_float4", "cc_jit_pymcubes", "cc_jit_classify", "cc_jit_mass",
                                             "cc_jit_ray_caster", "cc_jit_bitmap", "cc_jit_points", "cc_jit_parts", "cc_jit_columns",
@@ -1127,54 +1126,33 @@ static int load_cubin(cc_program *prog, int sink, const Cubin &bin, const cc_jit
         release_library(lib);
         return CC_ERR_CUDA;
     }
-    cudaKernel_t centers = nullptr;
+    // the unit's companion kernels (cc_program::jit_aux)
+    const bool parts = prog->dec.parts.enabled;
+    const char *aux[3] = {nullptr, nullptr, nullptr};
     if (sink == CC_SINK_PARTS) {
-        ce = cudaLibraryGetKernel(&centers, lib, "cc_jit_part_centers");
-        if (ce != cudaSuccess) {
-            *err = std::string("cudaLibraryGetKernel(cc_jit_part_centers): ") + cudaGetErrorString(ce);
+        aux[CC_AUX_CENTERS] = "cc_jit_part_centers";
+    } else if (sink == CC_SINK_COLUMNS) {
+        aux[CC_AUX_CENTERS] = parts ? "cc_jit_columns_centers" : nullptr;
+        aux[CC_AUX_COLUMNS] = "cc_jit_columns_profiles";
+        aux[CC_AUX_FULL] = "cc_jit_columns_full";
+    } else if (sink == CC_SINK_TILES_PYMCUBES || sink == CC_SINK_TILES_CLASSIFY || sink == CC_SINK_TILES_MASS) {
+        aux[CC_AUX_CENTERS] = parts ? "cc_jit_tile_centers" : nullptr;
+        aux[CC_AUX_COLUMNS] = meta.columns ? "cc_jit_tile_profiles" : nullptr;
+    }
+    cudaKernel_t aux_kernel[3] = {nullptr, nullptr, nullptr};
+    for (int k = 0; k < 3; ++k)
+        if (aux[k] && (ce = cudaLibraryGetKernel(&aux_kernel[k], lib, aux[k])) != cudaSuccess) {
+            *err = std::string("cudaLibraryGetKernel(") + aux[k] + "): " + cudaGetErrorString(ce);
             release_library(lib);
             return CC_ERR_CUDA;
         }
-        prog->jit_kernel_centers = (void *)centers;
-    }
-    const bool tile_unit = sink == CC_SINK_TILES_PYMCUBES || sink == CC_SINK_TILES_CLASSIFY || sink == CC_SINK_TILES_MASS;
-    if (sink == CC_SINK_COLUMNS || tile_unit) {
-        // what the kernels need from the host: the generator's own bookkeeping (a second, source-only pass)
-        std::string src;
-        size_t sm = 0;
-        cc_columns_meta meta;
-        meta.centers = prog->dec.parts.enabled;
-        if (generate(prog->dec, cfg, 1u << sink, &src, &sm, err, &meta) != CC_OK) {
-            release_library(lib);
-            return CC_ERR_CUDA;
-        }
-        const char *extra[3] = {nullptr, nullptr, nullptr};
-        if (tile_unit) {
-            extra[0] = prog->dec.parts.enabled ? "cc_jit_tile_centers" : nullptr;
-            extra[1] = meta.columns ? "cc_jit_tile_profiles" : nullptr;
-        } else {
-            extra[0] = meta.centers ? "cc_jit_columns_centers" : nullptr;
-            extra[1] = "cc_jit_columns_profiles";
-            extra[2] = "cc_jit_columns_full";
-        }
-        void **dst = tile_unit ? prog->jit_tile_kernels[sink - CC_SINK_TILES_PYMCUBES] : prog->jit_columns_kernels;
-        for (int k = 0; k < (tile_unit ? 2 : 3); ++k) {
-            cudaKernel_t kk = nullptr;
-            if (extra[k] && (ce = cudaLibraryGetKernel(&kk, lib, extra[k])) != cudaSuccess) {
-                *err = std::string("cudaLibraryGetKernel(") + extra[k] + "): " + cudaGetErrorString(ce);
-                release_library(lib);
-                return CC_ERR_CUDA;
-            }
-            dst[k] = (void *)kk;
-        }
-        if (tile_unit) prog->jit_tiles[sink - CC_SINK_TILES_PYMCUBES] = meta;
-        else prog->jit_columns = meta;
-    }
     if (prog->jit_library[sink]) release_library((cudaLibrary_t)prog->jit_library[sink]);
     prog->jit_smem[sink] = smem_bytes;
     for (int d = 0; d < CC_MAX_DEVICES; ++d) prog->jit_attr_done[sink][d] = false;
     prog->jit_library[sink] = (void *)lib;
     prog->jit_kernel[sink] = (void *)kern;
+    for (int k = 0; k < 3; ++k) prog->jit_aux[sink][k] = (void *)aux_kernel[k];
+    prog->jit_meta[sink] = meta;
     prog->jit_cfg[sink] = cfg;
     prog->jit_cubin_bytes += bin->size();
     return CC_OK;
@@ -1188,6 +1166,7 @@ struct cc_jit_job {
     Cubin bin;
     cc_jit_cfg cfg;
     size_t smem = 0;
+    cc_columns_meta meta;
     std::string err;
     double seconds = 0;
     bool cached = false;
@@ -1248,8 +1227,9 @@ int cc_jit_compile(cc_program *prog, int pts, unsigned sink_mask, double *second
         const cc_jit_cfg cfg = cc_jit_cfg_for(prog->dec, k, pts);
         Cubin bin;
         size_t smem = 0;
-        int rc = build_cubin(prog->dec, cfg, k, &bin, &smem, nullptr, err);
-        if (rc == CC_OK) rc = load_cubin(prog, k, bin, cfg, smem, err);
+        cc_columns_meta meta;
+        int rc = build_cubin(prog->dec, cfg, k, &bin, &smem, &meta, nullptr, err);
+        if (rc == CC_OK) rc = load_cubin(prog, k, bin, cfg, smem, meta, err);
         if (rc) return rc;
     }
     prog->use_jit = true;
@@ -1267,7 +1247,7 @@ void cc_jit_start(cc_program *prog, int sink)
     const cc_decoded *dec = &prog->dec;  // immutable; outlives the thread (destroy joins it)
     j->th = std::thread([j, dec, sink]() {
         auto t0 = std::chrono::steady_clock::now();
-        j->rc = build_cubin(*dec, j->cfg, sink, &j->bin, &j->smem, &j->cached, &j->err);
+        j->rc = build_cubin(*dec, j->cfg, sink, &j->bin, &j->smem, &j->meta, &j->cached, &j->err);
         j->seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         j->done.store(1, std::memory_order_release);
     });
@@ -1284,7 +1264,7 @@ int cc_jit_poll(cc_program *prog, int sink, bool wait, std::string *err)
     if (!wait && !j->done.load(std::memory_order_acquire)) return 0;
     if (j->th.joinable()) j->th.join();
     int rc = j->rc;
-    if (rc == CC_OK) rc = load_cubin(prog, sink, j->bin, j->cfg, j->smem, &j->err);
+    if (rc == CC_OK) rc = load_cubin(prog, sink, j->bin, j->cfg, j->smem, j->meta, &j->err);
     prog->jit_seconds += j->seconds;
     if (rc != CC_OK) {
         if (err) *err = j->err;
@@ -1306,14 +1286,17 @@ void cc_jit_release(cc_program *prog)
     prog->jit_cubin_bytes = 0;
 }
 
-// MaxDynamicSharedMemorySize is kept per device: set it the first time a device launches the kernel
+// MaxDynamicSharedMemorySize is kept per device: set it the first time a device launches the kernel (the companion
+// kernels share the value cells' layout, hence the size)
 static int ensure_smem_attr(const cc_program *prog, int sink, int dev_index)
 {
     cc_program *p = const_cast<cc_program *>(prog);
     if (p->jit_attr_done[sink][dev_index] || p->jit_smem[sink] == 0) return 0;
-    cudaError_t ce = cudaFuncSetAttribute((const void *)p->jit_kernel[sink], cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)p->jit_smem[sink]);
-    if (ce != cudaSuccess) return (int)ce;
+    for (void *k : {p->jit_kernel[sink], p->jit_aux[sink][0], p->jit_aux[sink][1], p->jit_aux[sink][2]})
+        if (k) {
+            cudaError_t ce = cudaFuncSetAttribute((const void *)k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p->jit_smem[sink]);
+            if (ce != cudaSuccess) return (int)ce;
+        }
     p->jit_attr_done[sink][dev_index] = true;
     return 0;
 }
@@ -1328,100 +1311,33 @@ int cc_jit_launch(const cc_program *prog, int sink, const cc_eval_args &a, void 
                                  args, prog->jit_smem[sink], (cudaStream_t)stream);
 }
 
-int cc_jit_launch_parts(const cc_program *prog, const cc_eval_args &a, uint32_t n_bricks, void *stream, int dev_index, bool centers_only)
+int cc_jit_launch_units(const cc_program *prog, int sink, const cc_eval_args &a, uint64_t n_units, int sm_count, void *stream,
+                        int dev_index, int *n_launches, bool centers_only)
 {
-    if (n_bricks == 0) return 0;
-    const int sink = CC_SINK_PARTS;
-    if (int e = ensure_smem_attr(prog, sink, dev_index)) return e;
-    const size_t smem = prog->jit_smem[sink];
-    if (smem) {  // the centre pass shares the value cells' layout (per device, like the main kernel's attribute)
-        cudaError_t ce = cudaFuncSetAttribute((const void *)prog->jit_kernel_centers, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (ce != cudaSuccess) return (int)ce;
-    }
-    const uint32_t threads = (uint32_t)prog->jit_cfg[sink].threads;
-    void *args[] = {(void *)&a};
-    cudaError_t ce = cudaLaunchKernel((const void *)prog->jit_kernel_centers, dim3((n_bricks + 2 * threads - 1) / (2 * threads)),
-                                      dim3(threads), args, smem, (cudaStream_t)stream);
-    if (ce != cudaSuccess || centers_only) return (int)ce;
-    return (int)cudaLaunchKernel((const void *)prog->jit_kernel[sink], dim3(n_bricks), dim3(threads), args, smem,
-                                 (cudaStream_t)stream);
-}
-
-// The hierarchy sinks (blocks x linear tiles) through their tile unit (CC_SINK_TILES_*): [tile centres ->] [column pass
-// over every block's columns ->] tile kernel.  The caller prepared tickets and tile status like cc_jit_launch,
-// a.part_masks (or null) and a.columns / a.column_flags (or null).
-int cc_jit_launch_tiles(const cc_program *prog, int sink, const cc_eval_args &a, void *stream, int dev_index, int *n_launches)
-{
-    const size_t smem = prog->jit_smem[sink];
-    if (int e = ensure_smem_attr(prog, sink, dev_index)) return e;
-    void *const *extra = prog->jit_tile_kernels[sink - CC_SINK_TILES_PYMCUBES];
-    if (smem)
-        for (int k = 0; k < 2; ++k)
-            if (extra[k]) {
-                cudaError_t ce = cudaFuncSetAttribute((const void *)extra[k], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (ce != cudaSuccess) return (int)ce;
-            }
-    const uint32_t threads = (uint32_t)prog->jit_cfg[sink].threads;
-    const uint64_t tiles = (uint64_t)a.tiles_per_block * a.n_blocks;
     *n_launches = 0;
-    if (tiles == 0) return 0;
-    void *args[] = {(void *)&a};
-    cudaError_t ce = cudaSuccess;
-    if (a.part_masks) {
-        ce = cudaLaunchKernel((const void *)extra[0], dim3((unsigned)((tiles + 2 * threads - 1) / (2 * threads))), dim3(threads), args, smem,
-                              (cudaStream_t)stream);
-        if (ce != cudaSuccess) return (int)ce;
-        ++*n_launches;
-    }
-    if (a.columns) {
-        const int axis = prog->jit_tiles[sink - CC_SINK_TILES_PYMCUBES].axis;
-        const uint64_t ncol = (uint64_t)std::max(1u, a.n_blocks) * (axis == 2 ? (uint64_t)a.nx * a.ny : axis == 1 ? (uint64_t)a.nx * a.nz : (uint64_t)a.ny * a.nz);
-        ce = cudaLaunchKernel((const void *)extra[1], dim3((unsigned)((ncol + 2 * threads - 1) / (2 * threads))), dim3(threads), args, smem,
-                              (cudaStream_t)stream);
-        if (ce != cudaSuccess) return (int)ce;
-        ++*n_launches;
-    }
-    ++*n_launches;
-    return (int)cudaLaunchKernel((const void *)prog->jit_kernel[sink], dim3((unsigned)tiles), dim3(threads), args, smem, (cudaStream_t)stream);
-}
-
-// CC_SINK_COLUMNS: [brick centres ->] column pass -> brick kernel [-> full walk of the flagged bricks]; the caller
-// prepared a.columns (and a.part_masks / a.column_flags + a.brick_list + a.brick_count as the program needs)
-int cc_jit_launch_columns(const cc_program *prog, const cc_eval_args &a, uint32_t n_bricks, int sm_count, void *stream, int dev_index,
-                          int *n_launches)
-{
-    if (n_bricks == 0) return 0;
-    const int sink = CC_SINK_COLUMNS;
-    const size_t smem = prog->jit_smem[sink];
+    if (n_units == 0) return 0;
     if (int e = ensure_smem_attr(prog, sink, dev_index)) return e;
-    if (smem)
-        for (void *k : prog->jit_columns_kernels)
-            if (k) {
-                cudaError_t ce = cudaFuncSetAttribute((const void *)k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (ce != cudaSuccess) return (int)ce;
-            }
+    void *const *aux = prog->jit_aux[sink];
     const uint32_t threads = (uint32_t)prog->jit_cfg[sink].threads;
-    cudaStream_t st = (cudaStream_t)stream;
+    const size_t smem = prog->jit_smem[sink];
     void *args[] = {(void *)&a};
-    cudaError_t ce = cudaSuccess;
-    *n_launches = 0;
-    if (a.part_masks) {
-        ce = cudaLaunchKernel((const void *)prog->jit_columns_kernels[0], dim3((n_bricks + 2 * threads - 1) / (2 * threads)), dim3(threads), args, smem, st);
-        if (ce != cudaSuccess) return (int)ce;
+    auto run = [&](const void *kernel, uint64_t grid) {
         ++*n_launches;
+        return cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(threads), args, smem, (cudaStream_t)stream);
+    };
+    // the centres and the column pass take two bricks / tiles / columns per thread (one packed pair)
+    const uint64_t pair = 2 * threads;
+    cudaError_t ce;
+    if (aux[CC_AUX_CENTERS] && a.part_masks) {
+        if ((ce = run(aux[CC_AUX_CENTERS], (n_units + pair - 1) / pair)) != cudaSuccess || centers_only) return (int)ce;
     }
-    const uint32_t ncol = prog->jit_columns.axis == 2 ? a.nx * a.ny : prog->jit_columns.axis == 1 ? a.nx * a.nz : a.ny * a.nz;
-    ce = cudaLaunchKernel((const void *)prog->jit_columns_kernels[1], dim3((ncol + 2 * threads - 1) / (2 * threads)), dim3(threads), args, smem, st);
-    if (ce != cudaSuccess) return (int)ce;
-    ce = cudaLaunchKernel((const void *)prog->jit_kernel[sink], dim3(n_bricks), dim3(threads), args, smem, st);
-    if (ce != cudaSuccess) return (int)ce;
-    *n_launches += 2;
-    if (a.column_flags) {
-        ce = cudaLaunchKernel((const void *)prog->jit_columns_kernels[2], dim3((unsigned)std::max(1, 2 * sm_count)), dim3(threads), args, smem, st);
-        if (ce != cudaSuccess) return (int)ce;
-        ++*n_launches;
+    if (aux[CC_AUX_COLUMNS] && a.columns) {
+        const uint64_t ncol = std::max(1u, a.n_blocks) * columns_along(prog->jit_meta[sink].axis, a.nx, a.ny, a.nz);
+        if ((ce = run(aux[CC_AUX_COLUMNS], (ncol + pair - 1) / pair)) != cudaSuccess) return (int)ce;
     }
-    return 0;
+    if ((ce = run(prog->jit_kernel[sink], n_units)) != cudaSuccess) return (int)ce;
+    if (aux[CC_AUX_FULL] && a.column_flags) ce = run(aux[CC_AUX_FULL], (uint64_t)std::max(1, 2 * sm_count));
+    return (int)ce;
 }
 
 int cc_jit_source(const cc_decoded &dec, int pts, unsigned sink_mask, std::string *src, std::string *err)
