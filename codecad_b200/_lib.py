@@ -111,6 +111,11 @@ SIGNATURES = {
     "cc_mesh_blocks": (_I, [_V, ctypes.POINTER(ctypes.c_double), ctypes.c_double, _U, _U, _U, _U,
                             ctypes.POINTER(ctypes.POINTER(ctypes.c_double)),
                             ctypes.POINTER(ctypes.POINTER(ctypes.c_uint32)), ctypes.POINTER(ctypes.c_uint64)]),
+    "cc_mesh_blocks_indexed": (_I, [_V, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int64), ctypes.c_double,
+                                    _U, _U, _U, _U,
+                                    ctypes.POINTER(ctypes.POINTER(ctypes.c_double)), ctypes.POINTER(ctypes.c_uint64),
+                                    ctypes.POINTER(ctypes.POINTER(ctypes.c_uint32)),
+                                    ctypes.POINTER(ctypes.POINTER(ctypes.c_uint32)), ctypes.POINTER(ctypes.c_uint64)]),
     "cc_free": (None, [_V]),
 }
 

@@ -1408,6 +1408,12 @@ struct DevBuf {
         cap = bytes;
         return CC_OK;
     }
+    void release()
+    {
+        if (p) cudaFreeAsync(p, g.compute);
+        p = nullptr;
+        cap = 0;
+    }
     template <class T> T *as() { return static_cast<T *>(p); }
 };
 
@@ -2159,49 +2165,65 @@ int cc_polygon_blocks(const cc_program *prog, const double *corners, double reso
     return CC_OK;
 }
 
-int cc_mesh_blocks(const cc_program *prog, const double *corners, double resolution, uint32_t nx, uint32_t ny,
-                   uint32_t nz, uint32_t n_blocks, double **out_vertices, uint32_t **out_triangle_block,
-                   uint64_t *out_triangles)
+}  // extern "C"
+
+// ---- mesh export: the triangle soup and the welded mesh share the chunks, the page-locked results
+// and the copy stream ----------------------------------------------------------------------------
+
+namespace {
+// One chunk of the blocks of a mesh export, with what lives on the device from its phase A to its
+// phase B.
+struct MeshChunk {
+    uint32_t b0 = 0, nb = 0, n_tri = 0, n_tiles = 0, n_vert = 0;
+    uint64_t vert_base = 0;  // vertices of the earlier chunks
+    DevBuf field, descs, corner, scratch, vbase, vmask;
+    DevBuf out[3];           // the chunk's rows of the outputs, in MeshPass::outputs order
+    cc_mesh_args m;
+};
+
+// What an export does on top of the shared evaluation, triangle count and copy-back.
+struct MeshPass {
+    uint32_t sample_bytes;  // device bytes per sample kept from phase A to phase B
+    struct Output {
+        size_t row_bytes;
+        bool per_vertex;    // one row per vertex (counter[2]) rather than per triangle
+    };
+    std::vector<Output> outputs;
+    std::function<int(MeshChunk &)> before_count;  // phase A, after the evaluation (optional)
+    std::function<int(MeshChunk &)> emit;          // phase B: fill c.out[*]
+};
+
+// Phase A per chunk of blocks: evaluate the field, pass.before_count, count triangles per tile, scan.
+// Phase B per chunk: pass.emit.  When every chunk's samples fit the budget at once (the usual case),
+// all of phase A runs first, the page-locked results are sized from the totals, and each chunk's rows
+// start crossing PCIe on the copy stream as soon as its emit pass is done, while the next chunk emits.
+// Larger meshes keep one field buffer, run A + B chunk by chunk and copy at the end.  Either way the
+// chunks run in input order.  out_host[k] receives output k (page-locked, released with cc_free);
+// out_rows = {triangles, vertices}.
+int mesh_chunks(const cc_program *prog, const double *corners, double resolution, uint32_t nx, uint32_t ny, uint32_t nz,
+                uint32_t n_blocks, const MeshPass &pass, void **out_host, uint64_t out_rows[2])
 {
-    NEED_INIT();
-    if (!prog || !corners || !out_vertices || !out_triangle_block || !out_triangles)
-        return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
-    if (nx < 2 || ny < 2 || nz < 2) return fail(CC_ERR_INVALID_ARGUMENT, "marching cubes needs at least 2 samples per axis");
     const uint64_t cells = (uint64_t)nx * ny * nz;
-    if (cells > (1ull << 30)) return fail(CC_ERR_INVALID_ARGUMENT, "block too large");
-    *out_vertices = nullptr;
-    *out_triangle_block = nullptr;
-    *out_triangles = 0;
-    if (n_blocks == 0) return CC_OK;
     if (!g.mesh_tables) {  // __constant__ tables are per device (and gone after cc_shutdown)
         int e = cc_mesh_upload_tables(g.compute);
         if (e) return cuda_fail((cudaError_t)e, "marching-cubes tables");
         g.mesh_tables = true;
     }
-    // Phase A per chunk of blocks: evaluate the field, count triangles per tile, scan.  Phase B per
-    // chunk: emit the triangles.  When every chunk's field fits the budget at once (the usual
-    // case), all of phase A runs first, the page-locked result is sized from the totals, and each
-    // chunk's triangles start crossing PCIe on the copy stream as soon as its emit pass is done,
-    // while the next chunk emits.  Larger meshes keep one field buffer, run A + B chunk by chunk
-    // and copy at the end.
-    struct Chunk {
-        uint32_t b0 = 0, nb = 0, n_tri = 0, n_tiles = 0;
-        DevBuf field, descs, corner, scratch, vertices, tri_block;
-        cc_mesh_args m;
-    };
+    using Chunk = MeshChunk;
     // (both sizes can be overridden for tests: CODECAD_B200_MESH_FIELD_BUDGET / _MESH_CHUNK_BYTES)
     uint64_t field_budget = 4ull << 30;
     if (const char *t = getenv("CODECAD_B200_MESH_FIELD_BUDGET")) field_budget = strtoull(t, nullptr, 10);
-    const bool resident = (uint64_t)n_blocks * cells * 4 <= field_budget;
-    // blocks per chunk: ~256 MiB of field when the copies are pipelined (several chunks to overlap),
+    const bool resident = (uint64_t)n_blocks * cells * pass.sample_bytes <= field_budget;
+    // blocks per chunk: ~256 MiB of samples when the copies are pipelined (several chunks to overlap),
     // ~1 GiB otherwise
     uint64_t chunk_bytes = resident ? (1ull << 28) : (1ull << 30);
     if (const char *t = getenv("CODECAD_B200_MESH_CHUNK_BYTES")) chunk_bytes = std::max<uint64_t>(1, strtoull(t, nullptr, 10));
-    const uint32_t chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(n_blocks, chunk_bytes / (cells * 4)));
+    const uint32_t chunk = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(n_blocks, chunk_bytes / (cells * pass.sample_bytes)));
     std::vector<std::unique_ptr<Chunk>> chunks;
     DevBuf counter, shared_field;
     int rc;
-    if ((rc = counter.reserve(8))) return rc;
+    if ((rc = counter.reserve(16))) return rc;
+    CU(cudaMemsetAsync(counter.p, 0, 16, g.compute));
     if (!resident && (rc = shared_field.reserve((size_t)chunk * cells * 4))) return rc;
     std::vector<cc_block_desc> h_desc(chunk);
     const float step = (float)resolution;  // numpy.float32(box_resolution), rendering/mesh.py:58
@@ -2247,49 +2269,61 @@ int cc_mesh_blocks(const cc_program *prog, const double *corners, double resolut
         if ((rc2 = c.scratch.reserve(words * 4))) return rc2;
         m.tile_offsets = c.scratch.as<uint32_t>();
         m.tile_list = m.tile_offsets + (words - tiles);
+        if (pass.before_count && (rc2 = pass.before_count(c))) return rc2;
         int e = cc_launch_mesh(m, false, 0, g.compute);  // count per tile + scan + list of non-empty tiles
         if (e) return cuda_fail((cudaError_t)e, "marching cubes (count)");
         g.launches += 4;
-        uint32_t h2[2] = {0, 0};
-        CU(cudaMemcpyAsync(h2, counter.p, 8, cudaMemcpyDeviceToHost, g.compute));
+        uint32_t h4[4] = {0, 0, 0, 0};
+        CU(cudaMemcpyAsync(h4, counter.p, 16, cudaMemcpyDeviceToHost, g.compute));
         CU(cudaStreamSynchronize(g.compute));  // also: h_desc is reused by the next chunk
-        c.n_tri = h2[0];
-        c.n_tiles = h2[1];
+        c.n_tri = h4[0];
+        c.n_tiles = h4[1];
+        c.n_vert = h4[2];
         return CC_OK;
     };
     auto phase_b = [&](Chunk &c) -> int {
         if (c.n_tri == 0) return CC_OK;
         int rc2;
-        if ((rc2 = c.vertices.reserve((size_t)c.n_tri * 9 * sizeof(double)))) return rc2;
-        if ((rc2 = c.tri_block.reserve((size_t)c.n_tri * 4))) return rc2;
-        c.m.vertices = c.vertices.as<double>();
-        c.m.tri_block = c.tri_block.as<uint32_t>();
-        int e = cc_launch_mesh(c.m, true, c.n_tiles, g.compute);
-        if (e) return cuda_fail((cudaError_t)e, "marching cubes (emit)");
-        g.launches += 1;
+        for (size_t k = 0; k < pass.outputs.size(); ++k) {
+            const auto &o = pass.outputs[k];
+            if ((rc2 = c.out[k].reserve((size_t)(o.per_vertex ? c.n_vert : c.n_tri) * o.row_bytes))) return rc2;
+        }
+        if ((rc2 = pass.emit(c))) return rc2;
+        c.vbase.release();  // the per-sample buffers of the indexed export
+        c.vmask.release();
         return CC_OK;
     };
 
+    uint64_t rows[2] = {0, 0};
     for (uint32_t b0 = 0; b0 < n_blocks; b0 += chunk) {
         chunks.emplace_back(new Chunk);
         Chunk &c = *chunks.back();
         c.b0 = b0;
         c.nb = std::min(chunk, n_blocks - b0);
+        c.vert_base = rows[1];
         if ((rc = phase_a(c))) return rc;
+        rows[0] += c.n_tri;
+        rows[1] += c.n_vert;
+        if (rows[1] > 0xFFFFFFFFull) return fail(CC_ERR_TOO_LARGE, "more than 2^32 - 1 vertices");
         if (!resident && (rc = phase_b(c))) return rc;  // the shared field is overwritten by the next chunk
     }
-    size_t n = 0;
-    for (auto &c : chunks) n += c->n_tri;
-    *out_triangles = n;
-    if (n == 0) return CC_OK;
-    double *v = (double *)g_pinned.get(n * 9 * sizeof(double));  // page-locked: the copy runs at PCIe speed
-    uint32_t *b = (uint32_t *)g_pinned.get(n * sizeof(uint32_t));
-    if (!v || !b) {
-        cc_free(v);
-        cc_free(b);
+    out_rows[0] = rows[0];
+    out_rows[1] = rows[1];
+    if (rows[0] == 0) return CC_OK;
+    std::vector<char *> host(pass.outputs.size(), nullptr);
+    bool ok = true;
+    for (size_t k = 0; k < host.size(); ++k) {  // page-locked: the copy runs at PCIe speed
+        host[k] = (char *)g_pinned.get(rows[pass.outputs[k].per_vertex ? 1 : 0] * pass.outputs[k].row_bytes);
+        ok = ok && host[k];
+    }
+    auto release = [&]() {
+        for (char *h : host) cc_free(h);
+    };
+    if (!ok) {
+        release();
         return fail(CC_ERR_INVALID_ARGUMENT, "out of host memory");
     }
-    size_t at = 0;
+    uint64_t at[2] = {0, 0};
     cudaError_t ce = cudaSuccess;
     rc = CC_OK;
     cudaEvent_t emitted = nullptr;
@@ -2302,25 +2336,178 @@ int cc_mesh_blocks(const cc_program *prog, const double *corners, double resolut
             if ((rc = phase_b(c))) break;
             ce = cudaEventRecord(emitted, g.compute);
             if (ce == cudaSuccess) ce = cudaStreamWaitEvent(g.copy, emitted, 0);
-            copy_on = g.copy;  // this chunk's triangles cross PCIe while the next chunk emits
+            copy_on = g.copy;  // this chunk's rows cross PCIe while the next chunk emits
         }
-        if (ce == cudaSuccess)
-            ce = cudaMemcpyAsync(v + at * 9, c.vertices.p, (size_t)c.n_tri * 9 * sizeof(double), cudaMemcpyDeviceToHost, copy_on);
-        if (ce == cudaSuccess)
-            ce = cudaMemcpyAsync(b + at, c.tri_block.p, (size_t)c.n_tri * 4, cudaMemcpyDeviceToHost, copy_on);
-        at += c.n_tri;
+        for (size_t k = 0; k < host.size() && ce == cudaSuccess; ++k) {
+            const auto &o = pass.outputs[k];
+            const uint64_t r = o.per_vertex ? c.n_vert : c.n_tri;
+            ce = cudaMemcpyAsync(host[k] + at[o.per_vertex] * o.row_bytes, c.out[k].p, r * o.row_bytes, cudaMemcpyDeviceToHost, copy_on);
+        }
+        at[0] += c.n_tri;
+        at[1] += c.n_vert;
     }
     if (ce == cudaSuccess) ce = cudaStreamSynchronize(g.compute);
     cudaError_t ce2 = cudaStreamSynchronize(g.copy);  // before the chunks' device buffers are released
     if (ce == cudaSuccess) ce = ce2;
     if (emitted) cudaEventDestroy(emitted);
     if (rc != CC_OK || ce != cudaSuccess) {
-        cc_free(v);
-        cc_free(b);
-        return rc != CC_OK ? rc : cuda_fail(ce, "triangles D2H");
+        release();
+        return rc != CC_OK ? rc : cuda_fail(ce, "mesh D2H");
     }
-    *out_vertices = v;
-    *out_triangle_block = b;
+    for (size_t k = 0; k < host.size(); ++k) out_host[k] = host[k];
+    return CC_OK;
+}
+
+// Leaf-block checks shared by the two entry points.
+int mesh_args_ok(const cc_program *prog, const double *corners, uint32_t nx, uint32_t ny, uint32_t nz)
+{
+    if (!prog || !corners) return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
+    if (nx < 2 || ny < 2 || nz < 2) return fail(CC_ERR_INVALID_ARGUMENT, "marching cubes needs at least 2 samples per axis");
+    if ((uint64_t)nx * ny * nz > (1ull << 30)) return fail(CC_ERR_INVALID_ARGUMENT, "block too large");
+    return CC_OK;
+}
+
+constexpr int kKeyBits = 21;  // CC_KEY_BITS in cc_mesh.cu
+}  // namespace
+
+extern "C" {
+
+int cc_mesh_blocks(const cc_program *prog, const double *corners, double resolution, uint32_t nx, uint32_t ny,
+                   uint32_t nz, uint32_t n_blocks, double **out_vertices, uint32_t **out_triangle_block,
+                   uint64_t *out_triangles)
+{
+    NEED_INIT();
+    if (!out_vertices || !out_triangle_block || !out_triangles) return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
+    int rc = mesh_args_ok(prog, corners, nx, ny, nz);
+    if (rc) return rc;
+    *out_vertices = nullptr;
+    *out_triangle_block = nullptr;
+    *out_triangles = 0;
+    if (n_blocks == 0) return CC_OK;
+    auto emit = [](MeshChunk &c) -> int {
+        c.m.vertices = c.out[0].as<double>();
+        c.m.tri_block = c.out[1].as<uint32_t>();
+        int e = cc_launch_mesh(c.m, true, c.n_tiles, g.compute);
+        if (e) return cuda_fail((cudaError_t)e, "marching cubes (emit)");
+        g.launches += 1;
+        return CC_OK;
+    };
+    const MeshPass pass{4, {{9 * sizeof(double), false}, {4, false}}, nullptr, emit};  // keeps the field
+    void *host[2] = {nullptr, nullptr};
+    uint64_t rows[2] = {0, 0};
+    if ((rc = mesh_chunks(prog, corners, resolution, nx, ny, nz, n_blocks, pass, host, rows))) return rc;
+    *out_vertices = (double *)host[0];
+    *out_triangle_block = (uint32_t *)host[1];
+    *out_triangles = rows[0];
+    return CC_OK;
+}
+
+int cc_mesh_blocks_indexed(const cc_program *prog, const double *corners, const int64_t *int_corners, double resolution,
+                           uint32_t nx, uint32_t ny, uint32_t nz, uint32_t n_blocks, double **out_vertices,
+                           uint64_t *out_n_vertices, uint32_t **out_triangles, uint32_t **out_triangle_block,
+                           uint64_t *out_n_triangles)
+{
+    NEED_INIT();
+    if (!int_corners || !out_vertices || !out_n_vertices || !out_triangles || !out_triangle_block || !out_n_triangles)
+        return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
+    int rc = mesh_args_ok(prog, corners, nx, ny, nz);
+    if (rc) return rc;
+    *out_vertices = nullptr;
+    *out_triangles = nullptr;
+    *out_triangle_block = nullptr;
+    *out_n_vertices = *out_n_triangles = 0;
+    if (n_blocks == 0) return CC_OK;
+    if (n_blocks > 1 && !(nx == ny && ny == nz)) return fail(CC_ERR_INVALID_ARGUMENT, "several blocks must be cubic");
+
+    // Block table: block coordinates (int corner - first int corner) / (n - 1) in array axes
+    // (i = -y, j = x, k = z), shifted to start at 0 and packed 21 bits each.
+    std::vector<uint64_t> key(n_blocks, 0);
+    if (n_blocks > 1) {
+        const int64_t step = nx - 1, limit = 1ll << 60;
+        std::vector<int64_t> q(3 * (size_t)n_blocks);
+        int64_t lo[3] = {INT64_MAX, INT64_MAX, INT64_MAX}, hi[3] = {INT64_MIN, INT64_MIN, INT64_MIN};
+        for (uint32_t b = 0; b < n_blocks; ++b)
+            for (int ax = 0; ax < 3; ++ax) {
+                const int64_t c = int_corners[3 * (size_t)b + ax], c0 = int_corners[ax];
+                if (c <= -limit || c >= limit) return fail(CC_ERR_INVALID_ARGUMENT, "int corner too wide");
+                if ((c - c0) % step) return fail(CC_ERR_INVALID_ARGUMENT, "int corners are not on one lattice of n - 1");
+                const int64_t v = (c - c0) / step;
+                const int arr = ax == 0 ? 1 : ax == 1 ? 0 : 2;  // x -> j, y -> i (reversed), z -> k
+                const int64_t w = ax == 1 ? -v : v;
+                q[3 * (size_t)b + arr] = w;
+                lo[arr] = std::min(lo[arr], w);
+                hi[arr] = std::max(hi[arr], w);
+            }
+        for (int ax = 0; ax < 3; ++ax)
+            if (hi[ax] - lo[ax] >= (1ll << kKeyBits) - 1) return fail(CC_ERR_INVALID_ARGUMENT, "blocks span too many block widths for the block table");
+        for (uint32_t b = 0; b < n_blocks; ++b)
+            for (int ax = 0; ax < 3; ++ax) key[b] = (key[b] << kKeyBits) | (uint64_t)(q[3 * (size_t)b + ax] - lo[ax]);
+    }
+    std::vector<uint32_t> order(n_blocks);
+    for (uint32_t b = 0; b < n_blocks; ++b) order[b] = b;
+    std::sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return key[x] < key[y]; });
+    std::vector<uint64_t> sorted_key(n_blocks);
+    for (uint32_t r = 0; r < n_blocks; ++r) {
+        sorted_key[r] = key[order[r]];
+        if (r && sorted_key[r] == sorted_key[r - 1]) return fail(CC_ERR_INVALID_ARGUMENT, "two blocks have the same int corner");
+    }
+    const uint32_t nf = std::max(nx, std::max(ny, nz));
+    const size_t face_samples = (size_t)n_blocks * 6 * nf * nf;
+    DevBuf d_key, d_sorted_key, d_sorted_block, face_field, face_vertex;
+    if ((rc = d_key.reserve((size_t)n_blocks * 8)) || (rc = d_sorted_key.reserve((size_t)n_blocks * 8)) ||
+        (rc = d_sorted_block.reserve((size_t)n_blocks * 4)) || (rc = face_field.reserve(face_samples * 4)) ||
+        (rc = face_vertex.reserve(face_samples * 8)))
+        return rc;
+    CU(cudaMemcpyAsync(d_key.p, key.data(), (size_t)n_blocks * 8, cudaMemcpyHostToDevice, g.compute));
+    CU(cudaMemcpyAsync(d_sorted_key.p, sorted_key.data(), (size_t)n_blocks * 8, cudaMemcpyHostToDevice, g.compute));
+    CU(cudaMemcpyAsync(d_sorted_block.p, order.data(), (size_t)n_blocks * 4, cudaMemcpyHostToDevice, g.compute));
+
+    const size_t cells = (size_t)nx * ny * nz;
+    auto reconcile = [&](MeshChunk &c) -> int {
+        cc_mesh_args &m = c.m;
+        m.block_key = d_key.as<uint64_t>();
+        m.sorted_key = d_sorted_key.as<uint64_t>();
+        m.sorted_block = d_sorted_block.as<uint32_t>();
+        m.n_all = n_blocks;
+        m.nf = nf;
+        m.face_field = face_field.as<float>();
+        m.face_vertex = face_vertex.as<uint32_t>();
+        const size_t samples = (size_t)c.nb * cells;
+        if (samples >= (1ull << 32)) return fail(CC_ERR_INVALID_ARGUMENT, "too many samples in one chunk");
+        DevBuf scan;  // released (stream-ordered) when the chunk's vertex offsets are done
+        int rc2;
+        if ((rc2 = c.vbase.reserve(samples * 4)) || (rc2 = c.vmask.reserve(samples)) ||
+            (rc2 = scan.reserve((cc_mesh_scan_scratch_words((uint32_t)samples) + samples) * 4)))
+            return rc2;
+        m.vbase = c.vbase.as<uint32_t>();
+        m.vmask = c.vmask.as<uint8_t>();
+        int e = cc_launch_mesh_reconcile(m, g.compute);
+        if (!e) e = cc_launch_mesh_scan(m.vbase, (uint32_t)samples, scan.as<uint32_t>() + samples, scan.as<uint32_t>(),
+                                        m.counter + 2, g.compute);
+        if (e) return cuda_fail((cudaError_t)e, "marching cubes (shared samples, vertex count)");
+        g.launches += 6;
+        return CC_OK;
+    };
+    auto emit = [&](MeshChunk &c) -> int {
+        c.m.vert_out = c.out[0].as<double>();
+        c.m.triangles = c.out[1].as<uint32_t>();
+        c.m.tri_block = c.out[2].as<uint32_t>();
+        c.m.vert_base = (uint32_t)c.vert_base;
+        int e = cc_launch_mesh_indexed_emit(c.m, c.n_tiles, g.compute);
+        if (e) return cuda_fail((cudaError_t)e, "marching cubes (indexed emit)");
+        g.launches += 2;
+        return CC_OK;
+    };
+    // keeps the field, the vertex base and the owned crossed edges of every sample
+    const MeshPass pass{4 + 4 + 1, {{3 * sizeof(double), true}, {3 * sizeof(uint32_t), false}, {4, false}}, reconcile, emit};
+    void *host[3] = {nullptr, nullptr, nullptr};
+    uint64_t rows[2] = {0, 0};
+    if ((rc = mesh_chunks(prog, corners, resolution, nx, ny, nz, n_blocks, pass, host, rows))) return rc;
+    *out_vertices = (double *)host[0];
+    *out_triangles = (uint32_t *)host[1];
+    *out_triangle_block = (uint32_t *)host[2];
+    *out_n_triangles = rows[0];
+    *out_n_vertices = rows[1];
     return CC_OK;
 }
 

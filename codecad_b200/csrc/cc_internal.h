@@ -267,11 +267,38 @@ struct cc_mesh_args {
     uint32_t first_block;  // added to the block index written to tri_block
     uint32_t *tile_offsets; // cc_mesh_scratch_words(tiles) words: triangle counts (count pass) -> exclusive offsets; scan scratch
     uint32_t *tile_list;    // ids of the tiles that hold triangles, increasing (inside the same scratch)
+
+    // ---- indexed export only (cc_mesh_blocks_indexed); blocks are cubic when there are several ----
+    // Block table of the whole call: block coordinates (int corner / (n-1)) in array axes (i = -y,
+    // j = x, k = z), shifted to be non-negative, packed 21 bits each (i highest).
+    const uint64_t *block_key;   // [n_all] key of every block, input order
+    const uint64_t *sorted_key;  // [n_all] the same keys, increasing
+    const uint32_t *sorted_block; // [n_all] block index of sorted_key[r]
+    uint32_t n_all;              // blocks in the call
+    uint32_t nf;                 // face archive row length: max(d0, d1, d2)
+    float *face_field;           // [n_all][6 faces][nf][nf] each block's face samples as evaluated
+    uint32_t *face_vertex;       // [n_all][6][nf][nf][2] global index of the owned vertex on each in-face edge
+    uint32_t *vbase;             // [n_blocks * samples] owned crossed edges per sample -> exclusive vertex offsets in the chunk
+    uint8_t *vmask;              // [n_blocks * samples] bit a: the edge along array axis a from this sample is owned and crossed
+    uint32_t vert_base;          // vertices of the earlier chunks
+    double *vert_out;            // [chunk vertices][3] (emit pass)
+    uint32_t *triangles;         // [n_triangles][3] vertex indices (emit pass)
 };
 
 int cc_mesh_upload_tables(void *stream);
 uint32_t cc_mesh_tiles_per_block(uint32_t d0, uint32_t d1, uint32_t d2);
 int cc_launch_mesh(const cc_mesh_args &a, bool emit, uint32_t emit_tiles, void *stream);
 size_t cc_mesh_scratch_words(uint32_t tiles);
+// In-place exclusive scan of v[0..n) with the ids of the non-zero elements in `list`; scratch holds
+// cc_mesh_scan_scratch_words(n) words.  counter[0] = sum, counter[1] = non-zero elements.
+size_t cc_mesh_scan_scratch_words(uint32_t n);
+int cc_launch_mesh_scan(uint32_t *v, uint32_t n, uint32_t *scratch, uint32_t *list, uint32_t *counter, void *stream);
+// Indexed export, per chunk (after the PYMCUBES evaluation into a.field):
+//   reconcile: archive the chunk's face samples, then replace every sample a block does not own with
+//              its owner's value; then count the owned crossed edges per sample into vbase / vmask.
+//   emit: vertex positions and face vertex indices, then (the tiles listed by the count pass) the
+//         triangles as vertex indices.
+int cc_launch_mesh_reconcile(const cc_mesh_args &a, void *stream);
+int cc_launch_mesh_indexed_emit(const cc_mesh_args &a, uint32_t emit_tiles, void *stream);
 
 #endif

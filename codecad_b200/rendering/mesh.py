@@ -11,6 +11,9 @@ post-transform (mesh.py:68-72).  Differences a caller can see: every piece is a 
 consumers in the reference (`render_stl` expands to a soup, tests merge duplicate vertices) are
 indifferent to it — and ambiguous faces are resolved by a fixed rule that keeps neighbouring cells
 consistent (tools/make_mc_tables.py).
+
+`indexed_mesh` (not in the reference) returns the same surface welded: shared vertices, triangles as
+vertex indices, watertight by index (`cc_mesh_blocks_indexed`, DESIGN.md 4.4), for PLY / 3MF export.
 """
 import ctypes
 
@@ -19,7 +22,7 @@ import numpy as np
 from . import _compat  # noqa: F401  (kept tiny: shape protocol helpers)
 from .. import _lib
 from ..geometry import Vector
-from ..subdivision import block_corners, subdivision
+from ..subdivision import LeafBlocks, block_corners, subdivision
 
 
 def _check_3d(obj):
@@ -44,6 +47,31 @@ def mesh_blocks(program_buffer, box_size, corners, resolution):
         return np.zeros((0, 3, 3), np.float64), np.zeros((0,), np.uint32)
     # wrap the library's buffers without copying; they are released when the arrays die
     return _adopt(out_v, (t, 3, 3)), _adopt(out_b, (t,))
+
+
+def indexed_mesh_blocks(program_buffer, box_size, corners, int_corners, resolution):
+    """Welded marching cubes over the same blocks as mesh_blocks; int_corners: int64 [n][3]
+    (LeafBlocks.int_corners).  Shared samples and vertices come from the first block that holds
+    them, so the mesh is watertight by index.  Returns (vertices float64 [v][3], triangles uint32
+    [t][3], block index uint32 [t]); vertices[triangles] is mesh_blocks' soup where neighbouring
+    blocks evaluate their shared samples alike."""
+    corners = np.ascontiguousarray(corners, dtype=np.float64).reshape(-1, 3)
+    int_corners = np.ascontiguousarray(int_corners, dtype=np.int64).reshape(-1, 3)
+    if len(int_corners) != len(corners):
+        raise ValueError("corners and int_corners differ in length")
+    out_v = ctypes.POINTER(ctypes.c_double)()
+    out_t = ctypes.POINTER(ctypes.c_uint32)()
+    out_b = ctypes.POINTER(ctypes.c_uint32)()
+    nv, nt = ctypes.c_uint64(), ctypes.c_uint64()
+    _lib.check(_lib.lib().cc_mesh_blocks_indexed(
+        program_buffer.handle, corners.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+        int_corners.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), float(resolution),
+        int(box_size[0]), int(box_size[1]), int(box_size[2]), len(corners),
+        ctypes.byref(out_v), ctypes.byref(nv), ctypes.byref(out_t), ctypes.byref(out_b), ctypes.byref(nt)))
+    v, t = int(nv.value), int(nt.value)
+    if t == 0:
+        return np.zeros((0, 3), np.float64), np.zeros((0, 3), np.uint32), np.zeros((0,), np.uint32)
+    return _adopt(out_v, (v, 3)), _adopt(out_t, (t, 3)), _adopt(out_b, (t,))
 
 
 class _Owner:
@@ -86,6 +114,22 @@ def mesh_arrays(obj, subdivision_grid_size=None):
     # every leaf block has the same size and resolution (subdivision.py:97-111)
     vertices, block = mesh_blocks(program_buffer, max_box_size, corners, boxes[0][2])
     return vertices, block, boxes
+
+
+def indexed_mesh(obj, subdivision_grid_size=None):
+    """The shape's welded mesh, on the blocks mesh_arrays uses: (vertices float64 [v][3],
+    triangles uint32 [t][3], block index uint32 [t], boxes)."""
+    _check_3d(obj)
+    program_buffer, max_box_size, boxes = subdivision(obj, obj.feature_size() / 2, grid_size=subdivision_grid_size)
+    if not len(boxes):
+        return np.zeros((0, 3), np.float64), np.zeros((0, 3), np.uint32), np.zeros((0,), np.uint32), boxes
+    if isinstance(boxes, LeafBlocks):
+        int_corners = boxes.int_corners
+    else:  # a single-level plan: one block
+        int_corners = np.array([[int(c) for c in b[3]] for b in boxes], dtype=np.int64).reshape(-1, 3)
+    vertices, triangles, block = indexed_mesh_blocks(program_buffer, max_box_size, block_corners(boxes), int_corners,
+                                                     boxes[0][2])
+    return vertices, triangles, block, boxes
 
 
 def triangular_mesh(obj, subdivision_grid_size=None, debug_subdivision_boxes=False):

@@ -341,6 +341,25 @@ int cc_mesh_blocks(const cc_program *prog, const double *corners, double resolut
                    uint32_t nx, uint32_t ny, uint32_t nz, uint32_t n_blocks,
                    double **out_vertices, uint32_t **out_triangle_block, uint64_t *out_triangles);
 
+/* Welded mesh of the same blocks: every vertex once, triangles as vertex indices, watertight by
+ * construction.  int_corners[n][3] are the blocks' int corners (resolution units, LeafBlocks.int_corners).
+ * Neighbouring blocks share their face samples; each block evaluates them from its own fp32 corner,
+ * so the copies can differ in their last bits.  Here every shared sample takes the value of the
+ * first block in input order that holds it (array index (i,j,k) of a block is the lattice point
+ * (X + j, Y + ny-1-i, Z + k)), and marching cubes runs on these fields with the triangle order,
+ * winding and triangle_block of cc_mesh_blocks.  One vertex per crossed lattice edge, placed as
+ * cc_mesh_blocks places it in the edge's owner (the first block holding both ends); vertices are
+ * ordered by owner block, then lower end in (i,j,k) order, then edge axis.  Results, page-locked,
+ * released with cc_free: vertices[n_vertices][3] (float64), triangles[n_triangles][3] (uint32) and
+ * triangle_block[n_triangles].  Where no shared sample differs, vertices[triangles] is
+ * cc_mesh_blocks' soup bit for bit.  CC_ERR_INVALID_ARGUMENT for several blocks that are not cubic,
+ * int corners that are not all congruent modulo n-1, repeated int corners, or blocks spread over
+ * 2^21 or more block widths along an axis. */
+int cc_mesh_blocks_indexed(const cc_program *prog, const double *corners, const int64_t *int_corners,
+                           double resolution, uint32_t nx, uint32_t ny, uint32_t nz, uint32_t n_blocks,
+                           double **out_vertices, uint64_t *out_n_vertices, uint32_t **out_triangles,
+                           uint32_t **out_triangle_block, uint64_t *out_n_triangles);
+
 void cc_free(void *p);
 
 #ifdef __cplusplus
