@@ -58,6 +58,7 @@ SIGNATURES = {
     "cc_synchronize": (_I, []),
     "cc_get_counters": (_I, [ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]),
     "cc_reset_counters": (None, []),
+    "cc_get_check_fallbacks": (_I, [ctypes.POINTER(ctypes.c_uint64)]),
     "cc_set_tuning": (_I, [_I, _I]),
     "cc_program_create": (_I, [c_float_p, _U, c_void_pp]),
     "cc_program_destroy": (None, [_V]),
@@ -245,6 +246,13 @@ def counters():
     a, b = ctypes.c_uint64(), ctypes.c_uint64()
     check(lib().cc_get_counters(ctypes.byref(a), ctypes.byref(b)))
     return a.value, b.value
+
+
+def check_fallbacks():
+    """Warps of the column brick kernel that failed their deferred range check and took the full walk."""
+    n = ctypes.c_uint64()
+    check(lib().cc_get_check_fallbacks(ctypes.byref(n)))
+    return n.value
 
 
 def f3(v):

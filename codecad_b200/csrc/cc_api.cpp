@@ -43,6 +43,7 @@ struct Context {
     size_t columns_cap = 0;
     uint32_t *d_part_masks = nullptr;
     size_t part_masks_cap = 0;
+    unsigned long long *d_check_fallbacks = nullptr;  // warps of the column brick kernel that took the full walk
     uint32_t jit_max_ops = 4096;  // programs longer than this are not specialised automatically
     uint64_t constant_program = 0;  // id of the program in this device's __constant__ window
     int index = 0;                  // position in g_ctx
@@ -437,6 +438,7 @@ int prepare_columns(const cc_columns_meta &meta, cc_eval_args &a, uint64_t n_bri
     a.column_flags = meta.checks ? reinterpret_cast<unsigned char *>(base + flags_at) : nullptr;
     a.brick_count = meta.checks && n_bricks ? reinterpret_cast<uint32_t *>(base + list_at) : nullptr;
     a.brick_list = a.brick_count ? a.brick_count + 1 : nullptr;
+    a.check_fallbacks = g.d_check_fallbacks;
     if (a.brick_count) CU(cudaMemsetAsync(a.brick_count, 0, 4, g.compute));
     return CC_OK;
 }
@@ -586,6 +588,8 @@ int init_context(Context &c, int device, int index)
     CU(cudaStreamCreateWithFlags(&c.copy, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&c.copy2, cudaStreamNonBlocking));
     CU(cudaMallocHost(&c.h_word, 64));
+    CU(cudaMalloc(&c.d_check_fallbacks, sizeof(unsigned long long)));
+    CU(cudaMemset(c.d_check_fallbacks, 0, sizeof(unsigned long long)));
     {
         // keep freed work-list memory in the pool instead of returning it to the driver at every sync
         cudaMemPool_t pool = nullptr;
@@ -780,6 +784,7 @@ void cc_shutdown(void)
         if (c.d_forest_scratch) cudaFree(c.d_forest_scratch);
         if (c.d_part_masks) cudaFree(c.d_part_masks);
         if (c.d_columns) cudaFree(c.d_columns);
+        if (c.d_check_fallbacks) cudaFree(c.d_check_fallbacks);
         if (c.h_word) cudaFreeHost(c.h_word);
         for (int i = 0; i < Context::kRing; ++i) {
             if (c.ring[i]) cudaFree(c.ring[i]);
@@ -843,6 +848,29 @@ int cc_get_counters(uint64_t *kernel_launches, uint64_t *points_evaluated)
 void cc_reset_counters(void)
 {
     for (int i = 0; i < CC_MAX_DEVICES; ++i) g_ctx[i].launches = g_ctx[i].points = 0;
+    int dev = -1;
+    if (g_n_ctx == 0 || cudaGetDevice(&dev) != cudaSuccess) return;
+    for (int i = 0; i < g_n_ctx; ++i)
+        if (g_ctx[i].d_check_fallbacks && cudaSetDevice(g_ctx[i].device) == cudaSuccess)
+            cudaMemsetAsync(g_ctx[i].d_check_fallbacks, 0, sizeof(unsigned long long), g_ctx[i].compute);
+    cudaSetDevice(dev);
+}
+
+int cc_get_check_fallbacks(uint64_t *warps)
+{
+    NEED_INIT();
+    uint64_t n = 0;
+    for (int i = 0; i < g_n_ctx; ++i) {
+        Context &c = g_ctx[i];
+        unsigned long long v = 0;
+        CU(cudaSetDevice(c.device));
+        CU(cudaMemcpyAsync(&v, c.d_check_fallbacks, sizeof v, cudaMemcpyDeviceToHost, c.compute));
+        CU(cudaStreamSynchronize(c.compute));
+        n += v;
+    }
+    CU(cudaSetDevice(g.device));
+    if (warps) *warps = n;
+    return CC_OK;
 }
 
 int cc_set_tuning(int points_per_thread, int program_space)

@@ -266,6 +266,27 @@ template <class V> CC_DEV cc_val<V> cc_col_load(const cc_col_ref &r, uint32_t k)
     for (int l = 0; l < cc_lane<V>::N; ++l) cc_lane_put(v, l, __ldg(r.rec[l] + k));
     return v;
 }
+// The brick kernel pairs a thread's two cells along the columns' axis (CC_COL_PAIR), so both read one record:
+// one load, and the same value in both lanes.  0 keeps the brick order of cc_kernel_body_bricks_at.
+#ifndef CC_COL_PAIR
+#define CC_COL_PAIR 1
+#endif
+struct cc_col_one {
+    const float4 *rec;  // the column record of both points of the thread's pair
+};
+template <class V> CC_DEV cc_val<V> cc_col_load(const cc_col_one &r, uint32_t k)
+{
+    const float4 c = __ldg(r.rec + k);
+    cc_val<V> v;
+#pragma unroll
+    for (int l = 0; l < cc_lane<V>::N; ++l) cc_lane_put(v, l, c);
+    return v;
+}
+#if CC_COL_PAIR
+typedef cc_col_one cc_brick_col_ref;
+#else
+typedef cc_col_ref cc_brick_col_ref;
+#endif
 CC_DEV bool cc_same_bits(float a, float b) { return __float_as_uint(a) == __float_as_uint(b) && a == a; }
 CC_DEV bool cc_same_bits(float2 a, float2 b) { return cc_same_bits(a.x, b.x) && cc_same_bits(a.y, b.y); }
 
@@ -334,7 +355,12 @@ CC_DEV bool cc_col_locate(const cc_eval_args &a, uint32_t block, const uint32_t 
     return a.column_flags ? __syncthreads_or(flagged) != 0 : false;
 }
 
-// the brick kernel of cc_kernel_body_bricks with the thread's two columns at hand
+// The brick kernel of cc_kernel_body_bricks with the thread's columns at hand.  With CC_COL_PAIR the two cells of a
+// thread differ only along the columns' axis (z-columns: z and z + 8, a warp's store is four 128-byte runs; y-columns:
+// y and y + 4; x-columns: the brick order's x and x + 4 already), so they share one column record.
+// EVAL (the generated SceneTile): `loop` is the per-cell body and its column reference; with EVAL::deferred its ops fold
+// their range tests into `range` instead of voting per op (DESIGN.md 4.10), and a warp in which some lane flags
+// evaluates its cells again with EVAL::full, the guarded full walk.
 template <int PTS, class EVAL>
 CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
 {
@@ -351,17 +377,35 @@ CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
         ix[j] = x0 + (c >> 7);
         iy[j] = y0 + ((c >> 4) & 7u);
         iz[j] = z0 + (c & 15u);
+        if (CC_COL_PAIR && CC_COL_AXIS == 2) {
+            ix[j] = x0 + (tid >> 6);
+            iy[j] = y0 + ((tid >> 3) & 7u);
+            iz[j] = z0 + (tid & 7u) + 8u * (uint32_t)j;
+        } else if (CC_COL_PAIR && CC_COL_AXIS == 1) {
+            ix[j] = x0 + (tid >> 6);
+            iy[j] = y0 + ((tid >> 4) & 3u) + 4u * (uint32_t)j;
+            iz[j] = z0 + (tid & 15u);
+        }
         gx[j] = cc_fma(a.step, (float)(ix[j] + a.x_offset), a.cx);
         gy[j] = cc_fma(a.step, (float)iy[j], a.cy);
         gz[j] = cc_fma(a.step, (float)iz[j], a.cz);
         const uint32_t u = CC_COL_AXIS == 0 ? iy[j] : ix[j], v = CC_COL_AXIS == 2 ? iy[j] : iz[j];
         col[j] = min(u, cc_col_dim_u(a) - 1u) * cc_col_dim_v(a) + min(v, cc_col_dim_v(a) - 1u);  // (cells past the edge read a neighbour's column)
-        eval.cr.rec[j] = reinterpret_cast<float4 *>(a.columns) + (size_t)col[j] * CC_COL_VALUES;
-        eval.cr.ok[j] = true;
     }
+#if CC_COL_PAIR
+    eval.loop.cr.rec = reinterpret_cast<const float4 *>(a.columns) + (size_t)col[0] * CC_COL_VALUES;
+    const int col_flag = a.column_flags ? (int)a.column_flags[col[0]] : 0;
+#else
+#pragma unroll
+    for (int j = 0; j < PTS; ++j) {
+        eval.loop.cr.rec[j] = reinterpret_cast<float4 *>(a.columns) + (size_t)col[j] * CC_COL_VALUES;
+        eval.loop.cr.ok[j] = true;
+    }
+    const int col_flag = a.column_flags ? (int)(a.column_flags[col[0]] | a.column_flags[col[1]]) : 0;
+#endif
     if (a.column_flags) {
         // a column whose "invariant" micro-ops do see z in some bit: the whole brick takes the full walk
-        const int flagged = __syncthreads_or((int)(a.column_flags[col[0]] | a.column_flags[col[1]]));
+        const int flagged = __syncthreads_or(col_flag);
         if (flagged) {
             if (tid == 0) a.brick_list[atomicAdd(a.brick_count, 1u)] = blockIdx.x;
             return;
@@ -372,7 +416,13 @@ CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
     vx[0] = cc_pack<V>(gx);
     vy[0] = cc_pack<V>(gy);
     vz[0] = cc_pack<V>(gz);
-    eval(vx, vy, vz, LV);
+    uint32_t range = 0;
+    eval(vx, vy, vz, LV, range);
+    if (EVAL::deferred && __any_sync(0xffffffffu, cc_range_flagged(range))) {
+        // some op of some lane had an operand outside its fast path's range: the warp's values are thrown away
+        if ((tid & 31u) == 0 && a.check_fallbacks) atomicAdd(a.check_fallbacks, 1ull);
+        eval.full(vx, vy, vz, LV);
+    }
     float4 *out = reinterpret_cast<float4 *>(a.out);
 #pragma unroll
     for (int j = 0; j < PTS; ++j)

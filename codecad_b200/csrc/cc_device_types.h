@@ -76,6 +76,8 @@ struct cc_eval_args {
     float *columns;
     unsigned char *column_flags;
     uint32_t *brick_list, *brick_count;
+    // warps of the column brick kernel whose deferred range check failed and that took the full walk (cc_body.cuh)
+    unsigned long long *check_fallbacks;
 };
 
 // bricks of the part-culling kernels: a CTA of 512 threads x 2 points

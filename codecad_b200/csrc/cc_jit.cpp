@@ -264,6 +264,24 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
         *err = "part culling needs a program with parts and 512 threads x 2 points";
         return CC_ERR_INVALID_ARGUMENT;
     }
+    // the columns unit's per-cell body defers its ops' range checks to one vote per warp (DESIGN.md 4.10) when every
+    // micro-op in it is pure arithmetic: no address and no loop bound depends on a value, so an op fed an operand out of
+    // its fast path's range yields inf or NaN that the fallback throws away, and cannot fault or loop
+    const bool column_unit = columns_mode && !tiles;
+    bool defer_checks = column_unit;
+    auto deferrable = [](uint32_t op) {
+        switch (op) {
+        case MOP_RETURN: case MOP_NOP: case MOP_LOAD:
+        case MOP_T_INIT: case MOP_T_TO: case MOP_T_FROM: case MOP_T_INIT_M: case MOP_T_TO_M: case MOP_T_FROM_M:
+        case MOP_RECTANGLE: case MOP_CIRCLE: case MOP_SPHERE:
+        case MOP_PRIM_CIRCLE: case MOP_PRIM_RECT: case MOP_PRIM_CIRCLE_M: case MOP_PRIM_RECT_M:
+        case MOP_EXTRUSION: case MOP_OFFSET: case MOP_SHELL: case MOP_MIRROR: case MOP_SYM_TO: case MOP_SYM_FROM:
+        case MOP_UNION: case MOP_ISECT: case MOP_SUB:
+            return true;
+        default:
+            return false;
+        }
+    };
     std::ostringstream hoisted;  // parts mode: value variables are declared ahead of the conditional blocks
     std::ostringstream ahead, in_loop, full;  // columns mode: the three bodies
     int full_open = -1, loop_open = -1;       // the part whose `if` is open in each body
@@ -586,6 +604,7 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
                 ahead << "        }\n";
             }
             if (ph & 2) {
+                if (!deferrable(op)) defer_checks = false;
                 const int from = cols.restore_from[(size_t)op_index];
                 if (from >= 0) {
                     const int from_part = (size_t)from < parts.part_of_op.size() && parts_mode ? parts.part_of_op[(size_t)from] : -1;
@@ -648,21 +667,43 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
           << "    __device__ __forceinline__ bool invariant" << sig << ", const V (&g_last)[G]) const\n    {\n"
           << "        bool ok = true;\n" << chk.str() << "        return ok;\n    }\n"
           << "    __device__ __forceinline__ void operator()" << sig << ") const\n    {\n" << hoisted.str() << "        Val L[G];\n" << zero_l
-          << ahead.str() << "    }\n};\n"
-          << "// per cell: the rest, reading the column's values\n"
-          << "struct SceneEval {\n    float4 *sm;\n    unsigned mask;\n    cc_col_ref cr;\n"
-          << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]) const\n    {\n" << hoisted.str() << zero_l
-          << in_loop.str();
+          << ahead.str() << "    }\n};\n";
+        std::string loop_text = in_loop.str();
+        if (column_unit && defer_checks)  // the deferred forms: the same calls with the accumulator as a last argument
+            for (const char *f : {"cc_extrusion_n(", "cc_circle_n(", "cc_rectangle_n(", "cc_sphere_n("})
+                for (size_t at = loop_text.find(f); at != std::string::npos; at = loop_text.find(f, at + 1)) {
+                    const size_t close = loop_text.find(");", at);
+                    loop_text.insert(close, ", range");
+                }
+        s << "// per cell: the rest, reading the column's values" << (column_unit && defer_checks ? "; the range checks go into `range`" : "") << "\n"
+          << "struct SceneEval {\n    float4 *sm;\n    unsigned mask;\n    " << (column_unit ? "cc_brick_col_ref" : "cc_col_ref") << " cr;\n"
+          << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]" << (column_unit ? ", unsigned &range" : "") << ") const\n    {\n"
+          << (column_unit ? "        (void)range;\n" : "") << hoisted.str() << zero_l << loop_text;
         if (cols.root_restore >= 0) s << "        CC_EACH L[g] = cc_col_load<V>(cr, " << carried_l[(size_t)cols.root_restore] << "u);\n";
         s << "    }\n};\n";
-        s << "// the hierarchy sinks (blocks x linear tiles): the rest per cell, or the full walk for a tile with a flagged column\n"
-          << "struct SceneTile {\n    SceneEval loop;\n    SceneFull full;\n    bool use_full;\n"
-          << "    __device__ __forceinline__ void locate(const cc_eval_args &a, unsigned tile, unsigned block, const unsigned (&ix)[PTS],\n"
-          << "                                           const unsigned (&iy)[PTS], const unsigned (&iz)[PTS])\n    {\n"
-          << "        use_full = cc_col_locate<PTS>(a, block, ix, iy, iz, loop.cr);\n"
-          << "        if (a.part_masks) loop.mask = full.mask = a.part_masks[tile];  // (cc_tile_centers_body)\n    }\n"
-          << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]) const\n    {\n"
-          << "        if (use_full) full(gx, gy, gz, L);\n        else loop(gx, gy, gz, L);\n    }\n};\n";
+        if (tiles)
+            s << "// the hierarchy sinks (blocks x linear tiles): the rest per cell, or the full walk for a tile with a flagged column\n"
+              << "struct SceneTile {\n    SceneEval loop;\n    SceneFull full;\n    bool use_full;\n"
+              << "    __device__ __forceinline__ void locate(const cc_eval_args &a, unsigned tile, unsigned block, const unsigned (&ix)[PTS],\n"
+              << "                                           const unsigned (&iy)[PTS], const unsigned (&iz)[PTS])\n    {\n"
+              << "        use_full = cc_col_locate<PTS>(a, block, ix, iy, iz, loop.cr);\n"
+              << "        if (a.part_masks) loop.mask = full.mask = a.part_masks[tile];  // (cc_tile_centers_body)\n    }\n"
+              << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]) const\n    {\n"
+              << "        if (use_full) full(gx, gy, gz, L);\n        else loop(gx, gy, gz, L);\n    }\n};\n";
+        else
+            s << "// the full walk of one thread's cells, out of line: cc_jit_columns_full and the brick kernel's fallback share it\n"
+              << "struct ScenePts {\n    V x[G], y[G], z[G];\n};\nstruct SceneVals {\n    Val L[G];\n};\n"
+              << "static __device__ __noinline__ SceneVals cc_full_walk(float4 *sm, unsigned mask, const ScenePts p)\n{\n"
+              << "    SceneVals r;\n    const SceneFull e{sm, mask, nullptr};\n    e(p.x, p.y, p.z, r.L);\n    return r;\n}\n"
+              << "struct SceneFullCall {\n    float4 *sm;\n    unsigned mask;\n"
+              << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]) const\n    {\n"
+              << "        ScenePts p;\n        CC_EACH { p.x[g] = gx[g]; p.y[g] = gy[g]; p.z[g] = gz[g]; }\n"
+              << "        const SceneVals r = cc_full_walk(sm, mask, p);\n        CC_EACH L[g] = r.L[g];\n    }\n};\n"
+              << "// the brick kernel (cc_kernel_body_brick_columns): the rest per cell, or the full walk for a warp in which a range check failed\n"
+              << "struct SceneTile {\n    SceneEval loop;\n"
+              << "    static constexpr bool deferred = " << (defer_checks ? "CC_DEFER_CHECKS != 0" : "false") << ";\n"
+              << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G], unsigned &range) const { loop(gx, gy, gz, L, range); }\n"
+              << "    __device__ __forceinline__ void full" << sig << ", Val (&L)[G]) const { SceneFullCall{loop.sm, loop.mask}(gx, gy, gz, L); }\n};\n";
         if (columns_meta) {
             columns_meta->n_values = n_carried;
             columns_meta->checks = !chk.str().empty();
@@ -730,12 +771,12 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
           << "    cc_column_profiles_body<PTS>(a, e);\n}\n";
     if (columns_mode && !tiles) {
         s << "extern \"C\" __global__ void __launch_bounds__(" << bounds << ") cc_jit_columns" << head
-          << "    SceneEval e;\n    e.sm = cc_cells + threadIdx.x;\n    e.mask = a.part_masks ? a.part_masks[blockIdx.x] : 0xffffffffu;\n"
+          << "    SceneTile e;\n    e.loop.sm = cc_cells + threadIdx.x;\n    e.loop.mask = a.part_masks ? a.part_masks[blockIdx.x] : 0xffffffffu;\n"
           << "    cc_kernel_body_brick_columns<PTS>(a, e);\n}\n"
           << "extern \"C\" __global__ void __launch_bounds__(" << bounds << ") cc_jit_columns_full" << head
           << "    const unsigned n = *a.brick_count;\n    for (unsigned i = blockIdx.x; i < n; i += gridDim.x) {\n"
           << "        const unsigned b = a.brick_list[i];\n"
-          << "        SceneFull e{cc_cells + threadIdx.x, a.part_masks ? a.part_masks[b] : 0xffffffffu, nullptr};\n"
+          << "        SceneFullCall e{cc_cells + threadIdx.x, a.part_masks ? a.part_masks[b] : 0xffffffffu};\n"
           << "        cc_kernel_body_bricks_at<PTS>(a, e, b);\n    }\n}\n";
         if (parts_mode)
             s << "extern \"C\" __global__ void __launch_bounds__(" << bounds << ") cc_jit_columns_centers" << head

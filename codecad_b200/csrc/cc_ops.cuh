@@ -103,8 +103,8 @@ CC_DEV void cc_each_lane(cc_val<V> (&L)[G], F f)
     }
 }
 
-template <class V, int G>
-CC_DEV void cc_rectangle_n(float hw, float hh, cc_val<V> (&L)[G])
+template <bool DEFER, class V, int G>
+CC_DEV void cc_rectangle_n_(uint32_t &range, float hw, float hh, cc_val<V> (&L)[G])
 {
     typedef typename cc_lane<V>::mask M;
     V ax[G], ay[G], s[G];
@@ -114,9 +114,10 @@ CC_DEV void cc_rectangle_n(float hw, float hh, cc_val<V> (&L)[G])
         ax[g] = vsub(vabs(L[g].x), vbc<V>(hw));
         ay[g] = vsub(vabs(L[g].y), vbc<V>(hh));
         s[g] = vfma(ax[g], ax[g], vmul(ay[g], ay[g]));
-        sp |= vspecial(s[g]);
+        if (DEFER) vrange(range, s[g]);
+        else sp |= vspecial(s[g]);
     }
-    if (__any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
+    if (!DEFER && __any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
         cc_each_lane(L, [&](float4 p, int, int) { return cc_rectangle_slow(hw, hh, p); });
         return;
     }
@@ -137,17 +138,18 @@ CC_DEV void cc_rectangle_n(float hw, float hh, cc_val<V> (&L)[G])
     }
 }
 
-template <class V, int G>
-CC_DEV void cc_circle_n(float r, cc_val<V> (&L)[G])
+template <bool DEFER, class V, int G>
+CC_DEV void cc_circle_n_(uint32_t &range, float r, cc_val<V> (&L)[G])
 {
     V s[G];
     bool sp = false;
 #pragma unroll
     for (int g = 0; g < G; ++g) {
         s[g] = vfma(L[g].x, L[g].x, vmul(L[g].y, L[g].y));
-        sp |= vspecial(s[g]);
+        if (DEFER) vrange(range, s[g]);
+        else sp |= vspecial(s[g]);
     }
-    if (__any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
+    if (!DEFER && __any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
         cc_each_lane(L, [&](float4 p, int, int) { return cc_circle_slow(r, p); });
         return;
     }
@@ -159,17 +161,18 @@ CC_DEV void cc_circle_n(float r, cc_val<V> (&L)[G])
     }
 }
 
-template <class V, int G>
-CC_DEV void cc_sphere_n(float r, cc_val<V> (&L)[G])
+template <bool DEFER, class V, int G>
+CC_DEV void cc_sphere_n_(uint32_t &range, float r, cc_val<V> (&L)[G])
 {
     V s[G];
     bool sp = false;
 #pragma unroll
     for (int g = 0; g < G; ++g) {
         s[g] = vfma(L[g].x, L[g].x, vfma(L[g].y, L[g].y, vmul(L[g].z, L[g].z)));
-        sp |= vspecial(s[g]);
+        if (DEFER) vrange(range, s[g]);
+        else sp |= vspecial(s[g]);
     }
-    if (__any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
+    if (!DEFER && __any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
         cc_each_lane(L, [&](float4 p, int, int) { return cc_sphere_slow(r, p); });
         return;
     }
@@ -182,8 +185,8 @@ CC_DEV void cc_sphere_n(float r, cc_val<V> (&L)[G])
 }
 
 // cz[g] = z coordinate of the point operand
-template <class V, int G>
-CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G], const V (&cz)[G])
+template <bool DEFER, class V, int G>
+CC_DEV void cc_extrusion_n_(uint32_t &range, float h, cc_val<V> (&L)[G], const V (&cz)[G])
 {
     typedef typename cc_lane<V>::mask M;
     V az[G], s[G];
@@ -192,9 +195,10 @@ CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G], const V (&cz)[G])
     for (int g = 0; g < G; ++g) {
         az[g] = vsub(vabs(cz[g]), vbc<V>(h));
         s[g] = vfma(az[g], az[g], vmul(L[g].w, L[g].w));
-        sp |= vspecial(s[g]);
+        if (DEFER) vrange(range, s[g]);
+        else sp |= vspecial(s[g]);
     }
-    if (__any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
+    if (!DEFER && __any_sync(0xffffffffu, sp)) {  // warp-uniform: keeps the interpreter's control flow convergent
         cc_each_lane(L, [&](float4 p, int g, int l) { return cc_extrusion_slow(h, p, vlane(cz[g], l)); });
         return;
     }
@@ -215,6 +219,45 @@ CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G], const V (&cz)[G])
         r.w = vsel(both, dist, vsel(first, az[g], in.w));
         L[g] = r;
     }
+}
+
+// the voting forms, and the deferred ones (last argument `range`): the fast path always, its range test folded into
+// `range`, which the caller tests once after all its ops (cc_range_flagged); CC_DEFER_CHECKS=0 makes them vote
+template <class V, int G> CC_DEV void cc_rectangle_n(float hw, float hh, cc_val<V> (&L)[G])
+{
+    uint32_t unused = 0;
+    cc_rectangle_n_<false>(unused, hw, hh, L);
+}
+template <class V, int G> CC_DEV void cc_rectangle_n(float hw, float hh, cc_val<V> (&L)[G], uint32_t &range)
+{
+    cc_rectangle_n_<CC_DEFER_CHECKS != 0>(range, hw, hh, L);
+}
+template <class V, int G> CC_DEV void cc_circle_n(float r, cc_val<V> (&L)[G])
+{
+    uint32_t unused = 0;
+    cc_circle_n_<false>(unused, r, L);
+}
+template <class V, int G> CC_DEV void cc_circle_n(float r, cc_val<V> (&L)[G], uint32_t &range)
+{
+    cc_circle_n_<CC_DEFER_CHECKS != 0>(range, r, L);
+}
+template <class V, int G> CC_DEV void cc_sphere_n(float r, cc_val<V> (&L)[G])
+{
+    uint32_t unused = 0;
+    cc_sphere_n_<false>(unused, r, L);
+}
+template <class V, int G> CC_DEV void cc_sphere_n(float r, cc_val<V> (&L)[G], uint32_t &range)
+{
+    cc_sphere_n_<CC_DEFER_CHECKS != 0>(range, r, L);
+}
+template <class V, int G> CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G], const V (&cz)[G])
+{
+    uint32_t unused = 0;
+    cc_extrusion_n_<false>(unused, h, L, cz);
+}
+template <class V, int G> CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G], const V (&cz)[G], uint32_t &range)
+{
+    cc_extrusion_n_<CC_DEFER_CHECKS != 0>(range, h, L, cz);
 }
 
 // shapes/common.cl:45-64

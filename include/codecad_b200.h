@@ -71,6 +71,10 @@ int cc_synchronize(void);
  * mass_properties.py:66-67,110-111). */
 int cc_get_counters(uint64_t *kernel_launches, uint64_t *points_evaluated);
 void cc_reset_counters(void);
+/* warps of the column brick kernel (DESIGN.md 4.10) since cc_init / the last reset whose deferred
+ * range check failed, so that they evaluated their cells again with the guarded full walk; waits
+ * for the work queued so far. */
+int cc_get_check_fallbacks(uint64_t *warps);
 /* tuning knobs, mainly for bench.py / profiling: points per thread (1,2,4; 0 = auto),
  * and where the microcode is fetched from (0 = auto, 1 = __constant__, 2 = shared). */
 int cc_set_tuning(int points_per_thread, int program_space);
