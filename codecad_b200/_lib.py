@@ -59,6 +59,7 @@ SIGNATURES = {
     "cc_get_counters": (_I, [ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]),
     "cc_reset_counters": (None, []),
     "cc_get_check_fallbacks": (_I, [ctypes.POINTER(ctypes.c_uint64)]),
+    "cc_get_flagged_bricks": (_I, [ctypes.POINTER(ctypes.c_uint64)]),
     "cc_set_tuning": (_I, [_I, _I]),
     "cc_program_create": (_I, [c_float_p, _U, c_void_pp]),
     "cc_program_destroy": (None, [_V]),
@@ -252,6 +253,13 @@ def check_fallbacks():
     """Warps of the column brick kernel that failed their deferred range check and took the full walk."""
     n = ctypes.c_uint64()
     check(lib().cc_get_check_fallbacks(ctypes.byref(n)))
+    return n.value
+
+
+def flagged_bricks():
+    """Bricks of the column brick kernel that a column failing its run-time check sent to the full walk."""
+    n = ctypes.c_uint64()
+    check(lib().cc_get_flagged_bricks(ctypes.byref(n)))
     return n.value
 
 

@@ -43,7 +43,9 @@ struct Context {
     size_t columns_cap = 0;
     uint32_t *d_part_masks = nullptr;
     size_t part_masks_cap = 0;
-    unsigned long long *d_check_fallbacks = nullptr;  // warps of the column brick kernel that took the full walk
+    // the column brick kernel's counters: [0] warps that took the full walk after a failed range check, [1] bricks its
+    // flagged columns sent to the full walk
+    unsigned long long *d_check_fallbacks = nullptr;
     uint32_t jit_max_ops = 4096;  // programs longer than this are not specialised automatically
     uint64_t constant_program = 0;  // id of the program in this device's __constant__ window
     int index = 0;                  // position in g_ctx
@@ -439,8 +441,18 @@ int prepare_columns(const cc_columns_meta &meta, cc_eval_args &a, uint64_t n_bri
     a.brick_count = meta.checks && n_bricks ? reinterpret_cast<uint32_t *>(base + list_at) : nullptr;
     a.brick_list = a.brick_count ? a.brick_count + 1 : nullptr;
     a.check_fallbacks = g.d_check_fallbacks;
+    a.flagged_bricks = g.d_check_fallbacks + 1;
     if (a.brick_count) CU(cudaMemsetAsync(a.brick_count, 0, 4, g.compute));
     return CC_OK;
+}
+
+// Bricks per CTA of the column brick kernel: CODECAD_B200_BRICK_RUN (read at every launch, so that one process can compare
+// run lengths; 1 is one brick per CTA) or CC_BRICK_RUN_DEFAULT, at most CC_BRICK_RUN_MAX and the bricks of a stack.
+uint32_t brick_run(int axis, const cc_eval_args &a)
+{
+    long run = CC_BRICK_RUN_DEFAULT;
+    if (const char *t = getenv("CODECAD_B200_BRICK_RUN")) run = atol(t);
+    return (uint32_t)std::max(1L, std::min(run, (long)std::min<uint32_t>(CC_BRICK_RUN_MAX, bricks_along(axis, a))));
 }
 
 // tiles_per_block for tiles of `tile` cells; the sinks that compact their output (CLASSIFY, MASS) also get a zeroed
@@ -553,6 +565,7 @@ int launch(int sink_kind, const cc_program *prog, cc_eval_args &a, uint64_t poin
             if (units >= (1ull << 31)) return fail(CC_ERR_INVALID_ARGUMENT, "too many bricks in one launch");
         }
         if (r.columns && (rc = prepare_columns(prog->jit_meta[r.sink], a, r.path == Path::tiles ? 0 : units))) return rc;
+        if (r.path == Path::columns) a.brick_run = brick_run(prog->jit_meta[r.sink].axis, a);
         if (r.masks && (rc = prepare_part_masks(prog, a, units))) return rc;
         if (r.path == Path::parts_interp) {
             const uint32_t *table = nullptr;
@@ -588,8 +601,8 @@ int init_context(Context &c, int device, int index)
     CU(cudaStreamCreateWithFlags(&c.copy, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&c.copy2, cudaStreamNonBlocking));
     CU(cudaMallocHost(&c.h_word, 64));
-    CU(cudaMalloc(&c.d_check_fallbacks, sizeof(unsigned long long)));
-    CU(cudaMemset(c.d_check_fallbacks, 0, sizeof(unsigned long long)));
+    CU(cudaMalloc(&c.d_check_fallbacks, 2 * sizeof(unsigned long long)));
+    CU(cudaMemset(c.d_check_fallbacks, 0, 2 * sizeof(unsigned long long)));
     {
         // keep freed work-list memory in the pool instead of returning it to the driver at every sync
         cudaMemPool_t pool = nullptr;
@@ -852,11 +865,12 @@ void cc_reset_counters(void)
     if (g_n_ctx == 0 || cudaGetDevice(&dev) != cudaSuccess) return;
     for (int i = 0; i < g_n_ctx; ++i)
         if (g_ctx[i].d_check_fallbacks && cudaSetDevice(g_ctx[i].device) == cudaSuccess)
-            cudaMemsetAsync(g_ctx[i].d_check_fallbacks, 0, sizeof(unsigned long long), g_ctx[i].compute);
+            cudaMemsetAsync(g_ctx[i].d_check_fallbacks, 0, 2 * sizeof(unsigned long long), g_ctx[i].compute);
     cudaSetDevice(dev);
 }
 
-int cc_get_check_fallbacks(uint64_t *warps)
+// counter k of the column brick kernel (Context::d_check_fallbacks), summed over the devices
+static int column_counter(int k, uint64_t *out)
 {
     NEED_INIT();
     uint64_t n = 0;
@@ -864,14 +878,18 @@ int cc_get_check_fallbacks(uint64_t *warps)
         Context &c = g_ctx[i];
         unsigned long long v = 0;
         CU(cudaSetDevice(c.device));
-        CU(cudaMemcpyAsync(&v, c.d_check_fallbacks, sizeof v, cudaMemcpyDeviceToHost, c.compute));
+        CU(cudaMemcpyAsync(&v, c.d_check_fallbacks + k, sizeof v, cudaMemcpyDeviceToHost, c.compute));
         CU(cudaStreamSynchronize(c.compute));
         n += v;
     }
     CU(cudaSetDevice(g.device));
-    if (warps) *warps = n;
+    if (out) *out = n;
     return CC_OK;
 }
+
+int cc_get_check_fallbacks(uint64_t *warps) { return column_counter(0, warps); }
+
+int cc_get_flagged_bricks(uint64_t *bricks) { return column_counter(1, bricks); }
 
 int cc_set_tuning(int points_per_thread, int program_space)
 {

@@ -355,22 +355,36 @@ CC_DEV bool cc_col_locate(const cc_eval_args &a, uint32_t block, const uint32_t 
     return a.column_flags ? __syncthreads_or(flagged) != 0 : false;
 }
 
-// The brick kernel of cc_kernel_body_bricks with the thread's columns at hand.  With CC_COL_PAIR the two cells of a
-// thread differ only along the columns' axis (z-columns: z and z + 8, a warp's store is four 128-byte runs; y-columns:
-// y and y + 4; x-columns: the brick order's x and x + 4 already), so they share one column record.
-// EVAL (the generated SceneTile): `loop` is the per-cell body and its column reference; with EVAL::deferred its ops fold
-// their range tests into `range` instead of voting per op (DESIGN.md 4.10), and a warp in which some lane flags
-// evaluates its cells again with EVAL::full, the guarded full walk.
-template <int PTS, class EVAL>
-CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
+// The runs of the column brick kernel.  The bricks of one set of columns form a stack along the columns' axis; a stack is
+// cut into runs of a.brick_run bricks (the last one shorter).  Run `run` starts at brick `first` (its corner x0, y0, z0),
+// holds `n` bricks, and its next brick is `stride` bricks further in the z-fastest brick order.
+CC_DEV void cc_brick_run_of(const cc_eval_args &a, uint32_t run, uint32_t &first, uint32_t &n, uint32_t &stride, uint32_t &x0,
+                            uint32_t &y0, uint32_t &z0)
 {
-    static_assert(PTS == 2 && CC_THREADS * PTS == CC_BRICK_X * CC_BRICK_Y * CC_BRICK_Z, "one brick per CTA");
-    typedef typename cc_pts<PTS>::V V;
-    uint32_t x0, y0, z0;
-    cc_brick_of(a, blockIdx.x, x0, y0, z0);
+    const uint32_t nbx = (a.nx + CC_BRICK_X - 1) / CC_BRICK_X, nby = (a.ny + CC_BRICK_Y - 1) / CC_BRICK_Y,
+                   nbz = (a.nz + CC_BRICK_Z - 1) / CC_BRICK_Z;
+    const uint32_t along = CC_COL_AXIS == 0 ? nbx : CC_COL_AXIS == 1 ? nby : nbz;
+    const uint32_t per_stack = (along + a.brick_run - 1) / a.brick_run;
+    const uint32_t stack = run / per_stack, start = (run - stack * per_stack) * a.brick_run;
+    n = min(a.brick_run, along - start);
+    // the stack's two other brick coordinates, numbered in the brick order (z fastest)
+    const uint32_t other = CC_COL_AXIS == 2 ? nby : nbz, s1 = stack / other, s0 = stack - s1 * other;
+    const uint32_t bx = CC_COL_AXIS == 0 ? start : s1, by = CC_COL_AXIS == 0 ? s1 : CC_COL_AXIS == 1 ? start : s0,
+                   bz = CC_COL_AXIS == 2 ? start : s0;
+    first = (bx * nby + by) * nbz + bz;
+    stride = CC_COL_AXIS == 0 ? nby * nbz : CC_COL_AXIS == 1 ? nbz : 1u;
+    x0 = bx * CC_BRICK_X;
+    y0 = by * CC_BRICK_Y;
+    z0 = bz * CC_BRICK_Z;
+}
+
+// The brick kernel of cc_kernel_body_bricks with the thread's columns at hand: the cells of a thread in the brick at
+// (x0, y0, z0).  With CC_COL_PAIR the two cells of a thread differ only along the columns' axis (z-columns: z and z + 8, a warp's store is four 128-byte runs; y-columns:
+// y and y + 4; x-columns: the brick order's x and x + 4 already), so they share one column record.
+template <int PTS>
+CC_DEV void cc_brick_col_cells(uint32_t x0, uint32_t y0, uint32_t z0, uint32_t (&ix)[PTS], uint32_t (&iy)[PTS], uint32_t (&iz)[PTS])
+{
     const uint32_t tid = threadIdx.x;
-    uint32_t ix[PTS], iy[PTS], iz[PTS], col[PTS];
-    float gx[PTS], gy[PTS], gz[PTS];
 #pragma unroll
     for (int j = 0; j < PTS; ++j) {
         const uint32_t c = (uint32_t)j * CC_THREADS + tid;
@@ -386,11 +400,37 @@ CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
             iy[j] = y0 + ((tid >> 4) & 3u) + 4u * (uint32_t)j;
             iz[j] = z0 + (tid & 15u);
         }
-        gx[j] = cc_fma(a.step, (float)(ix[j] + a.x_offset), a.cx);
-        gy[j] = cc_fma(a.step, (float)iy[j], a.cy);
-        gz[j] = cc_fma(a.step, (float)iz[j], a.cz);
-        const uint32_t u = CC_COL_AXIS == 0 ? iy[j] : ix[j], v = CC_COL_AXIS == 2 ? iy[j] : iz[j];
-        col[j] = min(u, cc_col_dim_u(a) - 1u) * cc_col_dim_v(a) + min(v, cc_col_dim_v(a) - 1u);  // (cells past the edge read a neighbour's column)
+    }
+}
+
+// A CTA walks a run of bricks along the columns' axis (cc_brick_run_of).  The bricks of a run read the same columns, so
+// the run's position, the thread's column record and the column flags are worked out once per run, and the run's part
+// masks come in with one load into shared memory.  Per brick the cells' indices and coordinates are rebuilt from the
+// brick's corner (a few integer ops and three FMAs per cell: cheaper than keeping them in registers across the per-cell
+// body), then the mask, the per-cell body and the stores; the warps go through the run without waiting for each other.
+// EVAL (the generated SceneTile): `loop` is the per-cell body, its part mask and its column reference; with
+// EVAL::deferred its ops fold their range tests into `range` instead of voting per op (DESIGN.md 4.10), and a warp in
+// which some lane flags evaluates its cells again with EVAL::full, the guarded full walk.
+template <int PTS, class EVAL>
+CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
+{
+    static_assert(PTS == 2 && CC_THREADS * PTS == CC_BRICK_X * CC_BRICK_Y * CC_BRICK_Z, "one brick per CTA");
+    static_assert(CC_BRICK_RUN_MAX <= CC_THREADS, "one thread loads each mask of a run");
+    typedef typename cc_pts<PTS>::V V;
+    __shared__ uint32_t s_mask[CC_BRICK_RUN_MAX];
+    uint32_t first, n, stride, x0, y0, z0;
+    cc_brick_run_of(a, blockIdx.x, first, n, stride, x0, y0, z0);
+    const uint32_t tid = threadIdx.x;
+    if (tid < n) s_mask[tid] = a.part_masks ? a.part_masks[first + tid * stride] : 0xffffffffu;
+    uint32_t col[PTS];
+    {
+        uint32_t ix[PTS], iy[PTS], iz[PTS];
+        cc_brick_col_cells<PTS>(x0, y0, z0, ix, iy, iz);
+#pragma unroll
+        for (int j = 0; j < PTS; ++j) {
+            const uint32_t u = CC_COL_AXIS == 0 ? iy[j] : ix[j], v = CC_COL_AXIS == 2 ? iy[j] : iz[j];
+            col[j] = min(u, cc_col_dim_u(a) - 1u) * cc_col_dim_v(a) + min(v, cc_col_dim_v(a) - 1u);  // (cells past the edge read a neighbour's column)
+        }
     }
 #if CC_COL_PAIR
     eval.loop.cr.rec = reinterpret_cast<const float4 *>(a.columns) + (size_t)col[0] * CC_COL_VALUES;
@@ -403,31 +443,50 @@ CC_DEV void cc_kernel_body_brick_columns(const cc_eval_args &a, EVAL &eval)
     }
     const int col_flag = a.column_flags ? (int)(a.column_flags[col[0]] | a.column_flags[col[1]]) : 0;
 #endif
-    if (a.column_flags) {
-        // a column whose "invariant" micro-ops do see z in some bit: the whole brick takes the full walk
-        const int flagged = __syncthreads_or(col_flag);
-        if (flagged) {
-            if (tid == 0) a.brick_list[atomicAdd(a.brick_count, 1u)] = blockIdx.x;
-            return;
+    // (also the barrier behind the masks' stores)
+    if (__syncthreads_or(col_flag)) {
+        // a column whose "invariant" micro-ops do see z in some bit: every brick of the run takes the full walk
+        if (tid < 32) {
+            uint32_t at = 0;
+            if (tid == 0) {
+                at = atomicAdd(a.brick_count, n);
+                if (a.flagged_bricks) atomicAdd(a.flagged_bricks, (unsigned long long)n);
+            }
+            at = __shfl_sync(0xffffffffu, at, 0);
+            for (uint32_t i = tid; i < n; i += 32) a.brick_list[at + i] = first + i * stride;
         }
+        return;
     }
-    V vx[1], vy[1], vz[1];
-    cc_val<V> LV[1];
-    vx[0] = cc_pack<V>(gx);
-    vy[0] = cc_pack<V>(gy);
-    vz[0] = cc_pack<V>(gz);
-    uint32_t range = 0;
-    eval(vx, vy, vz, LV, range);
-    if (EVAL::deferred && __any_sync(0xffffffffu, cc_range_flagged(range))) {
-        // some op of some lane had an operand outside its fast path's range: the warp's values are thrown away
-        if ((tid & 31u) == 0 && a.check_fallbacks) atomicAdd(a.check_fallbacks, 1ull);
-        eval.full(vx, vy, vz, LV);
-    }
-    float4 *out = reinterpret_cast<float4 *>(a.out);
+    for (uint32_t i = 0; i < n; ++i) {
+        uint32_t ix[PTS], iy[PTS], iz[PTS];
+        cc_brick_col_cells<PTS>(x0 + (CC_COL_AXIS == 0 ? i * CC_BRICK_X : 0u), y0 + (CC_COL_AXIS == 1 ? i * CC_BRICK_Y : 0u),
+                                z0 + (CC_COL_AXIS == 2 ? i * CC_BRICK_Z : 0u), ix, iy, iz);
+        float gx[PTS], gy[PTS], gz[PTS];
 #pragma unroll
-    for (int j = 0; j < PTS; ++j)
-        if (ix[j] < a.nx && iy[j] < a.ny && iz[j] < a.nz)
-            __stcs(out + ((size_t)ix[j] * a.ny + iy[j]) * a.nz + iz[j], cc_lane_get(LV[0], j));  // INDEX3
+        for (int j = 0; j < PTS; ++j) {
+            gx[j] = cc_fma(a.step, (float)(ix[j] + a.x_offset), a.cx);
+            gy[j] = cc_fma(a.step, (float)iy[j], a.cy);
+            gz[j] = cc_fma(a.step, (float)iz[j], a.cz);
+        }
+        eval.loop.mask = s_mask[i];
+        V vx[1], vy[1], vz[1];
+        cc_val<V> LV[1];
+        vx[0] = cc_pack<V>(gx);
+        vy[0] = cc_pack<V>(gy);
+        vz[0] = cc_pack<V>(gz);
+        uint32_t range = 0;
+        eval(vx, vy, vz, LV, range);
+        if (EVAL::deferred && __any_sync(0xffffffffu, cc_range_flagged(range))) {
+            // some op of some lane had an operand outside its fast path's range: the warp's values are thrown away
+            if ((tid & 31u) == 0 && a.check_fallbacks) atomicAdd(a.check_fallbacks, 1ull);
+            eval.full(vx, vy, vz, LV);
+        }
+        float4 *out = reinterpret_cast<float4 *>(a.out);
+#pragma unroll
+        for (int j = 0; j < PTS; ++j)
+            if (ix[j] < a.nx && iy[j] < a.ny && iz[j] < a.nz)
+                __stcs(out + ((size_t)ix[j] * a.ny + iy[j]) * a.nz + iz[j], cc_lane_get(LV[0], j));  // INDEX3
+    }
 }
 
 template <int PTS, class EVAL>

@@ -78,12 +78,20 @@ struct cc_eval_args {
     uint32_t *brick_list, *brick_count;
     // warps of the column brick kernel whose deferred range check failed and that took the full walk (cc_body.cuh)
     unsigned long long *check_fallbacks;
+    // bricks of the column brick kernel that a flagged column sent to the full walk (cc_body.cuh)
+    unsigned long long *flagged_bricks;
+    // bricks per CTA of the column brick kernel: a run along the columns' axis, 1 .. CC_BRICK_RUN_MAX (cc_body.cuh)
+    uint32_t brick_run;
 };
 
 // bricks of the part-culling kernels: a CTA of 512 threads x 2 points
 #define CC_BRICK_X 8
 #define CC_BRICK_Y 8
 #define CC_BRICK_Z 16
+// the longest run of bricks one CTA of the column brick kernel walks, and the run it walks unless asked otherwise
+// (CODECAD_B200_BRICK_RUN)
+#define CC_BRICK_RUN_MAX 64
+#define CC_BRICK_RUN_DEFAULT 8
 
 // arguments of the image renderers (rendering/ray_caster.cl:147-156, rendering/bitmap.cl:1-3)
 struct cc_render_args {

@@ -107,6 +107,18 @@ inline uint64_t columns_along(int axis, uint32_t nx, uint32_t ny, uint32_t nz)
     return axis == 2 ? (uint64_t)nx * ny : axis == 1 ? (uint64_t)nx * nz : (uint64_t)ny * nz;
 }
 
+// bricks of the launch along `axis`
+inline uint32_t bricks_along(int axis, const cc_eval_args &a)
+{
+    return axis == 0 ? (a.nx + CC_BRICK_X - 1) / CC_BRICK_X : axis == 1 ? (a.ny + CC_BRICK_Y - 1) / CC_BRICK_Y : (a.nz + CC_BRICK_Z - 1) / CC_BRICK_Z;
+}
+// CTAs of the column brick kernel: every stack of bricks along the columns' axis in runs of a.brick_run (cc_brick_run_of)
+inline uint64_t brick_runs(int axis, const cc_eval_args &a)
+{
+    const uint64_t stacks = (uint64_t)bricks_along(0, a) * bricks_along(1, a) * bricks_along(2, a) / bricks_along(axis, a);
+    return stacks * ((bricks_along(axis, a) + a.brick_run - 1) / a.brick_run);
+}
+
 #define CC_MAX_DEVICES 16  // devices one process can drive (cc_init_devices)
 
 struct cc_program {
@@ -144,7 +156,8 @@ int cc_jit_poll(cc_program *prog, int sink, bool wait, std::string *err);
 void cc_jit_release(cc_program *prog);
 // dev_index = index of the library context (device) the launch goes to
 int cc_jit_launch(const cc_program *prog, int sink, const cc_eval_args &a, void *stream, int dev_index);
-// the brick and tile units (CC_SINK_PARTS, CC_SINK_COLUMNS, CC_SINK_TILES_*) over `n_units` bricks or tiles, one CTA each:
+// the brick and tile units (CC_SINK_PARTS, CC_SINK_COLUMNS, CC_SINK_TILES_*) over `n_units` bricks or tiles, one CTA each
+// (CC_SINK_COLUMNS: one CTA per run of a.brick_run bricks, brick_runs):
 // [centres ->] [column pass ->] main kernel [-> full walk of the flagged bricks].  A companion runs where the unit has it and
 // the caller prepared its buffer (a.part_masks, a.columns, a.column_flags); `centers_only` stops after the centres.
 int cc_jit_launch_units(const cc_program *prog, int sink, const cc_eval_args &a, uint64_t n_units, int sm_count, void *stream,

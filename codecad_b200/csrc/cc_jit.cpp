@@ -771,7 +771,7 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
           << "    cc_column_profiles_body<PTS>(a, e);\n}\n";
     if (columns_mode && !tiles) {
         s << "extern \"C\" __global__ void __launch_bounds__(" << bounds << ") cc_jit_columns" << head
-          << "    SceneTile e;\n    e.loop.sm = cc_cells + threadIdx.x;\n    e.loop.mask = a.part_masks ? a.part_masks[blockIdx.x] : 0xffffffffu;\n"
+          << "    SceneTile e;\n    e.loop.sm = cc_cells + threadIdx.x;  // (the part mask: per brick of the CTA's run)\n"
           << "    cc_kernel_body_brick_columns<PTS>(a, e);\n}\n"
           << "extern \"C\" __global__ void __launch_bounds__(" << bounds << ") cc_jit_columns_full" << head
           << "    const unsigned n = *a.brick_count;\n    for (unsigned i = blockIdx.x; i < n; i += gridDim.x) {\n"
@@ -1376,7 +1376,9 @@ int cc_jit_launch_units(const cc_program *prog, int sink, const cc_eval_args &a,
         const uint64_t ncol = std::max(1u, a.n_blocks) * columns_along(prog->jit_meta[sink].axis, a.nx, a.ny, a.nz);
         if ((ce = run(aux[CC_AUX_COLUMNS], (ncol + pair - 1) / pair)) != cudaSuccess) return (int)ce;
     }
-    if ((ce = run(prog->jit_kernel[sink], n_units)) != cudaSuccess) return (int)ce;
+    // (the column brick kernel: one CTA per run of a.brick_run bricks along the columns' axis)
+    const uint64_t grid = sink == CC_SINK_COLUMNS ? brick_runs(prog->jit_meta[sink].axis, a) : n_units;
+    if ((ce = run(prog->jit_kernel[sink], grid)) != cudaSuccess) return (int)ce;
     if (aux[CC_AUX_FULL] && a.column_flags) ce = run(aux[CC_AUX_FULL], (uint64_t)std::max(1, 2 * sm_count));
     return (int)ce;
 }

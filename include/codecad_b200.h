@@ -75,6 +75,9 @@ void cc_reset_counters(void);
  * range check failed, so that they evaluated their cells again with the guarded full walk; waits
  * for the work queued so far. */
 int cc_get_check_fallbacks(uint64_t *warps);
+/* bricks of the column brick kernel since cc_init / the last reset that a column failing its run-time
+ * check sent to the full walk (DESIGN.md 4.10); waits for the work queued so far. */
+int cc_get_flagged_bricks(uint64_t *bricks);
 /* tuning knobs, mainly for bench.py / profiling: points per thread (1,2,4; 0 = auto),
  * and where the microcode is fetched from (0 = auto, 1 = __constant__, 2 = shared). */
 int cc_set_tuning(int points_per_thread, int program_space);
