@@ -403,6 +403,38 @@ CC_DEV void cc_brick_col_cells(uint32_t x0, uint32_t y0, uint32_t z0, uint32_t (
     }
 }
 
+// The lazy gradient of the column brick kernel (DESIGN.md 4.10): its per-cell body carries a distance and the id of the
+// leaf it came from through the ops (the sweep), then the winning leaf of each cell is evaluated again in full and taken
+// along its one path to the root (the replay, REPLAY::leaf).  0 keeps the eager body; CC_LAZY_CHECK=1 poisons a cell
+// whose replayed .w differs in any bit from the sweep's.
+#ifndef CC_LAZY_GRADIENT
+#define CC_LAZY_GRADIENT 1
+#endif
+#ifndef CC_LAZY_CHECK
+#define CC_LAZY_CHECK 0
+#endif
+// Both cells of the thread won by one leaf: one packed replay.  Otherwise one packed replay per leaf, each keeping its lane.
+template <class REPLAY, class V, int G>
+CC_DEV void cc_lazy_replay(const REPLAY &r, const V (&gx)[G], const V (&gy)[G], const V (&gz)[G], const V (&w)[G], const V (&id)[G],
+                           cc_val<V> (&L)[G])
+{
+    static_assert(G * cc_lane<V>::N == 2, "two points per thread");
+    constexpr int N = cc_lane<V>::N;
+    const int k0 = (int)vlane(id[0], 0), k1 = (int)vlane(id[G - 1], N - 1);
+    auto take = [&](const cc_val<V> (&T)[G], int j) {
+        float4 t = cc_lane_get(T[j / N], j % N);
+        const float sw = vlane(w[j / N], j % N);
+        if (CC_LAZY_CHECK && __float_as_uint(t.w) != __float_as_uint(sw)) t.x = t.y = t.z = __uint_as_float(0x7fbadbadu);
+        t.w = sw;
+        cc_lane_put(L[j / N], j % N, t);
+    };
+    cc_val<V> T[G];
+    r.leaf(k0, gx, gy, gz, T);
+    take(T, 0);
+    if (k1 != k0) r.leaf(k1, gx, gy, gz, T);
+    take(T, 1);
+}
+
 // A CTA walks a run of bricks along the columns' axis (cc_brick_run_of).  The bricks of a run read the same columns, so
 // the run's position, the thread's column record and the column flags are worked out once per run, and the run's part
 // masks come in with one load into shared memory.  Per brick the cells' indices and coordinates are rebuilt from the

@@ -402,6 +402,31 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
             }
         }
 
+    // the lazy gradient of the columns unit's per-cell body (DESIGN.md 4.10).  The sweep runs the body's ops with a
+    // distance and a leaf id per cell in place of each distance value (points stay whole), and the replay has one case
+    // per leaf: the leaf's value rebuilt from the cell's coordinates and its column record, then the ops that change
+    // a gradient on the leaf's one path to the root.  `lazy` stays true while every per-cell op has such a form and
+    // every leaf reaches the root along exactly one path.
+    bool lazy = column_unit && !coord_smem;
+    std::ostringstream sweep, sweep_hoisted;
+    int sweep_open = -1;
+    std::vector<char> dist_after, dist_iv(iv.size(), 0);  // per micro-op / interval: a distance (else a point)
+    struct Path {
+        int leaf;
+        std::vector<int> chain;  // op index of a transformation_from, ~op index of a subtrahend's negation
+    };
+    typedef std::vector<Path> Paths;
+    Paths l_paths;                   // the leaves the sweep's running distance may hold
+    std::vector<Paths> iv_paths(iv.size());
+    std::string l_recipe;            // statements that rebuild the running point into L ("" = unknown)
+    std::vector<std::string> iv_recipe(iv.size()), op_core((size_t)n_ops_total + 1), leaf_text;
+    bool l_dist = false;
+    auto new_leaf = [&](const std::string &text) {
+        leaf_text.push_back(text);
+        return (int)leaf_text.size() - 1;
+    };
+    auto set_id = [](int leaf) { return "CC_EACH Li[g] = vbc<V>(" + std::to_string(leaf) + ".0f);\n"; };
+
     uint32_t pc = 0;
     for (int op_index = 0;; ++op_index) {
         if (pc >= c.size()) {
@@ -414,7 +439,7 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
         }
         const uint32_t h = c[pc], op = CC_HDR_OP(h), src_slot = CC_HDR_SRC(h), dst = CC_HDR_DST(h);
         if (columns_mode) o.str(std::string());  // one micro-op at a time: its text goes to one body or both
-        std::string split_fused, split_a, split_b;  // a fused primitive cut in two (cc_columns::split_prim)
+        std::string split_fused, split_a, split_b, split_sweep;  // a fused primitive cut in two (cc_columns::split_prim)
         o << "        // pc " << pc << "\n";
         const int my_part = (parts_mode && op != MOP_RETURN && (size_t)op_index < parts.part_of_op.size()) ? parts.part_of_op[(size_t)op_index] : -1;
         const bool tree_union = parts_mode && op == MOP_UNION && (size_t)op_index < parts.union_a.size() &&
@@ -439,6 +464,7 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
             }
         }
         if (columns_mode) o << tree_union_open;  // (after the operand fetch: the other branch needs it too)
+        const size_t core_at = lazy ? o.str().size() : 0;
         switch (op) {
         case MOP_RETURN: break;
         case MOP_NOP: break;
@@ -475,6 +501,10 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
                     split_a = "        {\n          CC_EACH L[g] = " + to + ";\n" + profile + "          CC_EACH cc_col_store(cr, " + k + "u, L[g]);\n        }\n";
                     split_b = "        {\n          V pz_[G];\n          CC_EACH { const Val p_ = " + to + "; pz_[g] = p_.z; L[g] = cc_col_load<V>(cr, " + k +
                               "u); }\n" + tail;
+                    const std::string scaled = g.value(pc + 26) == 1.0f ? "w_" : "vmul(w_, vbc<V>(" + g.F(pc + 26) + "))";
+                    split_sweep = "        {\n          V pz_[G];\n          CC_EACH { const Val p_ = " + to + "; pz_[g] = p_.z; Lw[g] = cc_col_load<V>(cr, " + k +
+                                  "u).w; }\n          cc_extrusion_dist(" + g.F(pc + 15) + ", Lw, pz_, range);\n          CC_EACH { const V w_ = vsub(Lw[g], vbc<V>(" +
+                                  g.F(pc + 16) + ")); Lw[g] = " + scaled + "; }\n        }\n";
                 }
             }
             break;
@@ -541,6 +571,19 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
         default:
             *err = "internal: unknown micro-op " + std::to_string(op);
             return CC_ERR_INVALID_PROGRAM;
+        }
+        if (lazy) op_core[(size_t)op_index] = o.str().substr(core_at);
+        {
+            bool d = true;  // what L holds after this op
+            switch (op) {
+            case MOP_T_INIT: case MOP_T_INIT_M: case MOP_T_TO: case MOP_T_TO_M: case MOP_MIRROR: case MOP_SYM_TO:
+            case MOP_REV_TO: case MOP_TWIST_TO: case MOP_CREP_TO: case MOP_REPETITION: d = false; break;
+            case MOP_LOAD: d = dist_iv[(size_t)op_use[op_index]] != 0; break;
+            case MOP_NOP: case MOP_RETURN: d = dist_after.empty() ? false : dist_after.back() != 0; break;
+            default: break;
+            }
+            dist_after.push_back(d);
+            if (op_def[op_index] >= 0) dist_iv[(size_t)op_def[op_index]] = d;
         }
         if (op == MOP_RETURN) break;
         if (stop_after >= 0 && ++n_emitted > stop_after) break;
@@ -617,6 +660,181 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
                             std::to_string(carried_interval[(size_t)u]) + "u);\n";
                 put(in_loop, loop_open, my_part, fetch + text_loop);
             }
+            if ((ph & 2) && lazy) {
+                // the sweep's text of this op, the same control flow as the per-cell body's
+                std::ostringstream t;
+                const int from = cols.restore_from[(size_t)op_index];
+                int restored = -1;  // column value restored as the profile of this op's extrusion
+                if (from >= 0) {
+                    const std::string k = std::to_string(carried_l[(size_t)from]);
+                    const int from_part = (size_t)from < parts.part_of_op.size() && parts_mode ? parts.part_of_op[(size_t)from] : -1;
+                    const std::string load = "CC_EACH L[g] = cc_col_load<V>(cr, " + k + "u);\n";
+                    l_dist = dist_after[(size_t)from] != 0;
+                    if (!l_dist) {
+                        l_recipe = load;
+                        put(sweep, sweep_open, from_part, "        " + load);
+                    } else if (op == MOP_EXTRUSION) {
+                        restored = carried_l[(size_t)from];
+                        l_paths.clear();
+                        put(sweep, sweep_open, from_part, "        CC_EACH Lw[g] = cc_col_load<V>(cr, " + k + "u).w;\n");
+                    } else {
+                        const int leaf = new_leaf(load);
+                        l_paths = Paths{Path{leaf, {}}};
+                        put(sweep, sweep_open, from_part, "        CC_EACH Lw[g] = cc_col_load<V>(cr, " + k + "u).w;\n        " + set_id(leaf));
+                    }
+                }
+                // the operand: a distance (Bw, Bi and its paths) or a point (Bp and its recipe)
+                const int u = op_use[op_index];
+                const bool b_dist = u >= 0 && dist_iv[(size_t)u];
+                std::string Bw, Bi, Bp, b_recipe;
+                Paths b_paths;
+                if (u >= 0) {
+                    const std::string us = std::to_string(u), is = std::to_string(op_index);
+                    if (iv[u].carried) {
+                        const std::string k = std::to_string(carried_interval[(size_t)u]);
+                        if (b_dist) {
+                            const int leaf = new_leaf("CC_EACH L[g] = cc_col_load<V>(cr, " + k + "u);\n");
+                            b_paths = Paths{Path{leaf, {}}};
+                            t << "        V Iw" << us << "[G], Ii" << us << "[G]; CC_EACH { Iw" << us << "[g] = cc_col_load<V>(cr, " << k << "u).w; Ii" << us
+                              << "[g] = vbc<V>(" << leaf << ".0f); }\n";
+                            Bw = "Iw" + us + "[g]", Bi = "Ii" + us + "[g]";
+                        } else {
+                            t << "        Val I" << us << "[G]; CC_EACH I" << us << "[g] = cc_col_load<V>(cr, " << k << "u);\n";
+                            Bp = "I" + us + "[g]";
+                            b_recipe = "CC_EACH L[g] = cc_col_load<V>(cr, " + k + "u);\n";
+                        }
+                    } else if (b_dist) {
+                        b_paths = iv_paths[(size_t)u];
+                        if (iv[u].cell < 0) {
+                            Bw = "Iw" + us + "[g]", Bi = "Ii" + us + "[g]";
+                        } else {
+                            t << "        V Bw" << is << "[G], Bi" << is << "[G]; CC_EACH cc_slot_load_wi_opaque(CC_CELL(" << iv[u].cell << ", g), Bw" << is
+                              << "[g], Bi" << is << "[g]);\n";
+                            Bw = "Bw" + is + "[g]", Bi = "Bi" + is + "[g]";
+                        }
+                    } else {
+                        b_recipe = iv_recipe[(size_t)u];
+                        if (iv[u].cell < 0) {
+                            Bp = "I" + us + "[g]";
+                        } else {  // (the per-cell body's fetch)
+                            t << "        Val B" << is << "[G]; CC_EACH "
+                              << (op == MOP_EXTRUSION ? "cc_slot_load_z_opaque(CC_CELL(" : "cc_slot_load_opaque(CC_CELL(") << iv[u].cell << ", g), B" << is
+                              << "[g]" << (op == MOP_EXTRUSION ? ".z" : "") << ");\n";
+                            Bp = "B" + is + "[g]";
+                        }
+                    }
+                }
+                t << tree_union_open;
+                auto leaves_of = [](const Paths &p) { std::vector<int> r; for (const Path &x : p) r.push_back(x.leaf); return r; };
+                const std::string from_w = g.value(pc + 10) == 1.0f ? "Lw[g]" : "vmul(Lw[g], vbc<V>(" + g.F(pc + 10) + "))";
+                switch (op) {
+                case MOP_NOP: break;
+                case MOP_LOAD:
+                    if (b_dist) {
+                        t << "        CC_EACH { Lw[g] = " << Bw << "; Li[g] = " << Bi << "; }\n";
+                        l_paths = b_paths;
+                    } else {
+                        t << "        CC_EACH L[g] = " << Bp << ";\n";
+                        l_recipe = b_recipe;
+                    }
+                    l_dist = b_dist;
+                    break;
+                case MOP_T_INIT: case MOP_T_INIT_M:
+                    t << op_core[(size_t)op_index];
+                    l_recipe = op_core[(size_t)op_index];
+                    l_dist = false;
+                    break;
+                case MOP_T_TO: case MOP_T_TO_M: case MOP_MIRROR: case MOP_SYM_TO:
+                    if (l_dist || l_recipe.empty()) lazy = false;
+                    t << op_core[(size_t)op_index];
+                    l_recipe += op_core[(size_t)op_index];
+                    break;
+                case MOP_SPHERE: {
+                    if (l_dist || l_recipe.empty()) lazy = false;
+                    const int leaf = new_leaf(l_recipe + op_core[(size_t)op_index]);
+                    t << "        cc_sphere_dist(" << g.F(pc + 1) << ", L, Lw, range);\n        " << set_id(leaf);
+                    l_paths = Paths{Path{leaf, {}}};
+                    l_dist = true;
+                    break;
+                }
+                case MOP_EXTRUSION: {
+                    if (restored < 0 || u < 0 || b_dist || b_recipe.empty()) lazy = false;
+                    const int leaf = new_leaf("{\n        Val Q[G];\n        {\n" + b_recipe + "        CC_EACH Q[g] = L[g];\n        }\n        CC_EACH L[g] = cc_col_load<V>(cr, " +
+                                              std::to_string(restored) + "u);\n        { V cz[G]; CC_EACH cz[g] = Q[g].z; cc_extrusion_n(" + g.F(pc + 1) + ", L, cz); }\n        }\n");
+                    t << "        { V cz[G]; CC_EACH cz[g] = " << Bp << ".z; cc_extrusion_dist(" << g.F(pc + 1) << ", Lw, cz, range); }\n        " << set_id(leaf);
+                    l_paths = Paths{Path{leaf, {}}};
+                    l_dist = true;
+                    break;
+                }
+                case MOP_PRIM_CIRCLE: case MOP_PRIM_RECT: case MOP_PRIM_CIRCLE_M: case MOP_PRIM_RECT_M: {
+                    if (split_sweep.empty()) {
+                        lazy = false;
+                        break;
+                    }
+                    const int leaf = new_leaf(split_b);
+                    t << split_sweep << "        " << set_id(leaf);
+                    l_paths = Paths{Path{leaf, {}}};
+                    l_dist = true;
+                    break;
+                }
+                case MOP_OFFSET:
+                    if (!l_dist) lazy = false;
+                    t << "        CC_EACH Lw[g] = vsub(Lw[g], vbc<V>(" << g.F(pc + 1) << "));\n";
+                    break;
+                case MOP_T_FROM: case MOP_T_FROM_M:
+                    if (!l_dist) lazy = false;
+                    if (from_w != "Lw[g]") t << "        CC_EACH Lw[g] = " << from_w << ";\n";
+                    for (Path &p : l_paths) p.chain.push_back(op_index);
+                    break;
+                case MOP_UNION: case MOP_ISECT: case MOP_SUB: {
+                    if (!l_dist || !b_dist || l_paths.empty() || b_paths.empty()) {
+                        lazy = false;
+                        break;
+                    }
+                    for (int a : leaves_of(l_paths))
+                        for (int b : leaves_of(b_paths))
+                            if (a == b) lazy = false;  // a value reaching the root along two paths
+                    const std::string pred = op == MOP_UNION ? "vlt(Lw[g], " + Bw + ")" : op == MOP_ISECT ? "vlt(vneg(Lw[g]), vneg(" + Bw + "))"
+                                                                                                         : "vlt(vneg(Lw[g]), " + Bw + ")";
+                    const std::string other = op == MOP_SUB ? "vneg(" + Bw + ")" : Bw;
+                    t << "        CC_EACH { const auto m_ = " << pred << "; Lw[g] = vsel(m_, Lw[g], " << other << "); Li[g] = vsel(m_, Li[g], " << Bi << "); }\n";
+                    for (Path p : b_paths) {
+                        if (op == MOP_SUB) p.chain.push_back(~op_index);
+                        l_paths.push_back(p);
+                    }
+                    break;
+                }
+                default:
+                    lazy = false;
+                    break;
+                }
+                if (tree_union) t << "        } else if (!(mask & " << parts.union_b[(size_t)op_index] << "u)) {\n        CC_EACH { Lw[g] = " << Bw << "; Li[g] = " << Bi << "; }\n        }\n";
+                const int d = op_def[op_index];
+                if (d >= 0 && iv[d].last_read != iv[d].def) {
+                    const std::string ds = std::to_string(d);
+                    if ((dist_iv[(size_t)d] != 0) != l_dist) lazy = false;
+                    if (l_dist) {
+                        iv_paths[(size_t)d] = l_paths;
+                        if (iv[d].cell < 0) {
+                            sweep_hoisted << "        V Iw" << ds << "[G], Ii" << ds << "[G];\n";
+                            t << "        CC_EACH { Iw" << ds << "[g] = Lw[g]; Ii" << ds << "[g] = Li[g]; }\n";
+                        } else {
+                            t << "        CC_EACH cc_slot_store_wi(CC_CELL(" << iv[d].cell << ", g), Lw[g], Li[g]);\n";
+                        }
+                    } else {
+                        iv_recipe[(size_t)d] = l_recipe;
+                        if (iv[d].cell < 0) {
+                            sweep_hoisted << "        Val I" << ds << "[G];\n";
+                            t << "        CC_EACH I" << ds << "[g] = L[g];\n";
+                        } else if (iv[d].z_only) {
+                            t << "        CC_EACH cc_slot_store_z(CC_CELL(" << iv[d].cell << ", g), L[g].z);\n";
+                        } else {
+                            t << "        CC_EACH cc_slot_store(CC_CELL(" << iv[d].cell << ", g), L[g]);\n";
+                        }
+                    }
+                }
+                put(sweep, sweep_open, my_part, t.str());
+            }
         }
         pc += CC_HDR_LEN(h);
     }
@@ -668,19 +886,63 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
           << "        bool ok = true;\n" << chk.str() << "        return ok;\n    }\n"
           << "    __device__ __forceinline__ void operator()" << sig << ") const\n    {\n" << hoisted.str() << "        Val L[G];\n" << zero_l
           << ahead.str() << "    }\n};\n";
-        std::string loop_text = in_loop.str();
-        if (column_unit && defer_checks)  // the deferred forms: the same calls with the accumulator as a last argument
+        auto defer_calls = [](std::string &text) {  // the deferred forms: the same calls with the accumulator as a last argument
             for (const char *f : {"cc_extrusion_n(", "cc_circle_n(", "cc_rectangle_n(", "cc_sphere_n("})
-                for (size_t at = loop_text.find(f); at != std::string::npos; at = loop_text.find(f, at + 1)) {
-                    const size_t close = loop_text.find(");", at);
-                    loop_text.insert(close, ", range");
+                for (size_t at = text.find(f); at != std::string::npos; at = text.find(f, at + 1)) {
+                    const size_t close = text.find(");", at);
+                    text.insert(close, ", range");
                 }
+        };
+        std::string loop_text = in_loop.str();
+        if (column_unit && defer_checks) defer_calls(loop_text);
         s << "// per cell: the rest, reading the column's values" << (column_unit && defer_checks ? "; the range checks go into `range`" : "") << "\n"
           << "struct SceneEval {\n    float4 *sm;\n    unsigned mask;\n    " << (column_unit ? "cc_brick_col_ref" : "cc_col_ref") << " cr;\n"
           << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]" << (column_unit ? ", unsigned &range" : "") << ") const\n    {\n"
           << (column_unit ? "        (void)range;\n" : "") << hoisted.str() << zero_l << loop_text;
         if (cols.root_restore >= 0) s << "        CC_EACH L[g] = cc_col_load<V>(cr, " << carried_l[(size_t)cols.root_restore] << "u);\n";
         s << "    }\n};\n";
+        lazy = lazy && defer_checks;
+        std::ostringstream lazy_text;
+        if (lazy) {
+            if (sweep_open >= 0) sweep << "        }\n";
+            if (cols.root_restore >= 0) {
+                const std::string load = "CC_EACH L[g] = cc_col_load<V>(cr, " + std::to_string(carried_l[(size_t)cols.root_restore]) + "u);\n";
+                l_dist = dist_after[(size_t)cols.root_restore] != 0;
+                const int leaf = new_leaf(load);
+                l_paths = Paths{Path{leaf, {}}};
+                sweep << "        CC_EACH Lw[g] = cc_col_load<V>(cr, " << carried_l[(size_t)cols.root_restore] << "u).w;\n        " << set_id(leaf);
+            }
+            // every leaf reaches the root, along one path (a second one would have met the first in a union)
+            lazy = l_dist && l_paths.size() == leaf_text.size();
+        }
+        if (lazy) {
+            std::vector<const Path *> path_of(leaf_text.size(), nullptr);
+            for (const Path &p : l_paths) path_of[(size_t)p.leaf] = &p;
+            std::string cases;
+            for (size_t k = 0; k < leaf_text.size(); ++k) {
+                cases += "        case " + std::to_string(k) + ": {\n        " + leaf_text[k];
+                for (int op_at : path_of[k]->chain)
+                    cases += op_at >= 0 ? op_core[(size_t)op_at] : "        CC_EACH L[g] = cc_val_neg(L[g]);  // subtrahend (pc " + std::to_string(~op_at) + ")\n";
+                cases += "        break;\n        }\n";
+            }
+            defer_calls(cases);
+            lazy_text << "// the lazy gradient (DESIGN.md 4.10), the sweep: the per-cell body's ops on a distance and a leaf id per cell\n"
+              << "struct SceneSweep {\n    float4 *sm;\n    unsigned mask;\n    cc_brick_col_ref cr;\n"
+              << "    __device__ __forceinline__ void operator()" << sig << ", V (&Lw)[G], V (&Li)[G], unsigned &range) const\n    {\n"
+              << "        Val L[G];  // a point\n" << sweep_hoisted.str() << "        CC_EACH { Lw[g] = vbc<V>(0.f); Li[g] = vbc<V>(-1.f); }\n"
+              << sweep.str() << "    }\n};\n"
+              << "// the replay: leaf k's value from the cell's coordinates and column record, along its path to the root (out of line:\n"
+              << "// one copy for both cells of a thread, and nothing of it hoisted into the sweep)\n"
+              << "static __device__ __noinline__ SceneVals cc_replay_leaf(int k, const cc_brick_col_ref cr, const ScenePts p)\n{\n"
+              << "    SceneVals r;\n    Val (&L)[G] = r.L;\n    const V (&gx)[G] = p.x, (&gy)[G] = p.y, (&gz)[G] = p.z;\n"
+              << "    unsigned range = 0;\n    (void)range;\n    switch (k) {\n" << cases
+              << "    default:  // (the body's initial zero)\n"
+              << "        CC_EACH L[g] = Val{vbc<V>(0.f), vbc<V>(0.f), vbc<V>(0.f), vbc<V>(0.f)};\n        break;\n    }\n    return r;\n}\n"
+              << "struct SceneReplay {\n    cc_brick_col_ref cr;\n"
+              << "    __device__ __forceinline__ void leaf(int k, " << sig.substr(1) << ", Val (&L)[G]) const\n    {\n"
+              << "        ScenePts p;\n        CC_EACH { p.x[g] = gx[g]; p.y[g] = gy[g]; p.z[g] = gz[g]; }\n"
+              << "        const SceneVals r = cc_replay_leaf(k, cr, p);\n        CC_EACH L[g] = r.L[g];\n    }\n};\n";
+        }
         if (tiles)
             s << "// the hierarchy sinks (blocks x linear tiles): the rest per cell, or the full walk for a tile with a flagged column\n"
               << "struct SceneTile {\n    SceneEval loop;\n    SceneFull full;\n    bool use_full;\n"
@@ -699,10 +961,17 @@ int generate(const cc_decoded &dec, const cc_jit_cfg &cfg, unsigned sink_mask, s
               << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G]) const\n    {\n"
               << "        ScenePts p;\n        CC_EACH { p.x[g] = gx[g]; p.y[g] = gy[g]; p.z[g] = gz[g]; }\n"
               << "        const SceneVals r = cc_full_walk(sm, mask, p);\n        CC_EACH L[g] = r.L[g];\n    }\n};\n"
+              << lazy_text.str()
               << "// the brick kernel (cc_kernel_body_brick_columns): the rest per cell, or the full walk for a warp in which a range check failed\n"
               << "struct SceneTile {\n    SceneEval loop;\n"
               << "    static constexpr bool deferred = " << (defer_checks ? "CC_DEFER_CHECKS != 0" : "false") << ";\n"
-              << "    __device__ __forceinline__ void operator()" << sig << ", Val (&L)[G], unsigned &range) const { loop(gx, gy, gz, L, range); }\n"
+              << (!lazy ? "    __device__ __forceinline__ void operator()" + sig + ", Val (&L)[G], unsigned &range) const { loop(gx, gy, gz, L, range); }\n" :
+                  "    __device__ __forceinline__ void operator()" + sig + ", Val (&L)[G], unsigned &range) const\n    {\n"
+                  "#if CC_LAZY_GRADIENT && CC_DEFER_CHECKS\n"
+                  "        V w[G], id[G];\n        SceneSweep{loop.sm, loop.mask, loop.cr}(gx, gy, gz, w, id, range);\n"
+                  "        if (!__any_sync(0xffffffffu, cc_range_flagged(range)))  // (a warp that flags takes the full walk)\n"
+                  "            cc_lazy_replay(SceneReplay{loop.cr}, gx, gy, gz, w, id, L);\n"
+                  "#else\n        loop(gx, gy, gz, L, range);\n#endif\n    }\n")
               << "    __device__ __forceinline__ void full" << sig << ", Val (&L)[G]) const { SceneFullCall{loop.sm, loop.mask}(gx, gy, gz, L); }\n};\n";
         if (columns_meta) {
             columns_meta->n_values = n_carried;

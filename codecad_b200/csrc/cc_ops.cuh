@@ -260,6 +260,30 @@ template <class V, int G> CC_DEV void cc_extrusion_n(float h, cc_val<V> (&L)[G],
     cc_extrusion_n_<CC_DEFER_CHECKS != 0>(range, h, L, cz);
 }
 
+// The distance-only forms of the column brick kernel's sweep (DESIGN.md 4.10): exactly the arithmetic of the deferred
+// cc_sphere_n_ / cc_extrusion_n_ that produces .w and the range test, none of the gradient's.  P: the sphere's point;
+// w: the extrusion's profile distance in, its distance out.
+template <class V, int G> CC_DEV void cc_sphere_dist(float r, const cc_val<V> (&P)[G], V (&w)[G], uint32_t &range)
+{
+#pragma unroll
+    for (int g = 0; g < G; ++g) {
+        const V s = vfma(P[g].x, P[g].x, vfma(P[g].y, P[g].y, vmul(P[g].z, P[g].z)));
+        vrange(range, s);
+        w[g] = vsub(vsqrt_fast(s), vbc<V>(r));
+    }
+}
+template <class V, int G> CC_DEV void cc_extrusion_dist(float h, V (&w)[G], const V (&cz)[G], uint32_t &range)
+{
+#pragma unroll
+    for (int g = 0; g < G; ++g) {
+        const V zero = vbc<V>(0.0f), az = vsub(vabs(cz[g]), vbc<V>(h));
+        const V s = vfma(az, az, vmul(w[g], w[g]));
+        vrange(range, s);
+        const V dist = vsqrt_fast(s);
+        w[g] = vsel(mand(vgt(az, zero), vgt(w[g], zero)), dist, vsel(vgt(az, w[g]), az, w[g]));
+    }
+}
+
 // shapes/common.cl:45-64
 // cc-arith pins down two cases that the formula leaves to rounding noise (both are no-ops in exact
 // arithmetic, where |c| <= 1): (1) the blend is taken only if at least one operand is closer than
@@ -896,6 +920,21 @@ CC_DEV void cc_slot_load_z(const float4 *base, float2 &z) { z = *reinterpret_cas
 // store only the z component (cells whose every reader is an extrusion)
 CC_DEV void cc_slot_store_z(float4 *base, float z) { reinterpret_cast<float *>(base)[2] = z; }
 CC_DEV void cc_slot_store_z(float4 *base, float2 z) { *reinterpret_cast<float2 *>(base + CC_THREADS) = z; }
+// a distance and its leaf id (the column brick kernel's sweep): one float4 row, (w0,w1,id0,id1) for a packed pair
+CC_DEV void cc_slot_store_wi(float4 *base, float w, float id) { *reinterpret_cast<float2 *>(base) = make_float2(w, id); }
+CC_DEV void cc_slot_store_wi(float4 *base, float2 w, float2 id) { base[0] = make_float4(w.x, w.y, id.x, id.y); }
+CC_DEV void cc_slot_load_wi_opaque(const float4 *base, float &w, float &id)
+{
+    const float2 f = cc_lds64_opaque(reinterpret_cast<const float2 *>(base));
+    w = f.x;
+    id = f.y;
+}
+CC_DEV void cc_slot_load_wi_opaque(const float4 *base, float2 &w, float2 &id)
+{
+    const float4 f = cc_lds128_opaque(base);
+    w = make_float2(f.x, f.y);
+    id = make_float2(f.z, f.w);
+}
 
 
 #endif
