@@ -272,6 +272,12 @@ template <class V, int G> CC_DEV void cc_sphere_dist(float r, const cc_val<V> (&
         w[g] = vsub(vsqrt_fast(s), vbc<V>(r));
     }
 }
+// The sweep's extrusion picks its result with min / max (CC_SWEEP_MINMAX, DESIGN.md 4.10): fminf(az, w) > 0 for
+// az > 0 && w > 0, fmaxf(az, w) for az > w ? az : w.  They differ only where an operand is NaN or both are zeros of
+// opposite sign; then s is NaN or 0, the range test flags, and the warp throws its values away.  0 keeps the selects.
+#ifndef CC_SWEEP_MINMAX
+#define CC_SWEEP_MINMAX 1
+#endif
 template <class V, int G> CC_DEV void cc_extrusion_dist(float h, V (&w)[G], const V (&cz)[G], uint32_t &range)
 {
 #pragma unroll
@@ -280,7 +286,10 @@ template <class V, int G> CC_DEV void cc_extrusion_dist(float h, V (&w)[G], cons
         const V s = vfma(az, az, vmul(w[g], w[g]));
         vrange(range, s);
         const V dist = vsqrt_fast(s);
-        w[g] = vsel(mand(vgt(az, zero), vgt(w[g], zero)), dist, vsel(vgt(az, w[g]), az, w[g]));
+        if (CC_SWEEP_MINMAX)
+            w[g] = vsel(vgt(vmin(az, w[g]), zero), dist, vmax(az, w[g]));
+        else
+            w[g] = vsel(mand(vgt(az, zero), vgt(w[g], zero)), dist, vsel(vgt(az, w[g]), az, w[g]));
     }
 }
 
