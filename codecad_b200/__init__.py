@@ -15,13 +15,14 @@ CUDA library; importing this package does not touch the GPU, the first call does
 """
 from . import opcodes  # noqa: F401
 from .geometry import BoundingBox, Vector  # noqa: F401
-from .mass_properties import MassProperties, mass_properties  # noqa: F401
+from .mass_properties import AssemblyMassProperties, MassProperties, assembly_mass_properties, mass_properties  # noqa: F401
 from .subdivision import calculate_block_sizes, subdivision  # noqa: F401
 from .grid_eval import evaluate_points, grid_eval, grid_eval_pymcubes  # noqa: F401
 from .nodes import CompiledScene, make_program, make_program_buffer  # noqa: F401
 
 __all__ = [
-    "BoundingBox", "Vector", "MassProperties", "mass_properties", "calculate_block_sizes",
+    "BoundingBox", "Vector", "MassProperties", "mass_properties", "AssemblyMassProperties", "assembly_mass_properties",
+    "calculate_block_sizes",
     "subdivision", "grid_eval", "grid_eval_pymcubes", "CompiledScene", "make_program",
     "make_program_buffer",
 ]

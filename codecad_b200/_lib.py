@@ -98,6 +98,9 @@ SIGNATURES = {
     "cc_mass_properties_exact": (_I, [_V, ctypes.POINTER(ctypes.c_double), ctypes.c_double, ctypes.POINTER(Level), _U,
                                       _U, _U, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int32),
                                       ctypes.POINTER(ctypes.c_uint64)]),
+    "cc_assembly_mass_properties_exact": (_I, [c_void_pp, _U, ctypes.POINTER(ctypes.c_double), ctypes.c_double,
+                                               ctypes.POINTER(Level), _U, _U, _U, ctypes.POINTER(ctypes.c_int64),
+                                               ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_uint64)]),
     "cc_mass_limbs_to_integrals": (_I, [ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_int32),
                                         ctypes.POINTER(ctypes.c_double)]),
     "cc_sort_leaf_corners": (_I, [ctypes.POINTER(ctypes.c_int64), ctypes.c_uint64, ctypes.POINTER(Level), _U]),

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libcodecad_b200.so")
-SOURCES = ["cc_kernels.cu", "cc_parts.cu", "cc_forest.cu", "cc_mesh.cu", "cc_polygon.cu", "cc_program.cpp", "cc_api.cpp", "cc_jit.cpp"]
+SOURCES = ["cc_kernels.cu", "cc_parts.cu", "cc_assembly.cu", "cc_forest.cu", "cc_mesh.cu", "cc_polygon.cu", "cc_program.cpp", "cc_api.cpp", "cc_jit.cpp"]
 HEADERS = ["cc_internal.h", "cc_microcode.h", "cc_math.cuh", "cc_ops.cuh", "cc_interp.cuh", "cc_body.cuh", "cc_render.cuh", "cc_device_types.h", "cc_mc_table.h", "cc_scan.cuh",
            os.path.join("..", "..", "include", "codecad_b200.h")]
 

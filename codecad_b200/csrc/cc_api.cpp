@@ -1758,6 +1758,146 @@ int mass_share(const cc_program *prog, const double box_a[3], double resolution,
     return CC_OK;
 }
 
+// An assembly's level loop keeps its per-block counters, (parts + pairs) x 40 bytes a block, under this many bytes a chunk.
+const uint64_t kAssemblyCounterBytes = 1ull << 28;
+
+// grows `buf` to `need` bytes, keeping its first `used` bytes (a level's children, gathered chunk by chunk)
+int grow_keep(DevBuf &buf, size_t &cap, size_t used, size_t need)
+{
+    if (need <= cap) return CC_OK;
+    DevBuf bigger;
+    const size_t c = std::max(need, cap * 2);
+    if (int rc = bigger.reserve(c)) return rc;
+    if (used) CU(cudaMemcpyAsync(bigger.p, buf.p, used, cudaMemcpyDeviceToDevice, g.compute));
+    CU(cudaStreamSynchronize(g.compute));
+    std::swap(buf.p, bigger.p);
+    std::swap(buf.cap, bigger.cap);
+    cap = c;
+    return CC_OK;
+}
+
+// cc_assembly_mass_properties_exact on the current device for share `rank` of `world`: mass_share's hierarchy with the
+// blocks' part masks (cc_assembly.cu); limbs = one accumulator of 41 per set (parts, then pairs), stats as mass_share
+int assembly_share(const cc_program *const *parts, uint32_t n, const double box_a[3], double resolution, const cc_level *levels,
+                   uint32_t n_levels, uint32_t rank, uint32_t world, const cc_mass_quanta &quanta, int64_t *limbs, uint64_t stats[4])
+{
+    const uint32_t n_sets = n + n * (n - 1) / 2;
+    cc_assembly_args A;
+    std::memset(&A, 0, sizeof(A));
+    A.n_parts = n;
+    uint32_t max_words = 0;
+    for (uint32_t k = 0; k < n; ++k) {
+        if (int rc = program_on_device(parts[k], &A.part[k].code)) return rc;
+        A.part[k].code_words = parts[k]->dec.info.n_micro_words;
+        A.part[k].n_slots = parts[k]->dec.info.n_slots;
+        A.max_slots = std::max(A.max_slots, A.part[k].n_slots);
+        max_words = std::max(max_words, A.part[k].code_words);
+    }
+    const size_t smem = cc_parts_smem_bytes(A.max_slots, max_words, 2);
+    if (smem > (size_t)g.prop.sharedMemPerBlockOptin)
+        return fail(CC_ERR_TOO_LARGE, "the parts need " + std::to_string(smem) + " bytes of shared memory per CTA (limit " +
+                                          std::to_string(g.prop.sharedMemPerBlockOptin) + ")");
+
+    DevBuf corners_a, corners_b, masks_a, masks_b, blocks, hit_xyz, hit_block, hit_masks, counter, sums, acc;
+    int rc;
+    if ((rc = counter.reserve(4))) return rc;
+    const size_t acc_bytes = (size_t)n_sets * 41 * sizeof(unsigned long long);
+    if ((rc = acc.reserve(acc_bytes))) return rc;
+    CU(cudaMemsetAsync(acc.p, 0, acc_bytes, g.compute));
+    // the root block: every part undecided, none inside
+    const double root[3] = {box_a[0], box_a[1], box_a[2]};
+    const uint32_t root_masks[2] = {n == 32 ? 0xffffffffu : (1u << n) - 1u, 0u};
+    if ((rc = corners_a.reserve(sizeof(root))) || (rc = masks_a.reserve(sizeof(root_masks)))) return rc;
+    CU(cudaMemcpyAsync(corners_a.p, root, sizeof(root), cudaMemcpyHostToDevice, g.compute));
+    CU(cudaMemcpyAsync(masks_a.p, root_masks, sizeof(root_masks), cudaMemcpyHostToDevice, g.compute));
+    CU(cudaStreamSynchronize(g.compute));
+    DevBuf *cur = &corners_a, *nxt = &corners_b, *cur_m = &masks_a, *nxt_m = &masks_b;
+    uint64_t n_cur = 1, n_launch = 0, n_cells = 0, n_blocks_total = 0, n_dealt = 0;
+    const uint32_t deal = deal_level_mass(n_levels);
+    const float coord_max = root_coord_bound(box_a, levels, resolution);
+    const uint64_t counter_blocks = std::max<uint64_t>(1, kAssemblyCounterBytes / ((uint64_t)n_sets * 40));
+
+    for (uint32_t l = 0; l < n_levels && n_cur; ++l) {
+        const cc_level &L = levels[l];
+        const bool leaf = (l + 1 == n_levels);
+        const uint64_t cells = (uint64_t)L.nx * L.ny * L.nz;
+        const uint64_t chunk_blocks = std::max<uint64_t>(1, std::min(kChunkCells / cells, counter_blocks));
+        const double s = resolution * (double)L.cell_size;
+        const float thr = leaf ? 0.0f : (float)(s * std::sqrt(3.0) / 2);
+        const uint32_t w = (l == deal) ? world : 1u, r = (l == deal) ? rank : 0u;
+        uint64_t n_next = 0;
+        size_t next_cap = 0, next_m_cap = 0;
+        for (uint64_t b0 = 0; b0 < n_cur; b0 += chunk_blocks) {
+            const uint32_t nb = (uint32_t)std::min<uint64_t>(chunk_blocks, n_cur - b0);
+            const size_t sums_bytes = (size_t)nb * n_sets * 10 * 4;
+            const size_t list = leaf ? 16 : (size_t)nb * cells * 4;
+            if ((rc = blocks.reserve((size_t)nb * sizeof(cc_block_desc)))) return rc;
+            if ((rc = sums.reserve(sums_bytes))) return rc;
+            if ((rc = hit_xyz.reserve(list)) || (rc = hit_block.reserve(list)) || (rc = hit_masks.reserve(2 * list))) return rc;
+            int e = cc_launch_mass_make_blocks(cur->as<double>() + 3 * b0, nb, s, blocks.as<cc_block_desc>(), g.compute);
+            if (e) return cuda_fail((cudaError_t)e, "assembly make_blocks");
+            CU(cudaMemsetAsync(counter.p, 0, 4, g.compute));
+            CU(cudaMemsetAsync(sums.p, 0, sums_bytes, g.compute));
+            cc_eval_args &a = A.a;
+            std::memset(&a, 0, sizeof(a));
+            a.step = (float)s;
+            a.nx = L.nx; a.ny = L.ny; a.nz = L.nz; a.n_blocks = nb;
+            a.blocks = blocks.as<cc_block_desc>();
+            a.coord_max = coord_max;
+            a.threshold = thr;
+            a.counter = counter.as<uint32_t>();
+            a.list = hit_xyz.as<uint8_t>();
+            a.list_block = hit_block.as<uint32_t>();
+            if ((rc = prepare_tiles(CC_SINK_MASS, 2 * CC_THREADS, a))) return rc;
+            A.masks = cur_m->as<uint32_t>() + 2 * b0;
+            A.hit_masks = hit_masks.as<uint32_t>();
+            A.sums = sums.as<uint32_t>();
+            e = cc_launch_assembly(A, smem, g.compute);
+            if (e) return cuda_fail((cudaError_t)e, "cc_assembly_kernel launch");
+            g.launches += 1;
+            g.points += (uint64_t)nb * cells;
+            n_launch += 1;
+            n_cells += (uint64_t)nb * cells;
+            n_blocks_total += nb;
+            // levels up to the dealt one are evaluated by every share; share 0 alone counts their inside cells
+            if (l > deal || rank == 0 || world == 1) {
+                e = cc_launch_mass_integrals(cur->as<double>() + 3 * b0, sums.as<uint32_t>(), nb, s, quanta,
+                                             acc.as<unsigned long long>(), g.compute, n_sets);
+                if (e) return cuda_fail((cudaError_t)e, "assembly integrals");
+            }
+            g.launches += 2;  // make_blocks, integrals
+            if (leaf) continue;
+            uint32_t hits = 0;
+            if ((rc = read_counter(counter.as<uint32_t>(), &hits))) return rc;
+            const uint64_t mine = (hits > r) ? ((uint64_t)hits - r + w - 1) / w : 0;
+            if (mine) {
+                if ((rc = grow_keep(*nxt, next_cap, (size_t)n_next * 3 * sizeof(double), (size_t)(n_next + mine) * 3 * sizeof(double))) ||
+                    (rc = grow_keep(*nxt_m, next_m_cap, (size_t)n_next * 8, (size_t)(n_next + mine) * 8)))
+                    return rc;
+                e = cc_launch_mass_expand_children(cur->as<double>() + 3 * b0, hit_block.as<uint32_t>(), hit_xyz.as<uint8_t>(), hits, s,
+                                                   r, w, nxt->as<double>() + 3 * n_next, g.compute, hit_masks.as<uint32_t>(),
+                                                   nxt_m->as<uint32_t>() + 2 * n_next);
+                if (e) return cuda_fail((cudaError_t)e, "assembly expand_children");
+                g.launches += 1;
+                n_next += mine;
+            }
+        }
+        std::swap(cur, nxt);
+        std::swap(cur_m, nxt_m);
+        n_cur = n_next;
+        if (l == deal) n_dealt = n_cur;
+    }
+    std::vector<unsigned long long> h_acc((size_t)n_sets * 41);
+    CU(cudaMemcpyAsync(h_acc.data(), acc.p, acc_bytes, cudaMemcpyDeviceToHost, g.compute));
+    CU(cudaStreamSynchronize(g.compute));
+    for (size_t i = 0; i < h_acc.size(); ++i) limbs[i] = (int64_t)h_acc[i];
+    stats[0] = n_launch;
+    stats[1] = n_cells;
+    stats[2] = n_blocks_total;
+    stats[3] = n_dealt;
+    return CC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1846,6 +1986,56 @@ int cc_mass_properties_exact(const cc_program *prog, const double box_a[3], doub
         stats[4] = s4[3];      // blocks of the dealt level owned by this call's devices
         stats[5] = nd;         // devices used
         stats[6] = max_cells;  // cells evaluated by the busiest / the least busy device
+        stats[7] = min_cells;
+    }
+    return CC_OK;
+}
+
+int cc_assembly_mass_properties_exact(const cc_program *const *parts, uint32_t n_parts, const double box_a[3], double resolution,
+                                      const cc_level *levels, uint32_t n_levels, uint32_t rank, uint32_t world, int64_t *limbs,
+                                      int32_t exponents[10], uint64_t stats[8])
+{
+    NEED_INIT();
+    if (!parts || !box_a || !levels || !limbs || !exponents) return fail(CC_ERR_INVALID_ARGUMENT, "null argument");
+    if (n_parts == 0 || n_parts > CC_ASSEMBLY_MAX_PARTS) return fail(CC_ERR_INVALID_ARGUMENT, "an assembly has 1 to 32 parts");
+    for (uint32_t k = 0; k < n_parts; ++k)
+        if (!parts[k]) return fail(CC_ERR_INVALID_ARGUMENT, "null part program");
+    if (n_levels < 1) return fail(CC_ERR_INVALID_ARGUMENT, "no levels");
+    if (world == 0 || rank >= world) return fail(CC_ERR_INVALID_ARGUMENT, "bad rank/world");
+    int rc = check_levels(levels, n_levels);
+    if (rc) return rc;
+    if (!(resolution > 0)) return fail(CC_ERR_INVALID_ARGUMENT, "resolution must be positive");
+    const cc_mass_quanta quanta = mass_quanta(box_a, resolution, levels[0]);
+    const uint32_t n_sets = n_parts + n_parts * (n_parts - 1) / 2;
+    const uint32_t nd = (uint32_t)std::max(1, g_n_ctx);
+    std::vector<int64_t> part((size_t)nd * n_sets * 41, 0);
+    std::vector<uint64_t> st((size_t)nd * 4, 0);
+    rc = for_each_device([&](int i) {
+        return assembly_share(parts, n_parts, box_a, resolution, levels, n_levels, rank * nd + (uint32_t)i, world * nd, quanta,
+                              part.data() + (size_t)i * n_sets * 41, st.data() + (size_t)i * 4);
+    });
+    if (rc) return rc;
+    int64_t overflow = 0;
+    for (uint32_t set = 0; set < n_sets; ++set)
+        for (int k = 0; k < 40; ++k) limbs[(size_t)set * 40 + k] = 0;
+    uint64_t s4[4] = {0, 0, 0, 0}, max_cells = 0, min_cells = UINT64_MAX;
+    for (uint32_t i = 0; i < nd; ++i) {
+        for (uint32_t set = 0; set < n_sets; ++set) {
+            const int64_t *p = part.data() + ((size_t)i * n_sets + set) * 41;
+            for (int k = 0; k < 40; ++k) limbs[(size_t)set * 40 + k] += p[k];
+            overflow += p[40];
+        }
+        for (int k = 0; k < 4; ++k) s4[k] += st[(size_t)i * 4 + k];
+        max_cells = std::max(max_cells, st[(size_t)i * 4 + 1]);
+        min_cells = std::min(min_cells, st[(size_t)i * 4 + 1]);
+    }
+    if (overflow) return fail(CC_ERR_INVALID_ARGUMENT, "mass integrals left the range of the exact accumulator");
+    for (int i = 0; i < 10; ++i) exponents[i] = quanta.e[i];
+    if (stats) {
+        stats[0] = s4[0]; stats[1] = s4[1]; stats[2] = s4[2]; stats[3] = n_levels;
+        stats[4] = s4[3];
+        stats[5] = nd;
+        stats[6] = max_cells;
         stats[7] = min_cells;
     }
     return CC_OK;

@@ -26,12 +26,81 @@ CC_DEV auto cc_eval_locate_(int, EVAL &e, const T &...t) -> decltype(e.locate(t.
     e.locate(t...);
 }
 
+// Point j of a thread of a linear tile of the block with corner (cx, cy, cz): the cell
+// tile_in_block * CC_THREADS * PTS + j * CC_THREADS + tid in INDEX3 order (0 past the block's last cell, where `valid`
+// is false; returned) and its fp32 grid coordinates.  Every body over blocks x linear tiles takes its points from here
+// (cc_kernel_body, cc_assembly.cu): results that must agree bit for bit across them rest on these lines.
+template <int PTS>
+CC_DEV uint32_t cc_tile_cell(const cc_eval_args &a, uint32_t tile_in_block, int j, float cx, float cy, float cz, uint32_t &ix,
+                             uint32_t &iy, uint32_t &iz, float &gx, float &gy, float &gz, bool &valid)
+{
+    const uint32_t cells = a.nx * a.ny * a.nz, nyz = a.ny * a.nz;
+    uint32_t c = tile_in_block * (CC_THREADS * PTS) + j * CC_THREADS + threadIdx.x;
+    valid = c < cells;
+    c = valid ? c : 0u;
+    ix = c / nyz;
+    const uint32_t r = c - ix * nyz;
+    iy = r / a.nz;
+    iz = r - iy * a.nz;
+    // grid_eval.cl:13,31: corner + step * convert_float(id), one FMA per axis
+    gx = cc_fma(a.step, (float)(ix + a.x_offset), cx);
+    gy = cc_fma(a.step, (float)iy, cy);
+    gz = cc_fma(a.step, (float)iz, cz);
+    return c;
+}
+
+// A cell's ten index products, added to the MASS sink's sums: mass_properties.cl:34-41, order xx,xy,xz,x,yy,yz,y,zz,z,n
+CC_DEV void cc_add_moments(uint32_t (&sum)[10], uint32_t x, uint32_t y, uint32_t z)
+{
+    sum[0] += x * x; sum[1] += x * y; sum[2] += x * z; sum[3] += x;
+    sum[4] += y * y; sum[5] += y * z; sum[6] += y; sum[7] += z * z;
+    sum[8] += z; sum[9] += 1u;
+}
+
+// Ordered compaction of a tile's hits (CTA-wide): the list position of every point j with hit[j], in cell order (j major,
+// then warp, then lane) after the hits of all earlier tiles (ticket order, decoupled look-back on a.tile_status); the
+// tile of the launch's last ticket writes the final list length to *a.counter.
+template <int PTS>
+CC_DEV void cc_tile_rank(const cc_eval_args &a, uint32_t tile, const bool (&hit)[PTS], uint32_t (&pos)[PTS])
+{
+    __shared__ uint32_t s_warp[PTS * (CC_THREADS / 32)];
+    __shared__ uint32_t s_base;
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t ballot[PTS];
+#pragma unroll
+    for (int j = 0; j < PTS; ++j) {
+        ballot[j] = __ballot_sync(0xffffffffu, hit[j]);
+        if (lane == 0) s_warp[j * (CC_THREADS / 32) + warp] = __popc(ballot[j]);
+    }
+    __syncthreads();
+    if (warp == 0) {
+        // exclusive scan of the PTS * 4 warp counts (<= 32 entries) with shuffles
+        constexpr int NW = PTS * (CC_THREADS / 32);
+        static_assert(NW <= 32, "the warp-count scan covers at most 32 entries");
+        uint32_t v = (lane < NW) ? s_warp[lane] : 0u;
+        uint32_t incl = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            uint32_t t = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += t;
+        }
+        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+        if (lane < NW) s_warp[lane] = incl - v;
+        uint32_t base = cc_lookback(a.tile_status, tile, total, a.counter);
+        if (lane == 0) {
+            s_base = base;
+            if (tile == gridDim.x - 1) *a.counter = base + total;  // final list length
+        }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < PTS; ++j) pos[j] = s_base + s_warp[j * (CC_THREADS / 32) + warp] + __popc(ballot[j] & ((1u << lane) - 1u));
+}
+
 template <int PTS, int SINK, class EVAL, bool POINTS = false>
 CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
 {
     __shared__ uint32_t s_tile;
-    __shared__ uint32_t s_warp[PTS * (CC_THREADS / 32)];
-    __shared__ uint32_t s_base;
 
     const uint32_t tid = threadIdx.x;
     constexpr bool ORDERED = (SINK == CC_SINK_CLASSIFY || SINK == CC_SINK_MASS);
@@ -50,7 +119,6 @@ CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
         cx = bd.cx; cy = bd.cy; cz = bd.cz;
     }
     const uint32_t cells = a.nx * a.ny * a.nz;  // <= 2^31 per launch (host checks)
-    const uint32_t nyz = a.ny * a.nz;
 
     typedef typename cc_pts<PTS>::V V;
     constexpr int G = cc_pts<PTS>::G, NL = cc_lane<V>::N;
@@ -59,17 +127,7 @@ CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
     bool valid[PTS];
 #pragma unroll
     for (int j = 0; j < PTS; ++j) {
-        uint32_t c = tile_in_block * (CC_THREADS * PTS) + j * CC_THREADS + tid;
-        valid[j] = c < cells;
-        c = valid[j] ? c : 0u;
-        ix[j] = c / nyz;
-        uint32_t r = c - ix[j] * nyz;
-        iy[j] = r / a.nz;
-        iz[j] = r - iy[j] * a.nz;
-        // grid_eval.cl:13,31: corner + step * convert_float(id), one FMA per axis
-        gx[j] = cc_fma(a.step, (float)(ix[j] + a.x_offset), cx);
-        gy[j] = cc_fma(a.step, (float)iy[j], cy);
-        gz[j] = cc_fma(a.step, (float)iz[j], cz);
+        const uint32_t c = cc_tile_cell<PTS>(a, tile_in_block, j, cx, cy, cz, ix[j], iy[j], iz[j], gx[j], gy[j], gz[j], valid[j]);
         if (POINTS) {
             const float4 p = reinterpret_cast<const float4 *>(a.points)[c];
             gx[j] = p.x; gy[j] = p.y; gz[j] = p.z;
@@ -109,7 +167,7 @@ CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
         }
     } else {
         // ---- classification ----
-        const uint32_t lane = tid & 31, warp = tid >> 5;
+        const uint32_t lane = tid & 31;
         bool hit[PTS];
         uint32_t sum[10];
 #pragma unroll
@@ -122,13 +180,7 @@ CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
             } else {
                 const bool inside = valid[j] && (v <= -a.threshold);  // mass_properties.cl:31
                 hit[j] = valid[j] && !inside && (v < a.threshold);    // mass_properties.cl:43
-                if (inside) {
-                    // mass_properties.cl:34-41, order xx,xy,xz,x,yy,yz,y,zz,z,n
-                    const uint32_t x = ix[j], y = iy[j], z = iz[j];
-                    sum[0] += x * x; sum[1] += x * y; sum[2] += x * z; sum[3] += x;
-                    sum[4] += y * y; sum[5] += y * z; sum[6] += y; sum[7] += z * z;
-                    sum[8] += z; sum[9] += 1u;
-                }
+                if (inside) cc_add_moments(sum, ix[j], iy[j], iz[j]);
             }
         }
         if (SINK == CC_SINK_MASS) {
@@ -145,42 +197,14 @@ CC_DEV void cc_kernel_body(const cc_eval_args &a, EVAL &eval)
         // empty, and the tile neither ranks nor waits for its predecessors.  (Warp-uniform: a launch
         // argument.)  The leaf launch is 98 % of a mass_properties call.
         if (SINK == CC_SINK_MASS && a.threshold == 0.0f) return;
-        // ranks inside the tile, in cell order (j major, then warp, then lane)
-        uint32_t ballot[PTS];
-#pragma unroll
-        for (int j = 0; j < PTS; ++j) {
-            ballot[j] = __ballot_sync(0xffffffffu, hit[j]);
-            if (lane == 0) s_warp[j * (CC_THREADS / 32) + warp] = __popc(ballot[j]);
-        }
-        __syncthreads();
-        if (warp == 0) {
-            // exclusive scan of the PTS * 4 warp counts (<= 32 entries) with shuffles
-            constexpr int NW = PTS * (CC_THREADS / 32);
-            static_assert(NW <= 32, "the warp-count scan covers at most 32 entries");
-            uint32_t v = (lane < NW) ? s_warp[lane] : 0u;
-            uint32_t incl = v;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                uint32_t t = __shfl_up_sync(0xffffffffu, incl, d);
-                if (lane >= d) incl += t;
-            }
-            const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-            if (lane < NW) s_warp[lane] = incl - v;
-            uint32_t base = cc_lookback(a.tile_status, tile, total, a.counter);
-            if (lane == 0) {
-                s_base = base;
-                if (tile == gridDim.x - 1) *a.counter = base + total;  // final list length
-            }
-        }
-        __syncthreads();
-        const uint32_t base = s_base;
+        uint32_t pos[PTS];
+        cc_tile_rank<PTS>(a, tile, hit, pos);
 #pragma unroll
         for (int j = 0; j < PTS; ++j) {
             if (hit[j]) {
-                uint32_t pos = base + s_warp[j * (CC_THREADS / 32) + warp] + __popc(ballot[j] & ((1u << lane) - 1u));
-                reinterpret_cast<uchar4 *>(a.list)[pos] =
+                reinterpret_cast<uchar4 *>(a.list)[pos[j]] =
                     make_uchar4((unsigned char)ix[j], (unsigned char)iy[j], (unsigned char)iz[j], 0);
-                if (a.list_block) a.list_block[pos] = block;
+                if (a.list_block) a.list_block[pos[j]] = block;
             }
         }
     }

@@ -234,15 +234,36 @@ int cc_launch_expand_children(const int64_t *d_parent_corners, const uint32_t *d
 // mass properties: float64 corner chain + per-block integrals
 int cc_launch_mass_make_blocks(const double *d_corners, uint32_t n, double s, cc_block_desc *d_blocks,
                                void *stream);
+// d_hit_masks / d_child_masks (assemblies): the (eval, inside) part masks of every hit, copied to its child block
 int cc_launch_mass_expand_children(const double *d_parent_corners, const uint32_t *d_hit_block,
                                    const uint8_t *d_hit_xyz, uint32_t n_hits, double s,
-                                   uint32_t rank, uint32_t world, double *d_child_corners, void *stream);
+                                   uint32_t rank, uint32_t world, double *d_child_corners, void *stream,
+                                   const uint32_t *d_hit_masks = nullptr, uint32_t *d_child_masks = nullptr);
 // per-block integrals (mass_properties.py:139-148, float64) added to an exact fixed-point accumulator:
 // d_limbs[10][4] signed 64-bit sums of the 32-bit limbs of trunc(value / 2^quantum_exp[i]); d_limbs[40]
 // counts values outside the accumulator's range (must stay 0)
 struct cc_mass_quanta { int e[10]; };
+// n_sets sets of ten sums per block (stride 10 * n_sets), each into its own accumulator of 41 limbs
 int cc_launch_mass_integrals(const double *d_corners, const uint32_t *d_sums, uint32_t n_blocks, double s,
-                             cc_mass_quanta q, unsigned long long *d_limbs /* [41] */, void *stream);
+                             cc_mass_quanta q, unsigned long long *d_limbs /* [n_sets][41] */, void *stream,
+                             uint32_t n_sets = 1);
+
+// ---- mass properties of an assembly's parts and pairs in one hierarchy pass (cc_assembly.cu, DESIGN.md 4.11) --------
+#define CC_ASSEMBLY_MAX_PARTS 32
+struct cc_assembly_part {
+    const uint32_t *code;  // the part program's microcode on the launch's device
+    uint32_t code_words, n_slots;
+};
+struct cc_assembly_args {
+    cc_eval_args a;         // blocks x linear tiles of CC_THREADS x 2 cells; threshold, hit list, ticket and look-back
+    cc_assembly_part part[CC_ASSEMBLY_MAX_PARTS];
+    uint32_t n_parts;
+    uint32_t max_slots;     // the dynamic shared memory (cc_parts_smem_bytes, 2 points) holds max_slots register slots, then one microcode
+    const uint32_t *masks;  // per block: (eval, inside) part masks
+    uint32_t *hit_masks;    // per hit: the child block's (eval, inside)
+    uint32_t *sums;         // per block: n_parts + n_parts (n_parts - 1) / 2 sets of ten sums
+};
+int cc_launch_assembly(const cc_assembly_args &A, size_t smem, void *stream);
 
 // ---- 2-D outline extraction (cc_polygon.cu, rendering/polygon2d.cl) -----------------------------
 #ifdef __CUDACC__

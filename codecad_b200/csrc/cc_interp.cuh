@@ -28,6 +28,20 @@ struct Prog {
     }
 };
 
+// Copies `words` words of microcode (a multiple of four) from global to shared memory with 16-byte cp.async, all threads
+// of the CTA, and waits for them.  The caller makes sure no thread still reads what s_code held before.
+CC_DEV void cc_stage_code(const uint32_t *code, uint32_t words, uint32_t *s_code)
+{
+    const uint32_t n4 = words / 4;
+    for (uint32_t i = threadIdx.x; i < n4; i += CC_THREADS) {
+        uint32_t dsts = (uint32_t)__cvta_generic_to_shared(s_code + 4 * i);
+        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dsts), "l"(code + 4 * i) : "memory");
+    }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    __syncthreads();
+}
+
 template <int MODE>
 struct ProgFetch {
     Prog<MODE> P;

@@ -273,11 +273,13 @@ __global__ void cc_mass_make_blocks_kernel(const double *__restrict__ corners, u
     out[i] = b;
 }
 
-// mass_properties.py:154-157: child corner = Vector(i,j,k) * s + box_corner (float64)
+// mass_properties.py:154-157: child corner = Vector(i,j,k) * s + box_corner (float64).  With mask arrays (the assembly's
+// hierarchy, cc_assembly.cu) the hit's two part masks go to the child block too.
 __global__ void cc_mass_expand_children_kernel(const double *__restrict__ parents,
                                                const uint32_t *__restrict__ hit_block,
                                                const uchar4 *__restrict__ hit_xyz, uint32_t n_hits, double s,
-                                               uint32_t rank, uint32_t world, double *__restrict__ out)
+                                               uint32_t rank, uint32_t world, double *__restrict__ out,
+                                               const uint2 *__restrict__ hit_masks, uint2 *__restrict__ out_masks)
 {
     uint32_t h = blockIdx.x * blockDim.x + threadIdx.x;
     if (h >= n_hits || (h % world) != rank) return;
@@ -287,6 +289,7 @@ __global__ void cc_mass_expand_children_kernel(const double *__restrict__ parent
     out[3 * o + 0] = __dadd_rn(__dmul_rn((double)c.x, s), parents[3 * b + 0]);
     out[3 * o + 1] = __dadd_rn(__dmul_rn((double)c.y, s), parents[3 * b + 1]);
     out[3 * o + 2] = __dadd_rn(__dmul_rn((double)c.z, s), parents[3 * b + 2]);
+    if (hit_masks) out_masks[o] = hit_masks[h];
 }
 
 // mass_properties.py:119-148: per block, index sums -> the ten integrals, in float64 with the
@@ -318,12 +321,16 @@ __device__ __forceinline__ void cc_to_limbs(double v, int quantum_exp, long long
     for (int k = 0; k < 4; ++k) limb[k] = sign * (long long)((unsigned long long)(t >> (32 * k)) & 0xffffffffull);
 }
 
+// Several sets of sums per block (an assembly's parts and pairs): set blockIdx.y of block b is at
+// sums + b * set_stride + 10 * blockIdx.y and goes into accumulator acc + 41 * blockIdx.y.  One set: stride 10.
 __global__ void __launch_bounds__(256) cc_mass_integrals_kernel(const double *__restrict__ corners,
                                                                 const uint32_t *__restrict__ sums,
                                                                 uint32_t n_blocks, double s, cc_mass_quanta qe,
-                                                                unsigned long long *__restrict__ acc)
+                                                                unsigned long long *__restrict__ acc, uint32_t set_stride)
 {
     const uint32_t b = blockIdx.x * 256u + threadIdx.x;
+    sums += 10u * blockIdx.y;
+    acc += 41u * blockIdx.y;
     const double s2 = __dmul_rn(s, s);
     const double s3 = __dmul_rn(s, s2);
     const double half = __ddiv_rn(s, 2.0);
@@ -331,8 +338,8 @@ __global__ void __launch_bounds__(256) cc_mass_integrals_kernel(const double *__
     double v[10];
 #pragma unroll
     for (int i = 0; i < 10; ++i) v[i] = 0.0;
-    if (b < n_blocks && sums[(size_t)b * 10 + 9] != 0) {
-        const uint32_t *q = sums + (size_t)b * 10;
+    if (b < n_blocks && sums[(size_t)b * set_stride + 9] != 0) {
+        const uint32_t *q = sums + (size_t)b * set_stride;
         const double sxx = q[0], sxy = q[1], sxz = q[2], sx = q[3], syy = q[4], syz = q[5], sy = q[6],
                      szz = q[7], sz = q[8], n = q[9];
         const double bx = __dadd_rn(corners[3 * b + 0], half);
@@ -398,20 +405,21 @@ int cc_launch_mass_make_blocks(const double *d_corners, uint32_t n, double s, cc
 
 int cc_launch_mass_expand_children(const double *d_parent_corners, const uint32_t *d_hit_block,
                                    const uint8_t *d_hit_xyz, uint32_t n_hits, double s, uint32_t rank,
-                                   uint32_t world, double *d_child_corners, void *stream)
+                                   uint32_t world, double *d_child_corners, void *stream,
+                                   const uint32_t *d_hit_masks, uint32_t *d_child_masks)
 {
     if (!n_hits) return 0;
     cc_mass_expand_children_kernel<<<(n_hits + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
         d_parent_corners, d_hit_block, reinterpret_cast<const uchar4 *>(d_hit_xyz), n_hits, s, rank, world,
-        d_child_corners);
+        d_child_corners, reinterpret_cast<const uint2 *>(d_hit_masks), reinterpret_cast<uint2 *>(d_child_masks));
     return (int)cudaGetLastError();
 }
 
 int cc_launch_mass_integrals(const double *d_corners, const uint32_t *d_sums, uint32_t n_blocks, double s,
-                             cc_mass_quanta q, unsigned long long *d_limbs, void *stream)
+                             cc_mass_quanta q, unsigned long long *d_limbs, void *stream, uint32_t n_sets)
 {
     if (!n_blocks) return 0;
-    cc_mass_integrals_kernel<<<(n_blocks + 255) / 256, 256, 0, (cudaStream_t)stream>>>(d_corners, d_sums, n_blocks, s, q,
-                                                                                      d_limbs);
+    const dim3 grid((n_blocks + 255) / 256, n_sets);
+    cc_mass_integrals_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_corners, d_sums, n_blocks, s, q, d_limbs, 10u * n_sets);
     return (int)cudaGetLastError();
 }

@@ -19,14 +19,7 @@ struct cc_parts_interp_args {
 CC_DEV const uint32_t *ccp_stage(const cc_eval_args &a, float4 *smem4, int pts)
 {
     uint32_t *s_code = reinterpret_cast<uint32_t *>(smem4 + (size_t)a.n_slots * pts * CC_THREADS);
-    const uint32_t n4 = a.code_words / 4;
-    for (uint32_t i = threadIdx.x; i < n4; i += CC_THREADS) {
-        uint32_t dsts = (uint32_t)__cvta_generic_to_shared(s_code + 4 * i);
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dsts), "l"(a.code + 4 * i) : "memory");
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncthreads();
+    cc_stage_code(a.code, a.code_words, s_code);
     return s_code;
 }
 

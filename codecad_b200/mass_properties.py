@@ -7,6 +7,7 @@ come back (summed over ranks with an NCCL all-reduce when sharded).
 """
 import collections
 import ctypes
+import functools
 
 import numpy as np
 
@@ -38,6 +39,30 @@ def mass_limbs(program, box_a, resolution, block_sizes, rank=0, world=1):
                                                    len(block_sizes), int(rank), int(world), limbs, exps, stats))
     return (np.array(limbs[:], dtype=np.int64), np.array(exps[:], dtype=np.int32),
             dict(zip(STAT_NAMES, (int(v) for v in stats))))
+
+
+def assembly_limbs(programs, box_a, resolution, block_sizes, rank=0, world=1):
+    """The parts of an assembly and the overlaps of every pair of them in one hierarchy pass
+    (cc_assembly_mass_properties_exact, DESIGN.md 4.11): this rank's share as exact accumulators, (limbs
+    int64[sets][40], exponents int32[10], stats dict).  Row k < n is programs[k], bit for bit what
+    mass_limbs(programs[k], ...) returns; the pairs {a < b} follow in lexicographic order (pair_index)."""
+    n = len(programs)
+    sets = n + n * (n - 1) // 2
+    handles = (ctypes.c_void_p * max(n, 1))(*[p.handle if p is not None else None for p in programs])
+    limbs = (ctypes.c_int64 * (40 * max(sets, 1)))()
+    exps = (ctypes.c_int32 * 10)()
+    stats = (ctypes.c_uint64 * 8)()
+    a = (ctypes.c_double * 3)(float(box_a[0]), float(box_a[1]), float(box_a[2]))
+    _lib.check(_lib.lib().cc_assembly_mass_properties_exact(handles, n, a, float(resolution), _levels(block_sizes),
+                                                            len(block_sizes), int(rank), int(world), limbs, exps, stats))
+    return (np.array(limbs[:40 * sets], dtype=np.int64).reshape(sets, 40), np.array(exps[:], dtype=np.int32),
+            dict(zip(STAT_NAMES, (int(v) for v in stats))))
+
+
+def pair_index(n, a, b):
+    """Row of the pair {a, b} (a != b) among the sets of an assembly of n parts."""
+    a, b = min(a, b), max(a, b)
+    return n + a * n - a * (a + 1) // 2 + (b - a - 1)
 
 
 def limbs_to_integrals(limbs, exponents):
@@ -110,6 +135,54 @@ def mass_properties(shape, resolution, grid_size=None, group=None, stats=None):
     if world > 1:
         limbs = allreduce_limbs(limbs, None if group is True else group)
     return finish(limbs_to_integrals(limbs, exps))
+
+
+class AssemblyMassProperties(collections.namedtuple("AssemblyMassProperties", "parts interference")):
+    """`parts`: a MassProperties per shape, in the order given; `interference`: {(i, j): MassProperties} of the
+    overlap of shapes i < j, for the pairs whose overlap has a non-zero volume."""
+
+    __slots__ = ()
+
+
+def assembly_mass_properties(shapes, resolution, grid_size=None, group=None, stats=None):
+    """mass_properties() of every shape of an assembly, and of the overlap of every pair of them (the
+    interference check), in one hierarchy pass over the union of the shapes' bounding boxes.  Part k is
+    exactly mass_properties() of shapes[k] on that box.  `group` and `stats` as for mass_properties()."""
+    if grid_size is None:
+        grid_size = 64
+    shapes = list(shapes)
+    assert 1 <= len(shapes) <= 32, "an assembly has 1 to 32 parts"
+    assert all(s.dimension() == 3 for s in shapes), "2D objects are not supported yet"
+    assert resolution > 0, "Non-positive resolution makes no sense"
+    assert grid_size > 1, "Grid needs to be at least 2x2x2"
+    assert grid_size ** 5 <= 2 ** 32, "Centroid coordinate sums would overflow"
+
+    programs = [make_program_buffer(s) for s in shapes]
+    boxes = [s.bounding_box() for s in shapes]
+    box_a = functools.reduce(Vector.min, (as_vector(b[0]) for b in boxes))
+    box_b = functools.reduce(Vector.max, (as_vector(b[1]) for b in boxes))
+    block_sizes = calculate_block_sizes((box_a, box_b), 3, resolution, grid_size, overlap=False)
+
+    rank, world = 0, 1
+    if group is not None:
+        import torch.distributed as dist
+        pg = None if group is True else group
+        rank, world = dist.get_rank(pg), dist.get_world_size(pg)
+
+    limbs, exps, st = assembly_limbs(programs, box_a, resolution, block_sizes, rank, world)
+    if stats is not None:
+        stats.update(st)
+    if world > 1:
+        limbs = allreduce_limbs(limbs, None if group is True else group)
+    n = len(shapes)
+    parts = [finish(limbs_to_integrals(limbs[k], exps)) for k in range(n)]
+    interference = {}
+    for a in range(n):
+        for b in range(a + 1, n):
+            mp = finish(limbs_to_integrals(limbs[pair_index(n, a, b)], exps))
+            if mp.volume != 0:
+                interference[(a, b)] = mp
+    return AssemblyMassProperties(parts, interference)
 
 
 def allreduce_limbs(limbs, group=None):

@@ -295,6 +295,34 @@ int cc_mass_properties_exact(const cc_program *prog, const double box_a[3], doub
                              int64_t limbs[40], int32_t exponents[10], uint64_t stats[8]);
 int cc_mass_limbs_to_integrals(const int64_t limbs[40], const int32_t exponents[10], double integrals[10]);
 
+/* Mass properties of an assembly: every part, and the overlap of every pair of parts, in one
+ * hierarchy pass (DESIGN.md 4.11).  parts[0..n_parts) (1 <= n_parts <= 32) are ordinary programs,
+ * already placed; box_a, resolution and levels are those of cc_mass_properties_exact.
+ *
+ * The hierarchy is mass_properties' (same blocks, float64 corner chain, fp32 cell coordinates and
+ * thresholds; leaf threshold 0).  Every block carries `eval`, the parts undecided at its parent
+ * cell (the root: all), and `inside`, the parts decided inside at an ancestor cell (the root:
+ * none).  In a cell only the parts of `eval` are evaluated; part k is inside if D_k <= -thr, near
+ * if not inside and D_k < thr, outside otherwise (NaN included).  With N the parts newly inside and
+ * U the parts near:
+ *   - the cell's ten index products go into part k's sums for every k in N;
+ *   - ... and into pair {a, b}'s sums for every a in N, b in N u inside, a != b (once per pair);
+ *   - U nonempty: the cell becomes a child block with eval = U, inside = inside u N.
+ * So set k is bit for bit cc_mass_properties_exact(parts[k], ...) (part k is evaluated in exactly
+ * the blocks of its own hierarchy), and pair {a, b} is the intersection of the two parts' counted
+ * regions: [A, A] gives pair = A.  For 1-Lipschitz fields vol(A u B) = vol A + vol B - vol AB.
+ *
+ * limbs[sets][40] with sets = n_parts + n_parts (n_parts - 1) / 2: the parts, then pair {a < b}
+ * at n_parts + a n_parts - a (a + 1) / 2 + (b - a - 1); each set is an accumulator of
+ * cc_mass_properties_exact (same exponents, same sharding over ranks and devices).  stats as
+ * there.  CC_ERR_INVALID_ARGUMENT: no parts, more than 32, a null part, bad rank / world, an
+ * accumulator out of range; CC_ERR_TOO_LARGE: the parts' slots and microcode exceed a CTA's shared
+ * memory. */
+int cc_assembly_mass_properties_exact(const cc_program *const *parts, uint32_t n_parts, const double box_a[3],
+                                      double resolution, const cc_level *levels, uint32_t n_levels,
+                                      uint32_t rank, uint32_t world, int64_t *limbs /* sets x 40 */,
+                                      int32_t exponents[10], uint64_t stats[8]);
+
 /* matplotlib_slice  rendering/matplotlib_slice.cl:1-20 (global size (width, height),
  * rendering/matplotlib_slice.py:44-52): d_out[(x + y*width)*3 + 0..2] = distance, gradient x,
  * gradient y at corner + step * (x, y, 0) — the numpy array [height][width][3] the viewer plots. */
