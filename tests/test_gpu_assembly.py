@@ -9,6 +9,7 @@ import pytest
 
 import programs as P
 from assembly_oracle import assembly_mass_properties as oracle_assembly
+from exact_mass import buffers as _buffers, integrals as _integrals, lipschitz_parts, part_box as _part_box, plan as _plan
 
 pytestmark = pytest.mark.gpu
 
@@ -32,26 +33,10 @@ def jit(cb, request):
     _lib.check(_lib.lib().cc_set_jit_mode(old))
 
 
-def _buffers(words_list):
-    from codecad_b200.cl_util.buffer import ProgramBuffer
-    return [ProgramBuffer(np.asarray(w, np.float32)) for w in words_list]
-
-
-def _plan(box_a, box_b, resolution, grid):
-    from codecad_b200.geometry import Vector
-    from codecad_b200.subdivision import calculate_block_sizes
-    a, b = Vector(*box_a), Vector(*box_b)
-    return a, b, calculate_block_sizes((a, b), 3, resolution, grid, overlap=False)
-
-
 def _union_box(scenes_list):
     a = tuple(min(s.box_a[i] for s in scenes_list) for i in range(3))
     b = tuple(max(s.box_b[i] for s in scenes_list) for i in range(3))
     return a, b
-
-
-def _integrals(limbs, exps):
-    return np.array([mpm.limbs_to_integrals(row, exps) for row in np.atleast_2d(limbs)])
 
 
 # ---- groups of parts -------------------------------------------------------------------------------------------------
@@ -65,21 +50,6 @@ FIXTURE_GROUPS = {
 def _cloud(seed, n, spread=2.5, size=1.5):
     rng = np.random.default_rng(seed)
     return P.primitive_cloud(rng, n, (0.0, 0.0, 0.0), spread, size)
-
-
-def _part_box(parts, margin=0.5):
-    """a box around parts of tests/programs.py: each part's centre (where its placement puts its frame's origin) +- a
-    radius that bounds the part"""
-    lo, hi = [], []
-    for p in parts:
-        centre = -(P.quat_matrix(p.q).T @ np.asarray(p.t))
-        kind = p.profile[0]
-        r = float(np.linalg.norm(p.profile[1], axis=1).max()) if kind == "polygon" else \
-            float(np.hypot(p.profile[1], p.profile[2])) if kind == "rectangle" else p.profile[1]
-        r = float(np.hypot(r, p.h)) + (p.offset or 0.0) + margin
-        lo.append(centre - r)
-        hi.append(centre + r)
-    return tuple(np.min(lo, axis=0).tolist()), tuple(np.max(hi, axis=0).tolist())
 
 
 def _program_groups():
@@ -159,18 +129,9 @@ def test_pairs_match_the_restatement(cb, scenes, names, res, grid):
     assert (want[len(ss):, 0] > 0).any()
 
 
-def _lipschitz_parts(kind):
-    box = P.Part.placed(P.Part.box(1.0, 1.5, 1.2), (0.0, 0.0, 0.0), P.quat((1.0, 2.0, 0.5), 0.3))
-    cyl = P.Part.placed(P.Part.cylinder(1.1, 1.0), (1.2, 0.4, 0.3), P.quat((0.2, 1.0, 0.1), 0.7))
-    if kind == "two":
-        return [box, cyl]
-    far = P.Part.placed(P.Part.box(0.8, 0.8, 0.8), (-1.6, -0.4, 0.2))  # overlaps the box, not the cylinder
-    return [box, cyl, far]
-
-
 @pytest.mark.parametrize("kind", ["two", "three"])
 def test_inclusion_exclusion(cb, kind):
-    parts = _lipschitz_parts(kind)
+    parts = lipschitz_parts(kind)
     box_a, box_b = _part_box(parts)
     res = 0.03
     a, _, plan = _plan(box_a, box_b, res, 16)
@@ -188,6 +149,8 @@ def test_inclusion_exclusion(cb, kind):
     assert combined[0] == pytest.approx(u[0], rel=1e-12)
     m = max(abs(v) for v in box_a + box_b)
     assert np.allclose(combined[1:4], u[1:4], rtol=1e-12, atol=1e-12 * u[0] * m)
+    # the second moments (the inertia): the same bar, one more coordinate
+    assert np.allclose(combined[4:], u[4:], rtol=1e-12, atol=1e-12 * u[0] * m * m)
 
 
 def test_disjoint_parts(cb):
